@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- agent-steps/s of the Snake-v1 step path on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over the whole batch: ONE launch of snk_tile_kernel stepping every
 environment of the shard (rules + auto-reset + observation render).  Workload (config.workload): BASELINE
@@ -14,6 +14,11 @@ resident in HBM; e2e = the same metric through the C ABI's host-buffer call (snk
 actions H2D, step, obs + rewards + dones D2H, synchronise); roofline = the kernel against measured HBM
 peak; cpu_baseline = the unmodified reference SnakeEnv (oracle/_ref; the oracle port when that install is
 missing) on this box's host cores, run as the reference vectorises (one process per env).
+
+--dump-outputs DIR writes, after the timed region, what the last timed step returned to its caller for a fixed
+sample of DUMP_ENVS environments (seeded choice, sorted): obs.npy float32 [n, ns, oh, ow, 8], rewards.npy float64
+[n, ns], dones.npy float32 [n, ns].  The batch, the actions and the number of steps before the timed region are
+fixed by the arguments, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -28,13 +33,14 @@ sys.path.insert(0, ROOT)
 ENV_KW = dict(height=20, width=20, num_snakes=4, snake_length=3, vision_range=5, frame_stack=1)
 WORKLOAD = 'cfg5: 20x20, 4 snakes, len 3, vision_range 5, frame_stack 1, auto-reset, random actions'
 BURN_IN = 256          # steps before warm-up so the alive / reset mix is stationary (mean episode ~68)
-CLOCK_RAMP_S = 1.0     # extra untimed stepping after the CPU legs so the GPU is back at its load clocks
+CLOCK_RAMP_S = 1.0     # untimed stepping after the CPU legs so the GPU is back at its load clocks
+DUMP_ENVS, DUMP_SEED = 2048, 0     # --dump-outputs sample: 2048 x 3872 float32 observations = 32 MB
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=2000)
+    ap.add_argument('--steps', type=int, default=2000, help='timed steps')
     ap.add_argument('--warmup', type=int, default=100)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--envs-per-gpu', type=int, default=1 << 20)
@@ -45,7 +51,28 @@ def parse():
     ap.add_argument('--cpu-seconds', type=float, default=12.0)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-configs', action='store_true', help='skip the per-config block (cfg1-cfg4, strong scaling)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the last timed step\'s obs / rewards / dones of a fixed sample of environments '
+                         'as DIR/<name>.npy (rank 0)')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
+    return args
+
+
+def dump_outputs(out_dir, obs, rew, done):
+    """The caller-visible outputs of one step (obs uint8, rewards float64, dones bool, all [N, ns, ...] on the
+    device) for a seeded sample of environments, as .npy files in float32 / float64."""
+    import numpy as np
+    import torch
+    N = obs.shape[0]
+    idx = np.sort(np.random.RandomState(DUMP_SEED).choice(N, size=min(N, DUMP_ENVS), replace=False))
+    sel = torch.as_tensor(idx, device=obs.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x, dtype in (('obs', obs, np.float32), ('rewards', rew, np.float64), ('dones', done, np.float32)):
+        np.save(os.path.join(out_dir, name + '.npy'), x.index_select(0, sel).cpu().numpy().astype(dtype))
 
 
 # ------------------------------------------------------------------------------ CPU legs
@@ -196,28 +223,38 @@ def ours(args):
         N = args.envs_total // world
     else:
         N = args.envs_per_gpu
-    batch = SnakeBatch(N, device=local, seed=0, rng='philox', auto_reset=True, env_id_offset=rank * N, **ENV_KW)
+    def make_batch():
+        return SnakeBatch(N, device=local, seed=0, rng='philox', auto_reset=True, env_id_offset=rank * N, **ENV_KW)
     gen = torch.Generator(device=dev).manual_seed(1234 + rank)
     # A short action cycle would trap snakes in closed orbits (net turn of the cycle != 0 closes the
     # path after 4 cycles) and empty the workload of deaths and resets; 509 distinct tensors make the
     # cycle far longer than any snake lives (mean episode ~70 steps).
     NPOOL = 509
     pool = list(torch.randint(0, 3, (NPOOL, N, ns), dtype=torch.uint8, device=dev, generator=gen).unbind(0))   # one launch
+    # The CPU baseline legs above leave the GPU idle for ~20 s and it drops to its idle clocks; a quarter of a second
+    # of burn-in does not always bring the memory clock back (seen: 1.02 ms per step instead of 0.87).  Step for about
+    # a second of wall time first, on a batch that is then thrown away: the step count of a wall-time loop varies
+    # from run to run, and the measured batch must start from the same state every run.
+    batch = make_batch()
+    batch.reset()
+    t_ramp, step_no = time.perf_counter(), 0
+    while time.perf_counter() - t_ramp < CLOCK_RAMP_S:
+        for _ in range(64):
+            batch.step(pool[step_no % NPOOL], want_info=False)
+            step_no += 1
+        torch.cuda.synchronize()
+    # Creating and resetting the measured batch idles the GPU for a few milliseconds only, and its burn-in and warm-up
+    # (>= 356 steps, ~0.27 s at the default size) run back to back into the timed region; on a B200 (1000 W limit) this
+    # order measured the same step time as ramping the measured batch itself (0.7675-0.7685 ms against 0.7676-0.7677).
+    batch.close()
+    del batch
+    batch = make_batch()
     batch.reset()
     step_no = 0
     for t in range(BURN_IN + args.warmup):
         batch.step(pool[step_no % NPOOL], want_info=False)
         step_no += 1
     torch.cuda.synchronize()
-    # The CPU baseline legs above leave the GPU idle for ~20 s and it drops to its idle clocks; a quarter of a second
-    # of burn-in does not always bring the memory clock back (seen: 1.02 ms per step instead of 0.87).  Keep stepping
-    # for about a second of wall time before the timed region (these are extra warm-up steps, not timed).
-    t_ramp = time.perf_counter()
-    while time.perf_counter() - t_ramp < CLOCK_RAMP_S:
-        for _ in range(64):
-            batch.step(pool[step_no % NPOOL], want_info=False)
-            step_no += 1
-        torch.cuda.synchronize()
 
     sampler = ClockSampler(local)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -229,12 +266,15 @@ def ours(args):
     torch.cuda.cudart().cudaProfilerStart()
     ev0.record()
     for t in range(args.steps):
-        batch.step(pool[(step_no + t) % NPOOL], want_info=False)   # one kernel launch per step, current stream
+        last = batch.step(pool[(step_no + t) % NPOOL], want_info=False)   # one kernel launch per step, current stream
     ev1.record()
     torch.cuda.synchronize()
     torch.cuda.cudart().cudaProfilerStop()
     sampler.stop_flag.set()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last[:3])
+    del last
     if world > 1:
         dist.barrier()
         tms = torch.tensor([ms], device=dev, dtype=torch.float64)

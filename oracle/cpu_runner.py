@@ -12,6 +12,7 @@ Used only by bench.py's `cpu_baseline` leg and its `--impl reference` arm.  Two 
 Either way the run is shaped like the reference's vectorisation: one OS process per environment
 (wrappers.py:211-212), reset on all(done) (wrappers.py:141-143), random actions, module-global NumPy RNG.
 """
+import json
 import multiprocessing as mp
 import os
 import sys
@@ -32,6 +33,28 @@ def usable_cores():
 
 def reference_available():
     return os.path.exists(os.path.join(REF_DIR, 'marlenv', 'envs', 'snake_env.py'))
+
+
+def reference_checkout():
+    """Where the original project's checkout is looked for: SNK_REFERENCE_DIR, else the location BASELINE.json
+    records for it (reference_path)."""
+    if os.environ.get('SNK_REFERENCE_DIR'):
+        return os.environ['SNK_REFERENCE_DIR']
+    with open(os.path.join(os.path.dirname(HERE), 'BASELINE.json')) as f:
+        return json.load(f)['reference_path']
+
+
+def reference_search_path():
+    """The sys.path entry that holds the unmodified reference package `marlenv`: `marlenv/` of the original project's
+    checkout (reference_checkout()), else the install in oracle/_ref; None when neither is there.  A SNK_REFERENCE_DIR
+    that names no checkout is an error rather than a silent skip of every test that needs the original."""
+    path = os.path.join(reference_checkout(), 'marlenv')
+    if os.path.exists(os.path.join(path, 'marlenv', 'envs', 'snake_env.py')):
+        return path
+    if os.environ.get('SNK_REFERENCE_DIR'):
+        raise RuntimeError(f"SNK_REFERENCE_DIR={os.environ['SNK_REFERENCE_DIR']} is not a checkout of the original "
+                           'project (no marlenv/marlenv/envs/snake_env.py under it)')
+    return REF_DIR if reference_available() else None
 
 
 def make_reference_env(kw):
@@ -80,7 +103,7 @@ class CpuPool:
 
     def __init__(self, kw, procs=None, kind='port'):
         if kind == 'reference' and not reference_available():
-            raise RuntimeError('oracle/_ref is missing: run `make -C oracle ref` where /root/reference exists')
+            raise RuntimeError('oracle/_ref is missing: run `make -C oracle ref` where the original project is checked out')
         self.kind = kind
         self.procs = procs or usable_cores()
         ctx = mp.get_context('spawn')

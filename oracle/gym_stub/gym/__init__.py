@@ -1,7 +1,7 @@
 """Minimal structural stand-in for `gym` (TEST INFRASTRUCTURE ONLY).
 
 `gym` is not installed in this image and there is no network.  The reference
-environment (/root/reference/marlenv) needs gym only structurally (base classes,
+environment (marlenv/ of the original project) needs gym only structurally (base classes,
 spaces with .n/.shape/.sample(), the registry).  This stub lets the *unmodified*
 reference be imported so it can be used to generate golden vectors
 (tests/golden/make_golden.py) and to pin the oracle.  It implements none of the

@@ -9,12 +9,13 @@ loudly when its CUDA library is missing.
 Parity status: PINNED.  `tests/test_oracle_vs_golden.py` checks this file
 against trajectories recorded from the *unmodified* reference
 (`tests/golden/*.npz`, produced by `tests/golden/make_golden.py` which imports
-/root/reference behind `oracle/gym_stub`).  Where /root/reference is present the
-same test module additionally runs the reference live under the same
-`np.random.seed` and compares every step.
+the original project's checkout (SNK_REFERENCE_DIR, default BASELINE.json's
+reference_path) behind `oracle/gym_stub`).  Where the original is there (that
+checkout or its install in oracle/_ref) the same test module
+additionally runs it live under the same `np.random.seed` and compares every step.
 
-Reference lines each function follows (paths relative to
-/root/reference/marlenv/marlenv/):
+Reference lines each function follows (paths relative to marlenv/marlenv/ of the
+original project):
 
   spawn_candidates      core/grid_util.py:73-115   dfs_sweep_empty/_dfs_helper/_head_blocked
   OracleSnakeEnv.reset  envs/snake_env.py:131-159, 576-596; core/snake.py:53-74;

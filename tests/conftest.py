@@ -22,11 +22,13 @@ def _ensure_native_builds():
 def pytest_configure(config):
     _ensure_native_builds()
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "needs_reference: needs the original MARL-Snake project: its checkout at "
+                                       "SNK_REFERENCE_DIR or BASELINE.json's reference_path, or its install in oracle/_ref")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir('/root/reference/marlenv/marlenv')
+    from oracle.cpu_runner import reference_search_path
+    have_ref = reference_search_path() is not None
     try:
         import torch
         have_gpu = torch.cuda.is_available()
@@ -34,6 +36,6 @@ def pytest_collection_modifyitems(config, items):
         have_gpu = False
     for item in items:
         if 'needs_reference' in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason='/root/reference not present'))
+            item.add_marker(pytest.mark.skip(reason='original MARL-Snake not found (SNK_REFERENCE_DIR / BASELINE.json reference_path / oracle/_ref)'))
         if 'gpu' in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason='no CUDA device'))

@@ -1,11 +1,12 @@
 #!/usr/bin/env python
 """Generate golden trajectories by running the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the original project (tranthai189765/MARL-Snake) at SNK_REFERENCE_DIR or at BASELINE.json's
+reference_path:
 
     python tests/golden/make_golden.py
 
-Imports `marlenv.envs.snake_env.SnakeEnv` from /root/reference/marlenv behind the
+Imports `marlenv.envs.snake_env.SnakeEnv` from <checkout>/marlenv behind the
 structural gym stub in oracle/gym_stub, drives it with seeded random actions
 under the reference's own auto-reset rule (wrappers.py:138-146) and records, per
 step: actions, grid, rewards, dones, bit-packed observations, the signed
@@ -22,7 +23,10 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, 'oracle', 'gym_stub'))
-sys.path.insert(0, '/root/reference/marlenv')
+sys.path.insert(0, ROOT)
+from oracle.cpu_runner import reference_checkout  # noqa: E402
+REF = reference_checkout()
+sys.path.insert(0, os.path.join(REF, 'marlenv'))
 
 import gym  # noqa: E402  (the stub)
 import marlenv  # noqa: E402,F401  (registers Snake-v1)
@@ -30,7 +34,7 @@ from marlenv.core.snake import Snake, Direction  # noqa: E402
 from marlenv.core.grid_util import dfs_sweep_empty, make_grid, make_grid_from_txt  # noqa: E402
 import marlenv.envs.snake_env as ref_snake_env  # noqa: E402
 
-ASSETS = '/root/reference/marlenv/marlenv/assets'
+ASSETS = os.path.join(REF, 'marlenv', 'marlenv', 'assets')
 
 
 def load_asset_map(name, mapper=None):

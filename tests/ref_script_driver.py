@@ -7,7 +7,7 @@ backend   'ours'       repo root first on sys.path: `from marlenv.marlenv.wrappe
                        CUDA step path behind the C ABI.  Needs a GPU.
           'reference'  the unmodified reference package from oracle/_ref behind oracle/gym_stub.  CPU only; this leg
                        exists so that the harness itself (stubs, shortened configs) is proven on the reference first.
-scenario  'test_env'   /root/reference/test_env.py as __main__: make_snake -> RenderGUI -> reset -> render/step until
+scenario  'test_env'   the original's test_env.py as __main__: make_snake -> RenderGUI -> reset -> render/step until
                        all(done) -> close
           'train_dqn'  train_dqn.Trainer(config).train() for a few short episodes including update_model(),
                        target-net sync and checkpoint save/delete (train_dqn.py:187-199, 228-381), then
@@ -15,8 +15,8 @@ scenario  'test_env'   /root/reference/test_env.py as __main__: make_snake -> Re
           'train_ga'   train_ga.run_neat's environment loop: make_snake as :263-274, FeatureExtractor on the DQN
                        checkpoint written by the train_dqn scenario, eval_genomes (:224-258) on two genomes
 
-The scripts are read from oracle/_ref/scripts/ (copied there, git-ignored, by `make -C oracle ref`; /root/reference does
-not exist on the GPU box).  Third-party packages that are absent from the image (`neat`; cv2 windows on a headless box)
+The scripts are read from oracle/_ref/scripts/ (copied there, git-ignored, by `make -C oracle ref` from the
+original's checkout).  Third-party packages that are absent from the image (`neat`; cv2 windows on a headless box)
 are replaced by inert stand-ins -- none of them touches the environment.
 Prints one JSON line with what happened; exit code 0 = the script ran to completion.
 """

@@ -1,5 +1,5 @@
 """What the compact record layout rests on (DESIGN.md section 3), checked on the CPU against the oracle and -- where
-/root/reference exists -- against the unmodified reference itself:
+the original project is there (oracle.cpu_runner.reference_search_path) -- against the unmodified reference itself:
 
   after reset() and after every step(), the grid is exactly   wall layout + FRUIT cells + the bodies of the LIVE snakes
   (HEAD at coords[0], TAIL at coords[-1], BODY between), and the number of fruit cells never exceeds
@@ -14,6 +14,7 @@ import sys
 import numpy as np
 import pytest
 
+from oracle.cpu_runner import reference_search_path
 from oracle.snake_oracle import OracleSnakeEnv
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -78,16 +79,20 @@ def test_oracle_grid_is_walls_fruits_and_live_bodies(kw):
 @pytest.mark.needs_reference
 @pytest.mark.parametrize('kw', SHAPES, ids=lambda k: f"{k['height']}x{k['width']}x{k['num_snakes']}")
 def test_reference_grid_is_walls_fruits_and_live_bodies(kw):
-    sys.path.insert(0, '/root/reference/marlenv')
+    ref_pkg = reference_search_path()
+    sys.path.insert(0, ref_pkg)
     sys.path.insert(0, os.path.join(ROOT, 'oracle', 'gym_stub'))
+    for m in [m for m in sys.modules if m == 'gym' or m.startswith('gym.') or m == 'marlenv' or m.startswith('marlenv.')]:
+        del sys.modules[m]                   # this repository's `marlenv` import shim may already be loaded
     try:
         import gym
         import marlenv  # noqa: F401  (registers Snake-v1)
+        assert marlenv.__file__.startswith(ref_pkg), marlenv.__file__
         for seed in range(3):
             drive(lambda: gym.make('Snake-v1', **kw),
                   lambda e: (e.grid, [list(s.coords) for s in e.snakes], [s.alive for s in e.snakes]), kw, seed, 300)
     finally:
         sys.path.remove(os.path.join(ROOT, 'oracle', 'gym_stub'))
-        sys.path.remove('/root/reference/marlenv')
+        sys.path.remove(ref_pkg)
         for m in [m for m in sys.modules if m == 'gym' or m.startswith('gym.') or m == 'marlenv' or m.startswith('marlenv.')]:
             del sys.modules[m]

@@ -1,12 +1,16 @@
 """Pins oracle/snake_oracle.py to the reference: committed golden vectors (always) and the
-live reference under the same np.random seed (when /root/reference is present)."""
+live reference under the same np.random seed (where the original project is there: its checkout at
+SNK_REFERENCE_DIR or BASELINE.json's reference_path, or its install in oracle/_ref)."""
+import functools
+import hashlib
 import os
 import sys
 
 import numpy as np
 import pytest
 
-from golden_util import ROLLOUTS, Rollout, load_map_spawn_tables, load_scenarios, load_spawn_tables, unpack_obs
+from golden_util import GOLDEN_DIR, ROLLOUTS, Rollout, load_map_spawn_tables, load_scenarios, load_spawn_tables, unpack_obs
+from oracle.cpu_runner import reference_search_path
 from oracle.snake_oracle import (CoopOracleSnakeEnv, OracleSnakeEnv, ReplayDraws, RecordingDraws, TURN,
                                  spawn_candidates, competition_rank)
 
@@ -95,83 +99,22 @@ def test_reward_dict_keys_and_action_errors():
         env.step([0, 3])
 
 
-# ------------------------------------------------------------------ live reference (container only)
-def _compare_with_live_reference(kw, env_id='Snake-v1', steps=400, n_actions=3, reset_on_done=True):
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    sys.path.insert(0, os.path.join(root, 'oracle', 'gym_stub'))
-    sys.path.insert(1, '/root/reference/marlenv')
-    try:
-        import gym
-        import marlenv  # noqa: F401
-        ns = kw['num_snakes']
-        acts = np.random.RandomState(5).randint(0, n_actions, size=(steps, ns))
-        walls = kw.get('wall_map')
-        ref_kw = {k: v for k, v in kw.items() if k != 'wall_map'}
-        if walls is not None:     # the reference has no map parameter: its reset() gets the layout from `make_grid`
-            import marlenv.envs.snake_env as ref_snake_env
-            ref_snake_env.make_grid = lambda *a, **k: np.asarray(walls).copy()
-
-        def run(make):
-            np.random.seed(42)
-            env = make()
-            out = [env.reset()]
-            for a in acts:
-                o, r, d, info = env.step([int(x) for x in a])
-                if all(d) and reset_on_done:
-                    o = env.reset()
-                out.append((o, list(r), list(d), sorted(info.keys()),
-                            [list(np.asarray(info[k], dtype=np.float64)) for k in sorted(info.keys())],
-                            np.asarray(env.grid).copy()))
-            return out
-
-        cls = CoopOracleSnakeEnv if env_id == 'SnakeCoop-v1' else OracleSnakeEnv
-        ref = run(lambda: gym.make(env_id, **ref_kw))
-        mine = run(lambda: cls(**kw))
-        assert np.array_equal(ref[0], mine[0])
-        for t, (a, b) in enumerate(zip(ref[1:], mine[1:])):
-            assert np.array_equal(a[0], b[0]), (t, kw)
-            assert a[1] == b[1] and a[2] == b[2] and a[3] == b[3] and a[4] == b[4], (t, kw)
-            assert np.array_equal(a[5], b[5]), (t, kw)
-    finally:
-        sys.path.remove(os.path.join(root, 'oracle', 'gym_stub'))
-        sys.path.remove('/root/reference/marlenv')
-        for m in [m for m in sys.modules if m == 'gym' or m.startswith('gym.') or m == 'marlenv'
-                  or m.startswith('marlenv.')]:
-            del sys.modules[m]
-
-
-@pytest.mark.needs_reference
-@pytest.mark.parametrize('kw', [
+# ------------------------------------------------------------------ the cases run against the live reference
+SAME_SEED = [
     dict(height=20, width=20, num_snakes=4, snake_length=3, vision_range=5),
     dict(height=12, width=9, num_snakes=3, snake_length=4, vision_range=2, frame_stack=3,
          reward_dict={'fruit': 1.5, 'kill': 2.0, 'lose': -3.0, 'win': 4.0, 'time': 0.1}),
     dict(height=8, width=8, num_snakes=5, snake_length=2, num_fruits=7, max_episode_steps=25),
-])
-def test_same_seed_as_live_reference(kw):
-    _compare_with_live_reference(kw)
-
-
-@pytest.mark.needs_reference
-@pytest.mark.parametrize('name,kw', [
+]
+WALL_MAPS = [
     ('12x12', dict(num_snakes=3, snake_length=4, vision_range=3, frame_stack=2)),
     ('20x20_cross', dict(num_snakes=4, snake_length=3, vision_range=5)),
-])
-def test_custom_wall_map_same_seed_as_live_reference(name, kw):
-    """SURVEY N4: the oracle on a custom wall layout against the reference whose reset() is handed the same layout."""
-    walls, _, _ = load_map_spawn_tables()[name]
-    _compare_with_live_reference(dict(height=walls.shape[0], width=walls.shape[1], wall_map=walls.astype(np.int64), **kw),
-                                 steps=250)
-
-
-@pytest.mark.needs_reference
-@pytest.mark.parametrize('kw', [
+]
+FINISHED = [
     dict(height=9, width=9, num_snakes=3, snake_length=3, vision_range=2, max_episode_steps=6, num_fruits=2),
     dict(height=8, width=10, num_snakes=2, snake_length=2, frame_stack=2, num_fruits=1),
-])
-def test_stepping_a_finished_env_like_the_live_reference(kw):
-    """No reset after the episode ends (SURVEY E1, probe g3): the reference keeps stepping -- capped episodes
-    move on, dead snakes return 0 / True, info is emitted again every step."""
-    _compare_with_live_reference(kw, steps=60, reset_on_done=False)
+]
+LIVE_GOLDEN = os.path.join(GOLDEN_DIR, 'live_cases.npz')
 
 
 def small_fuzz_configs(n, seed):
@@ -195,6 +138,139 @@ def small_fuzz_configs(n, seed):
                                'time': -0.001 * rng.randint(0, 5)})
         out.append((kw, ['Snake-v1', 'Snake-v1', 'SnakeCoop-v1'][rng.randint(0, 3)]))
     return out
+
+
+def wall_map_kw(name, kw):
+    walls, _, _ = load_map_spawn_tables()[name]
+    return dict(height=walls.shape[0], width=walls.shape[1], wall_map=walls.astype(np.int64), **kw)
+
+
+@functools.lru_cache(maxsize=None)
+def live_cases():
+    """name -> (kw, env_id, steps, n_actions, reset_on_done) of every case the live-reference tests run."""
+    cases = {f'same_seed_{i}': (kw, 'Snake-v1', 400, 3, True) for i, kw in enumerate(SAME_SEED)}
+    for name, kw in WALL_MAPS:
+        cases[f'wall_map_{name}'] = (wall_map_kw(name, kw), 'Snake-v1', 250, 3, True)
+    for i, kw in enumerate(FINISHED):
+        cases[f'finished_{i}'] = (kw, 'Snake-v1', 60, 3, False)
+    for i, (kw, env_id) in enumerate(small_fuzz_configs(24, 777)):
+        cases[f'fuzz_{i}'] = (kw, env_id, 150, 5 if kw['observer'] == 'human' else 3, True)
+    return cases
+
+
+def trajectory(make, ns, steps, n_actions=3, reset_on_done=True):
+    """The live comparison's protocol: np.random.seed(42), make, reset, then `steps` steps of RandomState(5) actions,
+    resetting on all(done) when reset_on_done.  Returns [reset obs, (obs, rewards, dones, info keys, info values,
+    grid) per step]."""
+    acts = np.random.RandomState(5).randint(0, n_actions, size=(steps, ns))
+    np.random.seed(42)
+    env = make()
+    out = [env.reset()]
+    for a in acts:
+        o, r, d, info = env.step([int(x) for x in a])
+        if all(d) and reset_on_done:
+            o = env.reset()
+        out.append((o, list(r), list(d), sorted(info.keys()),
+                    [list(np.asarray(info[k], dtype=np.float64)) for k in sorted(info.keys())],
+                    np.asarray(env.grid).copy()))
+    return out
+
+
+def digests(traj):
+    """8-byte SHA-256 prefixes, one row for the reset observation and one per step over (obs, rewards, dones,
+    info, grid) in fixed dtypes: a whole trajectory pinned in a few bytes per step."""
+    def h(*arrays, text=''):
+        m = hashlib.sha256(text.encode())
+        for x in arrays:
+            m.update(repr(x.shape).encode() + x.tobytes())
+        return np.frombuffer(m.digest()[:8], np.uint8)
+    rows = [h(np.asarray(traj[0], np.uint8))]
+    for o, r, d, keys, vals, grid in traj[1:]:
+        rows.append(h(np.asarray(o, np.uint8), np.asarray(r, np.float64), np.asarray(d, np.uint8),
+                      np.asarray([x for v in vals for x in v], np.float64), np.asarray(grid, np.int64),
+                      text=repr([(k, len(v)) for k, v in zip(keys, vals)])))
+    return np.stack(rows)
+
+
+def oracle_record(name):
+    """The oracle's trajectory of one live case as stored in tests/golden/live_cases.npz."""
+    kw, env_id, steps, n_actions, reset_on_done = live_cases()[name]
+    cls = CoopOracleSnakeEnv if env_id == 'SnakeCoop-v1' else OracleSnakeEnv
+    traj = trajectory(lambda: cls(**kw), kw['num_snakes'], steps, n_actions, reset_on_done)
+    return {'digest': digests(traj), 'rewards': np.asarray([t[1] for t in traj[1:]], np.float64),
+            'dones': np.asarray([t[2] for t in traj[1:]], np.uint8)}
+
+
+@pytest.mark.parametrize('name', sorted(live_cases()))
+def test_live_reference_cases_against_stored_trajectories(name):
+    """Every case of the live-reference tests below, on every run: the oracle against the trajectory stored for it
+    in tests/golden/live_cases.npz (made by tests/golden/make_live_cases.py from this oracle; the live tests check
+    the oracle against the original project wherever it is installed)."""
+    want = np.load(LIVE_GOLDEN)
+    got = oracle_record(name)
+    assert np.array_equal(got['rewards'], want[f'{name}_rewards']), name
+    assert np.array_equal(got['dones'], want[f'{name}_dones']), name
+    bad = np.flatnonzero((got['digest'] != want[f'{name}_digest']).any(1))
+    assert got['digest'].shape == want[f'{name}_digest'].shape and bad.size == 0, \
+        f'{name}: first differing row {bad[:1]} (row 0 = reset, row t + 1 = step t)'
+
+
+# ------------------------------------------------------------------ live reference (reference_search_path)
+def _drop_gym_and_marlenv():
+    for m in [m for m in sys.modules if m == 'gym' or m.startswith('gym.') or m == 'marlenv' or m.startswith('marlenv.')]:
+        del sys.modules[m]
+
+
+def _compare_with_live_reference(kw, env_id='Snake-v1', steps=400, n_actions=3, reset_on_done=True):
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    ref_pkg = reference_search_path()
+    sys.path.insert(0, os.path.join(root, 'oracle', 'gym_stub'))
+    sys.path.insert(1, ref_pkg)
+    _drop_gym_and_marlenv()                  # this repository's `marlenv` import shim may already be loaded
+    try:
+        import gym
+        import marlenv  # noqa: F401
+        assert marlenv.__file__.startswith(ref_pkg), marlenv.__file__
+        walls = kw.get('wall_map')
+        ref_kw = {k: v for k, v in kw.items() if k != 'wall_map'}
+        if walls is not None:     # the reference has no map parameter: its reset() gets the layout from `make_grid`
+            import marlenv.envs.snake_env as ref_snake_env
+            ref_snake_env.make_grid = lambda *a, **k: np.asarray(walls).copy()
+
+        cls = CoopOracleSnakeEnv if env_id == 'SnakeCoop-v1' else OracleSnakeEnv
+        ns = kw['num_snakes']
+        ref = trajectory(lambda: gym.make(env_id, **ref_kw), ns, steps, n_actions, reset_on_done)
+        mine = trajectory(lambda: cls(**kw), ns, steps, n_actions, reset_on_done)
+        assert np.array_equal(ref[0], mine[0])
+        for t, (a, b) in enumerate(zip(ref[1:], mine[1:])):
+            assert np.array_equal(a[0], b[0]), (t, kw)
+            assert a[1] == b[1] and a[2] == b[2] and a[3] == b[3] and a[4] == b[4], (t, kw)
+            assert np.array_equal(a[5], b[5]), (t, kw)
+    finally:
+        sys.path.remove(os.path.join(root, 'oracle', 'gym_stub'))
+        sys.path.remove(ref_pkg)
+        _drop_gym_and_marlenv()
+
+
+@pytest.mark.needs_reference
+@pytest.mark.parametrize('kw', SAME_SEED)
+def test_same_seed_as_live_reference(kw):
+    _compare_with_live_reference(kw)
+
+
+@pytest.mark.needs_reference
+@pytest.mark.parametrize('name,kw', WALL_MAPS)
+def test_custom_wall_map_same_seed_as_live_reference(name, kw):
+    """SURVEY N4: the oracle on a custom wall layout against the reference whose reset() is handed the same layout."""
+    _compare_with_live_reference(wall_map_kw(name, kw), steps=250)
+
+
+@pytest.mark.needs_reference
+@pytest.mark.parametrize('kw', FINISHED)
+def test_stepping_a_finished_env_like_the_live_reference(kw):
+    """No reset after the episode ends (SURVEY E1, probe g3): the reference keeps stepping -- capped episodes
+    move on, dead snakes return 0 / True, info is emitted again every step."""
+    _compare_with_live_reference(kw, steps=60, reset_on_done=False)
 
 
 @pytest.mark.needs_reference

@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DRIVER = os.path.join(ROOT, 'tests', 'ref_script_driver.py')
 SCRIPTS = os.path.join(ROOT, 'oracle', '_ref', 'scripts')
 needs_scripts = pytest.mark.skipif(not os.path.exists(os.path.join(SCRIPTS, 'train_dqn.py')),
-                                   reason='oracle/_ref/scripts absent (make -C oracle ref needs /root/reference)')
+                                   reason='oracle/_ref/scripts absent (make -C oracle ref needs the original checkout)')
 SCENARIOS = ['test_env', 'train_dqn', 'train_ga']
 
 
