@@ -198,6 +198,11 @@ int snk_reset_host(snk_env* env, uint8_t* obs_host);
 int snk_step_host_bits(snk_env* env, const uint8_t* actions_host, uint8_t* bits_host,
                        double* rewards_host, uint8_t* dones_host);
 
+/* Work on this handle's buffers that the caller issued on `stream` outside the library -- a CUDA graph replay of
+ * captured device-pointer calls, for instance -- must be reported here before the next *_host call, which then
+ * waits for it on the device as it does for the library's own device-pointer calls.  Enqueues nothing. */
+int snk_note_stream(snk_env* env, void* stream);
+
 enum { SNK_XFER_RAW = 0, SNK_XFER_PACKED = 1 };
 /* threads: widening threads of the packed transport, 0 = one per core this process may run on (<= 32) */
 int snk_set_host_transport(snk_env* env, int mode, int threads);

@@ -69,6 +69,7 @@ PROTOTYPES = {
                                      C.POINTER(SnkStepExtra)]),
     'snk_step_host_bits': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     'snk_reset_host': (C.c_int, [C.c_void_p, C.c_void_p]),
+    'snk_note_stream': (C.c_int, [C.c_void_p, C.c_void_p]),
     'snk_set_host_transport': (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     'snk_get_host_transport': (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     'snk_pack_obs': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

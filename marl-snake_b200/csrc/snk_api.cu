@@ -395,6 +395,12 @@ static int own_stream_after_user_work(snk_env* h) {
   return SNK_OK;
 }
 
+extern "C" int snk_note_stream(snk_env* h, void* stream) {
+  if (!h) return fail(SNK_E_INVALID, "null handle");
+  note_user_stream(h, (cudaStream_t)stream);
+  return SNK_OK;
+}
+
 static int reset_impl(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, uint8_t* bits_dev, cudaStream_t stream) {
   if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
   KParams p = base_params(h);

@@ -101,9 +101,12 @@ class SnakeBatch:
                                    self._ep_kills.data_ptr())
         self.observation_space = Box(0, 1, (N,) + self.obs_shape, np.uint8)
         self.action_space = Discrete(len(self.action_dict))
-        self._has_obs = False            # self._obs holds the current observation of every env
-        self._rollout_alive = None       # rollout.collect's (alive, episode age) cache; dropped by any other mutation
-        self._rollout_age = None
+        # Every call that steps, resets, restores or replays the shard bumps `_mutations`; rollout.collect keeps its
+        # (alive, episode age) cache only while the counter still has the value it stored.  `_obs_stale` is None while
+        # self._obs holds the current observation of every env, else the name of the call that left it behind.
+        self._mutations = 0
+        self._obs_stale = 'construction (no reset yet)'
+        self._rollout_alive = self._rollout_age = self._rollout_mark = None
 
     # ---- lifecycle ---------------------------------------------------------------------------------
     def close(self):
@@ -119,6 +122,13 @@ class SnakeBatch:
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _mutated(self, obs_stale):
+        """Bookkeeping after a call that changed the shard: obs_stale None = self._obs is now current for every env,
+        False = whatever it was before (still current if it was), else the name of the call that outdated it."""
+        self._mutations += 1
+        if obs_stale is not False:
+            self._obs_stale = obs_stale
 
     # ---- hot path ----------------------------------------------------------------------------------
     def _bits_buffer(self):
@@ -140,8 +150,8 @@ class SnakeBatch:
             else:
                 out = self._obs
                 check(lib.snk_reset(self._h, _ptr(mask), _ptr(out), self._stream()))
-                self._has_obs = True
-        self._rollout_alive = None
+        # a masked reset rewrites the observation of the selected envs only: the others keep theirs
+        self._mutated('reset(bits=True)' if bits else (None if mask is None else False))
         return out.clone() if copy else out
 
     def step_bits(self, actions, copy=False, want_info=True):
@@ -154,6 +164,7 @@ class SnakeBatch:
         out = self._bits_buffer()
         check(lib.snk_step_bits(self._h, _ptr(actions), _ptr(out), _ptr(self._rew), _ptr(self._done),
                                 C.byref(self._extra) if want_info else None, self._stream()))
+        self._mutated('step_bits')
         info = {}
         if want_info:
             info = dict(finished=self._fin.view(torch.bool), rank=self._rank, episode_scores=self._ep_scores,
@@ -174,7 +185,7 @@ class SnakeBatch:
             raise ValueError('actions must be a contiguous uint8 CUDA tensor of shape [num_envs, num_snakes]')
         check(lib.snk_step(self._h, _ptr(actions), _ptr(self._obs if want_obs else None), _ptr(self._rew),
                            _ptr(self._done), C.byref(self._extra) if want_info else None, self._stream()))
-        self._has_obs, self._rollout_alive = self._has_obs and want_obs, None
+        self._mutated(None if want_obs else 'step(want_obs=False)')
         info = {}
         if want_info:
             info = dict(finished=self._fin.view(torch.bool), rank=self._rank, episode_scores=self._ep_scores,
@@ -200,6 +211,11 @@ class SnakeBatch:
             rewards = torch.empty((T, N, ns), dtype=torch.float64, device=self.device)
         if dones is None:
             dones = torch.empty((T, N, ns), dtype=torch.uint8, device=self.device)
+        for name, buf, dtype in (('rewards', rewards, torch.float64), ('dones', dones, torch.uint8)):
+            if buf.dtype != dtype or buf.device != self.device or not buf.is_contiguous() \
+                    or tuple(buf.shape) != (T, N, ns):
+                raise ValueError(f'{name} must be a contiguous {str(dtype)[6:]} CUDA tensor of shape '
+                                 '[T, num_envs, num_snakes]')
         every = None
         for name, buf, shape in (('obs', obs, self.obs_shape), ('bits', bits, self.bits_shape)):
             if buf is None:
@@ -217,11 +233,13 @@ class SnakeBatch:
             every = e
         extra = None
         if finished is not None:
-            if tuple(finished.shape) != (T, N) or finished.dtype != torch.uint8 or not finished.is_contiguous():
+            if tuple(finished.shape) != (T, N) or finished.dtype != torch.uint8 or finished.device != self.device \
+                    or not finished.is_contiguous():
                 raise ValueError('finished must be a contiguous uint8 CUDA tensor of shape [T, N]')
             extra = SnkStepExtra(finished.data_ptr(), 0, 0, 0, 0, 0)
         check(lib.snk_step_many(self._h, T, _ptr(actions), _ptr(obs), _ptr(bits), int(bool(every)), _ptr(rewards),
                                 _ptr(dones), C.byref(extra) if extra is not None else None, self._stream()))
+        self._mutated('step_many')
         return obs, rewards, dones, bits
 
     def step_host(self, actions, obs, rewards, dones):
@@ -230,16 +248,32 @@ class SnakeBatch:
         check(lib.snk_step_host(self._h, C.c_void_p(actions.data_ptr()),
                                 C.c_void_p(obs.data_ptr()) if obs is not None else C.c_void_p(0),
                                 C.c_void_p(rewards.data_ptr()), C.c_void_p(dones.data_ptr())))
+        self._mutated('step_host')
+
+    def step_host_info(self, actions, obs, rewards, dones, finished=None, rank=None, episode_scores=None,
+                       episode_steps=None, episode_fruits=None, episode_kills=None):
+        """step_host plus the terminal info arrays of step() (snk_step_host_info), each into a HOST buffer of the same
+        shape (finished uint8 [N], rank / episode_steps / _fruits / _kills int32 [N, ns], episode_scores float64
+        [N, ns]); any of them may be None.  Entries of envs that did not finish are unspecified."""
+        def hp(x):
+            return x.data_ptr() if x is not None else None
+        xh = SnkStepExtra(hp(finished), hp(rank), hp(episode_scores), hp(episode_steps), hp(episode_fruits),
+                          hp(episode_kills))
+        check(lib.snk_step_host_info(self._h, C.c_void_p(actions.data_ptr()),
+                                     C.c_void_p(obs.data_ptr()) if obs is not None else C.c_void_p(0),
+                                     C.c_void_p(rewards.data_ptr()), C.c_void_p(dones.data_ptr()), C.byref(xh)))
+        self._mutated('step_host_info')
 
     def step_host_bits(self, actions, bits, rewards, dones):
         """As step_host, but `bits` (uint8, obs shape with the last dimension divided by 8) receives channel
         bits -- one byte per (cell, frame) -- and nothing is widened on the host."""
         check(lib.snk_step_host_bits(self._h, C.c_void_p(actions.data_ptr()), C.c_void_p(bits.data_ptr()),
                                      C.c_void_p(rewards.data_ptr()), C.c_void_p(dones.data_ptr())))
+        self._mutated('step_host_bits')
 
     def reset_host(self, obs):
         check(lib.snk_reset_host(self._h, C.c_void_p(obs.data_ptr()) if obs is not None else C.c_void_p(0)))
-        self._host_reset_done = True
+        self._mutated('reset_host')
 
     def set_host_transport(self, mode, threads=0):
         """How step_host / reset_host move the observation block over PCIe: 'raw' (one D2H of the NHWC
@@ -303,7 +337,7 @@ class SnakeBatch:
         view = SnkStateView(**{k: v.data_ptr() for k, v in keep.items()}, max_cells=cells.shape[-1])
         check(lib.snk_set_state(self._h, C.byref(view), _ptr(self._obs), self._stream()))
         torch.cuda.current_stream(self.device).synchronize()      # `keep` must outlive the kernels
-        self._has_obs, self._rollout_alive = True, None
+        self._mutated(None)
         return self._obs
 
     def save_checkpoint(self):
@@ -317,7 +351,7 @@ class SnakeBatch:
     def load_checkpoint(self, blob):
         blob = np.ascontiguousarray(blob, dtype=np.uint8)
         check(lib.snk_checkpoint_load(self._h, blob.ctypes.data_as(C.c_void_p), blob.size))
-        self._has_obs, self._rollout_alive = False, None
+        self._mutated('load_checkpoint')
 
     def set_replay(self, draws_per_env):
         """draws_per_env: sequence of N int arrays -- recorded draw outputs in consumption order."""

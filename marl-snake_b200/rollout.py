@@ -7,7 +7,11 @@ epsilon-greedy straight from the device observation, transitions written into a 
 host synchronisation per step.  Everything here is torch tensor plumbing around `SnakeBatch.step`; the
 game itself stays in the CUDA library.
 """
+import ctypes as C
+
 import torch
+
+from ._lib import check, lib
 
 
 def epsilon_greedy(q_values, epsilon, generator=None):
@@ -81,6 +85,7 @@ class GraphedSteps:
         stream = torch.cuda.Stream(device=actions.device)
         stream.wait_stream(torch.cuda.current_stream(actions.device))
         self.graph = torch.cuda.CUDAGraph()
+        mark = (batch._mutations, batch._obs_stale)
         with torch.cuda.stream(stream):
             with torch.cuda.graph(self.graph, stream=stream):
                 for t in range(self.T):
@@ -89,11 +94,17 @@ class GraphedSteps:
                         self.rewards[t].copy_(rew)
                         self.dones[t].copy_(done)
         torch.cuda.current_stream(actions.device).wait_stream(stream)
+        batch._mutations, batch._obs_stale = mark              # capturing ran nothing
         self.obs = obs
 
     def replay(self):
         """Run the T captured steps (asynchronous; outputs are valid on the current stream afterwards)."""
+        b = self.batch
+        stream = torch.cuda.current_stream(b.device)
         self.graph.replay()
+        # the replayed kernels bypass the library: report the stream so that a following host-buffer call waits for them
+        check(lib.snk_note_stream(b._h, C.c_void_p(stream.cuda_stream)))
+        b._mutated(None)
         return self.obs, self.rewards, self.dones
 
 
@@ -115,12 +126,19 @@ def collect(batch, q_net, steps, buffer=None, epsilon=0.1, generator=None, early
         trainer's `step < MAX_STEPS_PER_EPISODE` loop condition does (:275, 270) -- one masked reset launch per step.
 
     The alive mask and the per-env episode age are read back from the device state (`snk_get_state`) when the batch
-    was touched by anything else since the last call, so consecutive calls continue the same rollout.
+    was stepped, reset, restored or replayed by anything else since the last call, so consecutive calls continue the
+    same rollout.  The observations come from the batch's own buffer, which step(), full reset(), set_state() and
+    GraphedSteps.replay() keep current; after any other stepping or resetting call (step_bits, step_many, the
+    host-buffer calls, reset(bits=True), load_checkpoint, step(want_obs=False)) collect raises ValueError until
+    reset() or step() renders it again.  A batch that was never reset is reset by the first call.
     Returns the number of transitions written (a device scalar); nothing is copied to the host."""
     N, ns = batch.num_envs, batch.num_snakes
-    if not batch._has_obs:
+    if batch._obs_stale is not None:
+        if batch._mutations:
+            raise ValueError(f"collect: the batch's observation buffer is out of date after {batch._obs_stale}; "
+                             'call reset() or step() to restore it')
         batch.reset()
-    if batch._rollout_alive is None:            # first call, or the batch was reset / stepped / restored in between
+    if batch._rollout_mark != batch._mutations:  # first call, or the batch was changed by another call in between
         st = batch.get_state()
         batch._rollout_alive, batch._rollout_age = st['alive'].bool(), st['episode_length']
     obs = batch._obs
@@ -149,5 +167,5 @@ def collect(batch, q_net, steps, buffer=None, epsilon=0.1, generator=None, early
             cut = age >= max_steps
             obs = batch.reset(mask=cut)
             alive, age = alive | cut[:, None], torch.where(cut, torch.zeros_like(age), age)
-    batch._rollout_alive, batch._rollout_age = alive, age
+    batch._rollout_alive, batch._rollout_age, batch._rollout_mark = alive, age, batch._mutations
     return written
