@@ -216,6 +216,15 @@ int snk_pack_obs(snk_env* env, const uint8_t* obs_dev, uint8_t* bits_dev, size_t
  * _encode (snake_env.py:484-492).  threads <= 1: on the calling thread. */
 int snk_widen_bits_host(const uint8_t* bits_host, uint8_t* obs_host, size_t n_units, int threads);
 
+/* Device memory for an observation block: `bytes` on `device`, mapped for that device only.  Where the device
+ * supports generic memory compression and grants it, the block is a compressible allocation (cuMemCreate with
+ * CU_MEM_ALLOCATION_COMP_GENERIC): the 0/1 observation bytes are mostly zero, and compressed lines cost less DRAM
+ * traffic between L2 and HBM.  Kernels, copies and torch see ordinary device memory either way.  Otherwise the
+ * block comes from cudaMalloc.  *compressed_out = 1 when compression was granted, else 0.  Free with
+ * snk_free_obs, which synchronises the device first. */
+int snk_alloc_obs(int device, size_t bytes, void** ptr_out, int* compressed_out);
+int snk_free_obs(void* ptr);
+
 /* ---- parity / checkpoint interface ---------------------------------------------------------- */
 
 /* The reference's env.grid / env.snakes[i] of every environment.  A handle with compact records (the default for

@@ -74,6 +74,8 @@ PROTOTYPES = {
     'snk_get_host_transport': (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     'snk_pack_obs': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     'snk_widen_bits_host': (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int]),
+    'snk_alloc_obs': (C.c_int, [C.c_int, C.c_size_t, C.POINTER(C.c_void_p), C.POINTER(C.c_int)]),
+    'snk_free_obs': (C.c_int, [C.c_void_p]),
     'snk_get_state': (C.c_int, [C.c_void_p, C.POINTER(SnkStateView), C.c_void_p]),
     'snk_set_state': (C.c_int, [C.c_void_p, C.POINTER(SnkStateView), C.c_void_p, C.c_void_p]),
     'snk_checkpoint_bytes': (C.c_size_t, [C.c_void_p]),

@@ -1,4 +1,5 @@
 // snk_api.cu -- the C ABI declared in include/snk.h.
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -6,7 +7,9 @@
 #include <string.h>
 
 #include <cmath>
+#include <mutex>
 #include <new>
+#include <map>
 #include <vector>
 
 #include "../../include/snk.h"
@@ -18,6 +21,8 @@ using namespace snk;
 enum { XFER_RAW = 0, XFER_PACKED = 1, XFER_MAX_CHUNKS = 64 };
 
 static thread_local char g_err[512] = "";
+
+static bool in_compressible_block(const void* p);
 
 static int fail(int code, const char* fmt, ...) {
   va_list ap;
@@ -263,7 +268,8 @@ static int create_impl(const snk_config* c, const uint8_t* walls_host, snk_env**
   h->l2_keep = env_int("SNK_L2_KEEP", d.fs > 1 ? 1 : 0);
   h->l2_keep_frac = (float)env_int("SNK_L2_KEEP_PCT", 100) / 100.0f;
   {
-    // the uncapped-register instance of the warp-private kernel once the batch is many waves deep
+    // the uncapped-register instance of the warp-private kernel once the batch is many waves deep (a step that writes
+    // its observation into a compressible block runs the capped one all the same: see step_impl)
     const int64_t tiles = ((int64_t)d.N + EPW - 1) / EPW;
     h->bigreg = (!coop && tiles >= (int64_t)env_int("SNK_BIGREG_TILES", 24576)) ? 1 : 0;
   }
@@ -426,6 +432,10 @@ static int step_impl(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, u
     p.ep_steps = x->episode_steps; p.ep_fruits = x->episode_fruits; p.ep_kills = x->episode_kills;
   }
   p.vec16 = check_vec16(h, obs_dev);
+  // An observation block in compressible memory costs the step far less DRAM time, and the step is then bound by the
+  // latency of its rule phase: the 64-register instance, with twice the resident warps, is the faster one there
+  // (cfg5, 1 048 576 envs on a B200 at 1000 W: 0.671 ms against 0.758 ms uncapped; profiles/r03_retune.txt).
+  if (p.bigreg && obs_dev && in_compressible_block(obs_dev)) p.bigreg = 0;
   CU(launch_tile_kernel(p, h->threads, h->smem_bytes, stream));
   note_user_stream(h, stream);
   return SNK_OK;
@@ -755,6 +765,165 @@ extern "C" int snk_widen_bits_host(const uint8_t* bits_host, uint8_t* obs_host, 
   WidenPool pool(threads);
   pool.submit(bits_host, obs_host, n_units);
   pool.wait();
+  return SNK_OK;
+}
+
+// ---- observation blocks in compressible memory ---------------------------------------------------------------------
+// The driver API is reached through the runtime's entry-point query, so libsnk.so does not link libcuda and still
+// loads on a machine without a GPU driver.
+struct DriverVmm {
+  decltype(&::cuGetErrorString) error_string = nullptr;
+  decltype(&::cuDeviceGetAttribute) device_attribute = nullptr;
+  decltype(&::cuMemGetAllocationGranularity) granularity = nullptr;
+  decltype(&::cuMemCreate) create = nullptr;
+  decltype(&::cuMemGetAllocationPropertiesFromHandle) properties = nullptr;
+  decltype(&::cuMemAddressReserve) reserve = nullptr;
+  decltype(&::cuMemMap) map = nullptr;
+  decltype(&::cuMemSetAccess) set_access = nullptr;
+  decltype(&::cuMemUnmap) unmap = nullptr;
+  decltype(&::cuMemAddressFree) address_free = nullptr;
+  decltype(&::cuMemRelease) release = nullptr;
+};
+struct ObsAlloc {
+  int device;
+  size_t size;                                   // mapped bytes (granularity-rounded) of a compressible block
+  CUmemGenericAllocationHandle handle;
+  bool vmm;                                      // false: the block came from cudaMalloc
+};
+static std::mutex g_obs_mu;                      // guards everything below
+static DriverVmm g_vmm;
+static bool g_vmm_loaded = false;
+static std::map<uintptr_t, ObsAlloc> g_obs_allocs;   // by base address
+
+template <typename F>
+static cudaError_t driver_fn(const char* name, F* fn) {
+  cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+  void* p = nullptr;
+  cudaError_t e = cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q);
+  if (e == cudaSuccess && (q != cudaDriverEntryPointSuccess || !p)) e = cudaErrorSymbolNotFound;
+  *fn = reinterpret_cast<F>(p);
+  return e;
+}
+
+static int load_vmm() {                          // called with g_obs_mu held
+  if (g_vmm_loaded) return SNK_OK;
+  CU(driver_fn("cuGetErrorString", &g_vmm.error_string));
+  CU(driver_fn("cuDeviceGetAttribute", &g_vmm.device_attribute));
+  CU(driver_fn("cuMemGetAllocationGranularity", &g_vmm.granularity));
+  CU(driver_fn("cuMemCreate", &g_vmm.create));
+  CU(driver_fn("cuMemGetAllocationPropertiesFromHandle", &g_vmm.properties));
+  CU(driver_fn("cuMemAddressReserve", &g_vmm.reserve));
+  CU(driver_fn("cuMemMap", &g_vmm.map));
+  CU(driver_fn("cuMemSetAccess", &g_vmm.set_access));
+  CU(driver_fn("cuMemUnmap", &g_vmm.unmap));
+  CU(driver_fn("cuMemAddressFree", &g_vmm.address_free));
+  CU(driver_fn("cuMemRelease", &g_vmm.release));
+  g_vmm_loaded = true;
+  return SNK_OK;
+}
+
+static int drv_fail(CUresult r, const char* what) {
+  const char* s = nullptr;
+  if (g_vmm.error_string(r, &s) != CUDA_SUCCESS || !s) s = "unknown error";
+  return fail(SNK_E_CUDA, "%s failed: %s (%d)", what, s, (int)r);
+}
+#define DRV(call)                                                                                                \
+  do {                                                                                                           \
+    CUresult _r = (call);                                                                                        \
+    if (_r != CUDA_SUCCESS) return drv_fail(_r, #call);                                                          \
+  } while (0)
+
+// A compressible block of `bytes` on `device`: *ptr = nullptr when the driver did not grant compression.
+static int alloc_compressible(int device, size_t bytes, void** ptr, ObsAlloc* rec) {
+  *ptr = nullptr;
+  int supported = 0;
+  DRV(g_vmm.device_attribute(&supported, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, device));
+  if (!supported) return SNK_OK;
+  CUmemAllocationProp prop;
+  memset(&prop, 0, sizeof prop);
+  prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+  prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+  prop.location.id = device;
+  prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+  size_t gran = 0;
+  DRV(g_vmm.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED));
+  const size_t size = (bytes + gran - 1) / gran * gran;
+  CUmemGenericAllocationHandle handle;
+  DRV(g_vmm.create(&handle, size, &prop, 0));
+  CUmemAllocationProp got;
+  memset(&got, 0, sizeof got);
+  CUresult r = g_vmm.properties(&got, handle);
+  if (r != CUDA_SUCCESS || got.allocFlags.compressionType != CU_MEM_ALLOCATION_COMP_GENERIC) {
+    g_vmm.release(handle);
+    if (r != CUDA_SUCCESS) return drv_fail(r, "cuMemGetAllocationPropertiesFromHandle");
+    return SNK_OK;                               // not granted: the caller falls back to cudaMalloc
+  }
+  CUdeviceptr va = 0;
+  r = g_vmm.reserve(&va, size, gran, 0, 0);
+  if (r != CUDA_SUCCESS) { g_vmm.release(handle); return drv_fail(r, "cuMemAddressReserve"); }
+  r = g_vmm.map(va, size, 0, handle, 0);
+  if (r != CUDA_SUCCESS) { g_vmm.address_free(va, size); g_vmm.release(handle); return drv_fail(r, "cuMemMap"); }
+  CUmemAccessDesc access;
+  memset(&access, 0, sizeof access);
+  access.location = prop.location;
+  access.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+  r = g_vmm.set_access(va, size, &access, 1);
+  if (r != CUDA_SUCCESS) {
+    g_vmm.unmap(va, size); g_vmm.address_free(va, size); g_vmm.release(handle);
+    return drv_fail(r, "cuMemSetAccess");
+  }
+  *ptr = reinterpret_cast<void*>(va);
+  *rec = ObsAlloc{device, size, handle, true};
+  return SNK_OK;
+}
+
+extern "C" int snk_alloc_obs(int device, size_t bytes, void** ptr_out, int* compressed_out) {
+  if (!ptr_out || !compressed_out || !bytes) return fail(SNK_E_INVALID, "null argument or zero size");
+  *ptr_out = nullptr;
+  *compressed_out = 0;
+  DeviceGuard guard(device);
+  if (guard.err != cudaSuccess) return fail(SNK_E_CUDA, "cudaSetDevice(%d): %s", device, cudaGetErrorString(guard.err));
+  std::lock_guard<std::mutex> lock(g_obs_mu);
+  int rc = load_vmm();
+  if (rc) return rc;
+  void* p = nullptr;
+  ObsAlloc rec{device, bytes, 0, false};
+  rc = alloc_compressible(device, bytes, &p, &rec);
+  if (rc) return rc;
+  if (!p) CU(cudaMalloc(&p, bytes));
+  g_obs_allocs[(uintptr_t)p] = rec;
+  *ptr_out = p;
+  *compressed_out = rec.vmm ? 1 : 0;
+  return SNK_OK;
+}
+
+// Whether `p` points into a live compressible block of snk_alloc_obs.
+static bool in_compressible_block(const void* p) {
+  std::lock_guard<std::mutex> lock(g_obs_mu);
+  auto it = g_obs_allocs.upper_bound((uintptr_t)p);
+  if (it == g_obs_allocs.begin()) return false;
+  --it;
+  return it->second.vmm && (uintptr_t)p < it->first + it->second.size;
+}
+
+extern "C" int snk_free_obs(void* ptr) {
+  if (!ptr) return SNK_OK;
+  std::lock_guard<std::mutex> lock(g_obs_mu);
+  auto it = g_obs_allocs.find((uintptr_t)ptr);
+  if (it == g_obs_allocs.end()) return fail(SNK_E_INVALID, "pointer was not returned by snk_alloc_obs");
+  const ObsAlloc rec = it->second;
+  g_obs_allocs.erase(it);
+  DeviceGuard guard(rec.device);
+  if (guard.err != cudaSuccess) return fail(SNK_E_CUDA, "cudaSetDevice(%d): %s", rec.device, cudaGetErrorString(guard.err));
+  if (!rec.vmm) {
+    CU(cudaFree(ptr));                           // synchronises the device itself
+    return SNK_OK;
+  }
+  CU(cudaDeviceSynchronize());                   // no kernel or copy may still touch the mapping
+  const CUdeviceptr va = reinterpret_cast<CUdeviceptr>(ptr);
+  DRV(g_vmm.unmap(va, rec.size));
+  DRV(g_vmm.address_free(va, rec.size));
+  DRV(g_vmm.release(rec.handle));
   return SNK_OK;
 }
 

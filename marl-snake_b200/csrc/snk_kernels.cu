@@ -1217,6 +1217,8 @@ __device__ __forceinline__ void encode_env_stacked(const KParams& p, const SH& s
 //       3 the plain step again, compiled without a register cap (88 registers instead of 64): fewer resident warps, more
 //         loads in flight per warp -- 2 % faster once the batch is many waves deep (cfg5: 0.756 against 0.772 ms), 3.5 %
 //         slower on a 131 072-env shard (profiles/r02_ab_tiles3.txt); the launch picks by batch size (KParams::bigreg).
+//         Only while the observation writes are bound by DRAM: into a compressible block (snk_alloc_obs) the capped
+//         instance is 11 % faster at cfg5 (0.671 against 0.758 ms, profiles/r03_retune.txt), and the step picks it.
 // Warp-private instances of variants 0 and 1 are capped at 64 registers (eight 128-thread CTAs per SM).
 template <int kNS, int kW, int kOH, int kOW, int kFS, bool kCoop, int kEnc, int kVar>
 __global__ void __launch_bounds__(kCoop ? SNK_MAX_THREADS_COOP : SNK_MAX_THREADS, (!kCoop && kVar <= 1) ? 8 : (!kCoop && kVar == 3) ? 1 : 0)

@@ -87,7 +87,8 @@ class SnakeBatch:
         self.bits_shape = self.obs_shape[:-1] + (self.obs_shape[-1] // 8,)   # channel-bit form: one byte per cell and frame
         self._bits = None
         N, ns, dev = self.num_envs, self.num_snakes, self.device
-        self._obs = torch.empty((N,) + self.obs_shape, dtype=torch.uint8, device=dev)
+        self._obs_block = _ObsBlock(dev.index, N * int(np.prod(self.obs_shape)))
+        self._obs = torch.as_tensor(self._obs_block, device=dev).view((N,) + self.obs_shape)
         self._rew = torch.empty((N, ns), dtype=torch.float64, device=dev)
         self._done = torch.empty((N, ns), dtype=torch.uint8, device=dev)
         self._fin = torch.zeros((N,), dtype=torch.uint8, device=dev)
@@ -107,6 +108,12 @@ class SnakeBatch:
         self._mutations = 0
         self._obs_stale = 'construction (no reset yet)'
         self._rollout_alive = self._rollout_age = self._rollout_mark = None
+
+    @property
+    def obs_compressed(self):
+        """True when the observation buffer is compressible device memory (snk_alloc_obs): the device supports
+        generic compression and granted it.  Values and layout are the same either way."""
+        return self._obs_block.compressed
 
     # ---- lifecycle ---------------------------------------------------------------------------------
     def close(self):
@@ -395,6 +402,26 @@ class SnakeBatch:
 
     def algorithmic_bytes_per_env_step(self):
         return int(lib.snk_algorithmic_bytes_per_env_step(self._h))
+
+
+class _ObsBlock:
+    """Owner of one observation buffer from snk_alloc_obs: `nbytes` of uint8 device memory, compressible where the
+    device grants it.  torch.as_tensor(owner) keeps the owner alive for as long as any tensor views the memory, so
+    an observation returned by a batch stays valid after the batch is closed or gone; only __del__ frees it."""
+
+    def __init__(self, device, nbytes):
+        ptr, comp = C.c_void_p(), C.c_int(0)
+        check(lib.snk_alloc_obs(int(device), int(nbytes), C.byref(ptr), C.byref(comp)))
+        self.ptr, self.compressed = ptr, bool(comp.value)
+        self.__cuda_array_interface__ = dict(shape=(int(nbytes),), typestr='|u1', data=(ptr.value, False), version=2)
+
+    def __del__(self):
+        try:
+            if self.ptr.value:
+                lib.snk_free_obs(self.ptr)
+                self.ptr = C.c_void_p()
+        except Exception:
+            pass
 
 
 def _tensor_from_ptr(ptr, n, dtype, device):
