@@ -117,8 +117,6 @@ static KParams base_params(const snk_env* h) {
   p.T = 1;
   p.enc_flavour = h->enc_flavour;
   p.enc_copy_bytes = (h->enc_flavour == ENC_LEGACY) ? h->enc_blob_bytes : h->enc_tab_off;     // LUT only
-  p.view_bits = h->d.oh + h->d.ow;
-  p.view_bias = h->d.V * h->d.W + h->d.V;
   {
     const uint64_t one = (uint64_t)1 << 32;
     const uint64_t wpr = (uint64_t)(h->d.W >> 2 > 1 ? h->d.W >> 2 : 2), nw = (uint64_t)h->d.H * wpr;
@@ -458,6 +456,7 @@ static int step_many_impl(snk_env* h, int T, const uint8_t* actions_dev, uint8_t
     if (many) p.E = h->many_tile_envs;
     p.mode = MODE_STEP; p.T = T; p.obs_every_step = every ? 1 : 0;
     p.actions = actions_dev; p.obs = obs_dev; p.bits = bits_dev; p.rew = rewards_dev; p.done = dones_dev;
+    p.vec16 = check_vec16(h, obs_dev);          // the per-step blocks of obs_every_step are whole environment blocks apart
     if (x) {
       p.fin = x->finished; p.rank = x->rank; p.ep_scores = x->episode_scores;
       p.ep_steps = x->episode_steps; p.ep_fruits = x->episode_fruits; p.ep_kills = x->episode_kills;

@@ -14,8 +14,9 @@
 //            match for the tail-growth rule, float64 reward, clear-then-write grid update      (step_group)
 //   rare     whole warp per environment: fruit respawn = k-th empty cell by word-wise rank-select;
 //            auto-reset = spawn picks + paint-and-vote overlap test + fruit seeding
-//   encode   whole warp per (environment, viewer): two crop cells per lane -> LUT -> one 128-bit
-//            streaming store (frame_stack 1; register / direct / padded-plane / table flavours); channel-bit frames
+//   encode   whole warp per (environment, viewer), or per pair of viewers on 16-byte aligned blocks: two crop cells
+//            per lane -> LUT -> one 128-bit streaming store (frame_stack 1; register / direct / padded-plane / table
+//            flavours); channel-bit frames
 //            staged in output order and expanded with flat 128-bit stores (frame_stack > 1); optionally the channel
 //            bits themselves instead of / beside the NHWC bytes
 //
@@ -371,6 +372,10 @@ struct Shape {
   // ENC_PAD plane geometry (mirrors finalize_layout; egocentric windows only, so V = (oh - 1) / 2)
   static constexpr int kV = (kOH - 1) / 2, kPadLeft = (kV + 3) / 4 * 4, kPitch0 = (kPadLeft + kW + kV + 3) / 4 * 4;
   static constexpr int kPitch = ((kPitch0 >> 2) & 1) ? kPitch0 : kPitch0 + 4;
+  // ENC_REG packing (see make_viewer_word): width of the row / column one-hot field, and the bias that makes a crop
+  // origin non-negative
+  __device__ __forceinline__ int view_bits() const { return oh() + ow(); }
+  __device__ __forceinline__ int view_bias() const { return (kW && kOH) ? kV * kW + kV : d.V * d.W + d.V; }
   __device__ __forceinline__ int pad_pitch() const { return (kW && kOH) ? kPitch : d.pad_pitch; }
   __device__ __forceinline__ int pad_left() const { return (kW && kOH) ? kPadLeft : d.pad_left; }
   static constexpr int kUnits = (kOH * kOW != 0 && kOH * kOW <= 127) ? 2 : 4;   // 16-byte units a lane owns per viewer
@@ -905,12 +910,96 @@ __device__ __forceinline__ CellWords make_cell_words(const SH& sh, int B) {
 template <class SH>
 __device__ __forceinline__ uint32_t make_viewer_word(const KParams& p, const SH& sh, const uint8_t* base, int v) {
   const Dims& d = p.d;
-  const int W = sh.W(), oh = sh.oh(), ow = sh.ow(), B = p.view_bits;
+  const int W = sh.W(), oh = sh.oh(), ow = sh.ow(), B = sh.view_bits();
   int r0, c0;
   viewer_origin(d, base, sh.ns(), W, d.V, v, r0, c0);
   const int rlo = max(0, -r0), rhi = min(oh, d.H - r0), clo = max(0, -c0), chi = min(ow, W - c0);
   const uint32_t valid = (((1u << rhi) - 1u) & ~((1u << rlo) - 1u)) | ((((1u << chi) - 1u) & ~((1u << clo) - 1u)) << oh);
-  return (~valid & ((1u << B) - 1u)) | ((uint32_t)(r0 * W + c0 + p.view_bias) << B);
+  return (~valid & ((1u << B) - 1u)) | ((uint32_t)(r0 * W + c0 + sh.view_bias()) << B);
+}
+
+// ---- ENC_REG, viewer pairs (warp-private tiles, frame_stack 1, NHWC only) ---------------------------
+// With an odd window (ohw cells) a viewer block of 8 * ohw bytes is only 8-byte aligned, but two consecutive viewers
+// (v, v+1) make 2 * ohw cells = ohw whole 16-byte units, and with an even number of viewers per environment every such
+// pair block starts 16-byte aligned whenever the environment blocks do (p.vec16).  Unit S = ohw / 2 holds the last cell
+// of v and the first of v+1.  Lane l owns four units, at the same place in every pair block:
+//   slot 0: unit l,  slot 1: unit 32 + l      (viewer v, while <= S; cell b of unit S is cell 0 of v+1)
+//   slot 2: unit S+1 + l,  slot 3: unit S+33 + l  (viewer v+1, while < ohw)
+// so which viewer a cell belongs to is fixed per lane: only the one lane holding unit S switches viewers for cell b.
+// The cell words (same packing as make_cell_words, idle cells flagged in bit 31) live in a CellWords:
+// w[0][k] = cell a, w[1][k] = cell b of slot k.
+__device__ __forceinline__ int pair_unit(int k, int lane, int S) { return k < 2 ? 32 * k + lane : S + 1 + 32 * (k - 2) + lane; }
+
+template <class SH>
+__device__ __forceinline__ bool pair_unit_used(const SH& sh, int k, int lane) {
+  const int S = sh.ohw() >> 1, u = pair_unit(k, lane, S);
+  return k < 2 ? u <= S : u < sh.ohw();
+}
+
+template <class SH>
+__device__ __forceinline__ CellWords make_pair_cell_words(const SH& sh) {
+  const int lane = (int)lane_id(), ohw = sh.ohw(), ow = sh.ow(), oh = sh.oh(), W = sh.W(), B = sh.view_bits();
+  CellWords cw;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const int u = pair_unit(k, lane, ohw >> 1);
+    const bool used = pair_unit_used(sh, k, lane);
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      int c = 2 * u + s;
+      if (c >= ohw) c -= ohw;                                  // window cell inside its own viewer
+      uint32_t w = 0x80000000u;
+      if (used) {
+        const int ci = c / ow, cj = c - ci * ow;
+        w = (1u << ci) | (1u << (oh + cj)) | ((uint32_t)(ci * W + cj) << B);
+      }
+      cw.w[s][k] = w;
+    }
+  }
+  return cw;
+}
+
+// All viewer pairs of one environment.  view32: shared address of the environment's viewer words (s_view), outl: its
+// observation block plus 16 * lane.  kMask: grid bytes carry direction bits (code_mask 63).
+template <class SH, bool kMask>
+__device__ __forceinline__ void encode_env_pairs(const KParams& p, const SH& sh, uint32_t grid32, uint32_t view32,
+                                                 const CellWords& cw, uint8_t* outl, uint32_t lut32) {
+  const int lane = (int)lane_id();
+  const int ns = sh.ns(), ohw = sh.ohw(), S = ohw >> 1, B = sh.view_bits(), LS = sh.lut_stride();
+  const uint32_t field = (1u << B) - 1u;
+  const uint32_t gbase = grid32 - (uint32_t)sh.view_bias();
+  const uint32_t zero = lut32;                                   // LUT entry 0 of viewer 0: a zero byte (code EMPTY)
+  const uint32_t cm = (uint32_t)p.d.code_mask;
+  // the lane holding unit S, in slot 0 or 1
+  const bool split0 = S < 32 && lane == S, split1 = S >= 32 && lane == S - 32;
+  const bool st0 = pair_unit_used(sh, 0, lane), st1 = pair_unit_used(sh, 1, lane);
+  const bool st2 = pair_unit_used(sh, 2, lane), st3 = pair_unit_used(sh, 3, lane);
+  const int o2 = 16 * (S + 1), o3 = 16 * (S + 33);              // byte offsets of slots 2 and 3 (lane part in outl)
+  auto cell = [&](uint32_t e, uint32_t bad, uint32_t org, uint32_t lut) -> uint2 {
+    const uint32_t a = (e & bad) ? zero : org + (e >> B);
+    SNK_ASSERT(p, a == zero || a - grid32 < (uint32_t)p.d.HW);
+    const uint32_t k = kMask ? lds_u8(a) & cm : lds_u8(a);      // (an AND with 0xff would not be folded: lds_u8 is asm)
+    SNK_ASSERT(p, k < (uint32_t)LS);
+    return lds_v2(lut + k * 8u);
+  };
+#pragma unroll 1
+  for (int v = 0; v < ns; v += 2) {
+    const uint2 vw = lds_v2(view32 + 4u * (uint32_t)v);
+    const uint32_t bad0 = (vw.x & field) | 0x80000000u, bad1 = (vw.y & field) | 0x80000000u;
+    const uint32_t org0 = gbase + (vw.x >> B), org1 = gbase + (vw.y >> B);
+    const uint32_t lut0 = lut32 + (uint32_t)(v * LS) * 8u, lut1 = lut0 + (uint32_t)LS * 8u;
+    const uint2 q0a = cell(cw.w[0][0], bad0, org0, lut0);
+    const uint2 q0b = cell(cw.w[1][0], split0 ? bad1 : bad0, split0 ? org1 : org0, split0 ? lut1 : lut0);
+    const uint2 q1a = cell(cw.w[0][1], bad0, org0, lut0);
+    const uint2 q1b = cell(cw.w[1][1], split1 ? bad1 : bad0, split1 ? org1 : org0, split1 ? lut1 : lut0);
+    const uint2 q2a = cell(cw.w[0][2], bad1, org1, lut1), q2b = cell(cw.w[1][2], bad1, org1, lut1);
+    const uint2 q3a = cell(cw.w[0][3], bad1, org1, lut1), q3b = cell(cw.w[1][3], bad1, org1, lut1);
+    uint8_t* const o = outl + (size_t)v * ohw * 8;
+    if (st0) st_cs_128(o, q0a, q0b);
+    if (st1) st_cs_128(o + 512, q1a, q1b);
+    if (st2) st_cs_128(o + o2, q2a, q2b);
+    if (st3) st_cs_128(o + o3, q3a, q3b);
+  }
 }
 
 template <class SH>
@@ -918,10 +1007,10 @@ __device__ __forceinline__ void encode_viewer_reg(const KParams& p, const SH& sh
                                                   const CellWords& cw, int v, uint8_t* outv, uint32_t lut32,
                                                   uint8_t* bitsv, uint32_t lutb32) {
   const int lane = (int)lane_id();
-  const int ohw = sh.ohw(), B = p.view_bits;
+  const int ohw = sh.ohw(), B = sh.view_bits();
   const uint32_t lutv32 = lut32 + (uint32_t)(v * sh.lut_stride()) * 8u;          // entry 0 is all zero
   const uint32_t bad = (vw & ((1u << B) - 1u)) | 0x80000000u;
-  const uint32_t gorg = grid32 + (vw >> B) - (uint32_t)p.view_bias;
+  const uint32_t gorg = grid32 + (vw >> B) - (uint32_t)sh.view_bias();
   const int shift = (int)((reinterpret_cast<uintptr_t>(outv) >> 3) & 1);
   const int units = (ohw + shift + 1) >> 1;                                       // <= 64
   const uint32_t e0 = shift ? cw.w[1][0] : cw.w[0][0], e1 = shift ? cw.w[1][1] : cw.w[0][1];
@@ -1442,8 +1531,33 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
         }
       }
     } else if (render) {
-      if (kEnc == ENC_REG && !cw_ready) { cw = make_cell_words(sh, p.view_bits); cw_ready = true; }
-      if (kCoop) {
+      // viewer pairs (encode_env_pairs): warp-private ENC_REG tiles writing NHWC bytes only, odd window, even
+      // viewer count, 16-byte aligned environment blocks
+      constexpr bool kPairable = kEnc == ENC_REG && !kCoop && !(kVar == 1) && (kOH * kOW == 0 || ((kOH * kOW) & 1)) &&
+                                 (kNS == 0 || (kNS & 1) == 0);
+      const bool pairs = kPairable && obs_t && !bits_t && p.vec16 && (ohw & 1) && (ns & 1) == 0;
+      if (kEnc == ENC_REG && !cw_ready) { cw = pairs ? make_pair_cell_words(sh) : make_cell_words(sh, sh.view_bits()); cw_ready = true; }
+      if (kPairable && pairs) {
+        const uint32_t view32 = (uint32_t)__cvta_generic_to_shared(s_view);
+        uint8_t* const outl = obs_t + (size_t)e0 * d.obs_env_bytes + 16 * lane;
+        if (d.code_mask == 0xff) {
+#pragma unroll 1
+          for (int q = 0; q < ne; ++q) {
+            if (s_flag[q] & F_SKIP) continue;
+            encode_env_pairs<Shape<kNS, kW, kOH, kOW, kFS>, false>(p, sh, (uint32_t)__cvta_generic_to_shared(tp.G(q)),
+                                                                   view32 + 4u * (uint32_t)(q * G), cw,
+                                                                   outl + (size_t)q * d.obs_env_bytes, lut32);
+          }
+        } else {
+#pragma unroll 1
+          for (int q = 0; q < ne; ++q) {
+            if (s_flag[q] & F_SKIP) continue;
+            encode_env_pairs<Shape<kNS, kW, kOH, kOW, kFS>, true>(p, sh, (uint32_t)__cvta_generic_to_shared(tp.G(q)),
+                                                                  view32 + 4u * (uint32_t)(q * G), cw,
+                                                                  outl + (size_t)q * d.obs_env_bytes, lut32);
+          }
+        }
+      } else if (kCoop) {
 #pragma unroll 1
         for (int pv = wfirst; pv < ne * ns; pv += wstep) {
           const int q = pv / ns, v = pv - q * ns;

@@ -53,7 +53,7 @@ struct KParams {
   const uint8_t* mask;
   int32_t mode;
   int32_t E;                   // environments per tile: 32 / group size, or fewer (a power of two) in coop mode
-  int32_t vec16;               // 128-bit observation stores are legal for every tile (fs > 1 path)
+  int32_t vec16;               // every environment's observation block is 16-byte aligned (fs > 1 path, ENC_REG viewer pairs)
   int32_t force_generic;       // run the unspecialised kernel instance (tests)
   const uint8_t* enc_blob;     // fs == 1: host-built encode tables (see encode_blob_fill)
   int32_t enc_blob_bytes;
@@ -65,8 +65,6 @@ struct KParams {
   int32_t use_tma;             // move the record tile with cp.async.bulk (TMA) instead of LDG/STG
   int32_t enc_flavour;         // ENC_* (fs == 1)
   int32_t enc_copy_bytes;      // bytes of the blob the kernel stages (the table is skipped when unused)
-  int32_t view_bits;           // ENC_REG: oh + ow, the width of the row/column one-hot field
-  int32_t view_bias;           // ENC_REG: V*W + V, added to the crop origin so it packs as unsigned
   uint32_t inv_grid_words;     // ENC_PAD: ceil(2^32 / (H*W/4)) and ceil(2^32 / (W/4)): exact division of word indices
   uint32_t inv_row_words;      //          below 2^16 by a multiply-high
   int32_t pdl;                 // launch with programmatic stream serialization (SNK_PDL=0 switches it off)
