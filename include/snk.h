@@ -56,9 +56,12 @@ enum {
   SNK_DEV_SPAWN_GIVEUP = 8,      /* no overlap-free spawn found within the attempt cap               */
   SNK_DEV_INTERNAL = 16,         /* a bounds / alignment check failed (debug build, -DSNK_DEBUG_CHECKS) */
   SNK_DEV_TMA_TIMEOUT = 32,      /* a record tile's bulk copy did not complete within 2 s; that tile was not stepped */
-  SNK_DEV_STATE = 64             /* snk_set_state: the grid is not the handle's walls + fruit cells + the live snakes'
+  SNK_DEV_STATE = 64,            /* snk_set_state: the grid is not the handle's walls + fruit cells + the live snakes'
                                     bodies (the resident record stores only those), or it holds more fruit cells than
-                                    the record has slots (num_fruits + num_snakes, rounded up to 8)       */
+                                    the record has slots (num_fruits + num_snakes, rounded up to 8); with a
+                                    wall-map pool, in either record layout: its walls are not those of next_map */
+  SNK_DEV_MAP_RANGE = 128        /* wall-map pool: a map id (next_map, or cur_map rewritten by the caller) was not below
+                                    the number of maps; map 0 was used instead                          */
 };
 
 enum { SNK_RNG_PHILOX = 0, SNK_RNG_REPLAY = 1 };
@@ -128,6 +131,26 @@ int snk_create(const snk_config* cfg, snk_env** out);
  * any grid, :73-99) and fruits land on its empty cells.  The outer ring must be wall (SNK_E_INVALID otherwise): the
  * reference would let a snake walk out of the array there.  The map is copied; walls_host may be freed after the call. */
 int snk_create_map(const snk_config* cfg, const uint8_t* walls_host, snk_env** out);
+/* A POOL of num_maps wall layouts (1..SNK_MAX_MAPS), all height x width: walls_host is uint8 [num_maps, height, width],
+ * each map following the rules of snk_create_map (nonzero = WALL, outer ring all wall, at least num_snakes spawn poses;
+ * SNK_E_INVALID names the first map that breaks one).  Every environment has two map ids (uint8 [N] device arrays,
+ * snk_map_ids_dev):
+ *   next_map[e]  the map env e's next reset starts from -- every reset until it is rewritten.  The caller may rewrite it
+ *                on the device between any two calls (e.g. fill it with random ids after every step to draw a fresh map
+ *                for each auto-reset);
+ *   cur_map[e]   the map of env e's current episode.  Every reset -- snk_reset / _bits (masked or not), the auto-reset of
+ *                a step, snk_reset_host, snk_set_state -- sets it to next_map[e]; nothing else changes it.
+ * map_ids_host: the initial next_map (uint8 [N], every id < num_maps), or NULL for (env_id_offset + e) % num_maps, so a
+ * sharded run equals the single-device run.  A reset on map m draws its spawn pose from map m's table with the same
+ * Philox counters as snk_create_map (a pool of identical maps gives that handle's trajectories); replayed spawn indices
+ * index map m's table.  An id >= num_maps found at a reset reads as map 0 and raises SNK_DEV_MAP_RANGE. */
+#define SNK_MAX_MAPS 256
+int snk_create_maps(const snk_config* cfg, int32_t num_maps, const uint8_t* walls_host, const uint8_t* map_ids_host,
+                    snk_env** out);
+/* Device pointers of next_map and cur_map (uint8 [N] each) of a pool handle; SNK_E_STATE for a handle without a pool. */
+int snk_map_ids_dev(snk_env* env, uint8_t** next_dev, uint8_t** cur_dev);
+/* Number of maps in the handle's pool, 0 for a handle without one. */
+int snk_num_maps(const snk_env* env);
 /* SnakeEnv.close (snake_env.py:298) */
 int snk_destroy(snk_env* env);
 const char* snk_last_error(void);
@@ -240,7 +263,7 @@ int snk_set_state(snk_env* env, const snk_state_view* in, uint8_t* obs_dev, void
 
 /* Exact checkpoint / resume of a shard (the reference never saves env state; its trainers checkpoint only
  * their networks, train_dqn.py:356-383): the raw records, frame histories and rollout statistics as one host
- * blob.  A handle created with the same configuration (same seed and env_id_offset for the same Philox
+ * blob -- with a wall-map pool also next_map, cur_map and a digest of the pool, which must match on load.  A handle created with the same configuration (same seed and env_id_offset for the same Philox
  * stream; replay streams are set separately) continues bit for bit after snk_checkpoint_load. */
 size_t snk_checkpoint_bytes(const snk_env* env);
 int snk_checkpoint_save(snk_env* env, void* blob_host, size_t bytes);

@@ -17,7 +17,9 @@ DEV_ERRORS = {1: 'action outside {0,1,2}', 2: 'replay stream exhausted',
               4: 'replayed draw out of range / replayed spawn overlaps', 8: 'spawn sampling gave up',
               16: 'internal bounds check failed (debug build)',
               32: "a record tile's bulk copy timed out; the tile was skipped",
-              64: 'set_state: grid is not walls + fruits + live snakes, or too many fruit cells'}
+              64: 'set_state: grid is not walls + fruits + live snakes, or too many fruit cells',
+              128: 'a map id was not below the number of wall maps; map 0 was used'}
+SNK_MAX_MAPS = 256
 STAT_NAMES = ('episodes', 'return_sum', 'episode_steps_sum', 'fruits_sum', 'kills_sum', 'deaths',
               'env_steps', 'reserved')
 
@@ -49,6 +51,9 @@ class SnkStateView(C.Structure):
 PROTOTYPES = {
     'snk_create': (C.c_int, [C.POINTER(SnkConfig), C.POINTER(C.c_void_p)]),
     'snk_create_map': (C.c_int, [C.POINTER(SnkConfig), C.c_void_p, C.POINTER(C.c_void_p)]),
+    'snk_create_maps': (C.c_int, [C.POINTER(SnkConfig), C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
+    'snk_map_ids_dev': (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
+    'snk_num_maps': (C.c_int, [C.c_void_p]),
     'snk_destroy': (C.c_int, [C.c_void_p]),
     'snk_last_error': (C.c_char_p, []),
     'snk_abi_version': (C.c_int, []),

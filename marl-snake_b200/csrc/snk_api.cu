@@ -65,6 +65,13 @@ struct snk_env {
   uint64_t* spawn = nullptr;
   uint32_t* wall_map = nullptr;                  // custom wall layout (snk_create_map): H*W cell codes, padded to words
   uint8_t* base_grid = nullptr;                  // compact records: the wall layout, one copy per environment of a tile
+  // wall-map pool (snk_create_maps): num_maps layouts of off_c0 bytes, each map's part of `spawn`, the per-env map ids
+  int num_maps = 0;                              // 0: no pool
+  uint8_t* maps = nullptr;
+  uint2* map_tab = nullptr;
+  uint8_t* next_map = nullptr;
+  uint8_t* cur_map = nullptr;
+  uint64_t pool_digest = 0;                      // layouts + spawn-table sizes: a checkpoint only loads into the same pool
   int32_t* replay = nullptr;
   int64_t* replay_off = nullptr;
   uint32_t* err = nullptr;
@@ -115,6 +122,10 @@ static KParams base_params(const snk_env* h) {
   p.enc_lutb_off = h->enc_lutb_off;
   p.lut_dual = h->lut_dual; p.coop = h->coop; p.use_tma = h->use_tma; p.pdl = h->pdl; p.bigreg = h->bigreg; p.l2_keep = h->l2_keep; p.l2_keep_frac = h->l2_keep_frac;
   p.T = 1;
+  if (h->num_maps) {
+    p.pool = h->maps; p.map_tab = h->map_tab; p.next_map = h->next_map; p.cur_map = h->cur_map; p.num_maps = h->num_maps;
+    p.bigreg = 0;                                // pool handles run the capped instances (no uncapped pool instance is built)
+  }
   p.enc_flavour = h->enc_flavour;
   p.enc_copy_bytes = (h->enc_flavour == ENC_LEGACY) ? h->enc_blob_bytes : h->enc_tab_off;     // LUT only
   {
@@ -126,14 +137,28 @@ static KParams base_params(const snk_env* h) {
   return p;
 }
 
-static int create_impl(const snk_config* c, const uint8_t* walls_host, snk_env** out);
-extern "C" int snk_create(const snk_config* c, snk_env** out) { return create_impl(c, nullptr, out); }
+// num_maps == 0: snk_create (walls_host null) or snk_create_map (one layout, no pool); num_maps >= 1: a wall-map pool of
+// num_maps layouts of height * width bytes, back to back in walls_host
+static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_host, const uint8_t* map_ids_host, snk_env** out);
+extern "C" int snk_create(const snk_config* c, snk_env** out) { return create_impl(c, 0, nullptr, nullptr, out); }
 extern "C" int snk_create_map(const snk_config* c, const uint8_t* walls_host, snk_env** out) {
   if (!walls_host) return fail(SNK_E_INVALID, "null wall map");
-  return create_impl(c, walls_host, out);
+  return create_impl(c, 0, walls_host, nullptr, out);
+}
+extern "C" int snk_create_maps(const snk_config* c, int32_t num_maps, const uint8_t* walls_host, const uint8_t* map_ids_host,
+                               snk_env** out) {
+  if (num_maps < 1 || num_maps > SNK_MAX_MAPS) return fail(SNK_E_INVALID, "num_maps must be in 1..%d", SNK_MAX_MAPS);
+  if (!walls_host) return fail(SNK_E_INVALID, "null wall maps");
+  return create_impl(c, num_maps, walls_host, map_ids_host, out);
 }
 
-static int create_impl(const snk_config* c, const uint8_t* walls_host, snk_env** out) {
+static uint64_t fnv1a(uint64_t h, const void* data, size_t n) {
+  const uint8_t* b = (const uint8_t*)data;
+  for (size_t i = 0; i < n; ++i) { h ^= b[i]; h *= 0x100000001B3ull; }
+  return h;
+}
+
+static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_host, const uint8_t* map_ids_host, snk_env** out) {
   if (!c || !out) return fail(SNK_E_INVALID, "null argument");
   if (c->abi_version != SNK_ABI_VERSION) return fail(SNK_E_INVALID, "abi_version %d != %d", c->abi_version, SNK_ABI_VERSION);
   if (c->num_envs < 1) return fail(SNK_E_INVALID, "num_envs must be >= 1");
@@ -165,31 +190,71 @@ static int create_impl(const snk_config* c, const uint8_t* walls_host, snk_env**
 
   // custom wall layout (make_grid_from_txt, core/grid_util.py:23-33): normalised to cell codes, one word-padded plane.
   // The outer ring must be wall -- it is what keeps a head inside the array (the reference would index out of it).
+  // A wall-map pool keeps every map so, off_c0 bytes apart.
+  const int nmaps = walls_host ? (num_maps ? num_maps : 1) : 0;
+  const size_t plane = num_maps ? (size_t)d.off_c0 : ((size_t)d.HW + 3) / 4 * 4;
   std::vector<uint8_t> walls;
   if (walls_host) {
-    walls.assign(((size_t)d.HW + 3) / 4 * 4, 0);
-    for (int i = 0; i < d.HW; ++i) walls[i] = walls_host[i] ? (uint8_t)WALL : (uint8_t)EMPTY;
-    for (int i = 0; i < d.HW; ++i) {
-      const int r = i / d.W, cc = i % d.W;
-      if ((r == 0 || r == d.H - 1 || cc == 0 || cc == d.W - 1) && !walls[i]) {
-        delete h;
-        return fail(SNK_E_INVALID, "wall map: border cell (%d, %d) is not a wall", r, cc);
+    walls.assign((size_t)nmaps * plane, 0);
+    for (int m = 0; m < nmaps; ++m) {
+      const uint8_t* src = walls_host + (size_t)m * d.HW;
+      uint8_t* dst = walls.data() + (size_t)m * plane;
+      for (int i = 0; i < d.HW; ++i) dst[i] = src[i] ? (uint8_t)WALL : (uint8_t)EMPTY;
+      for (int i = 0; i < d.HW; ++i) {
+        const int r = i / d.W, cc = i % d.W;
+        if ((r == 0 || r == d.H - 1 || cc == 0 || cc == d.W - 1) && !dst[i]) {
+          delete h;
+          if (num_maps) return fail(SNK_E_INVALID, "wall map %d: border cell (%d, %d) is not a wall", m, r, cc);
+          return fail(SNK_E_INVALID, "wall map: border cell (%d, %d) is not a wall", r, cc);
+        }
       }
     }
   }
   const uint8_t* wm = walls_host ? walls.data() : nullptr;
 
-  // spawn table (host) -- core/grid_util.py:73-115
-  const int64_t n_cand = spawn_enumerate(d.H, d.W, d.K, nullptr, nullptr, 0, SPAWN_TABLE_LIMIT, wm);
-  if (n_cand < d.ns) { delete h; return fail(SNK_E_INVALID, "only %lld spawn poses for %d snakes", (long long)n_cand, c->num_snakes); }
-  if (n_cand > SPAWN_TABLE_LIMIT) {
-    delete h;
-    return fail(SNK_E_INVALID, "more than %lld spawn poses for a %dx%d grid and snake_length %d (the reference enumerates "
-                "them on every reset; here the table would not fit)", (long long)SPAWN_TABLE_LIMIT, c->height, c->width, c->snake_length);
+  // spawn table (host) -- core/grid_util.py:73-115.  A pool concatenates one table per map.
+  std::vector<uint64_t> table;
+  std::vector<uint2> map_tab;
+  for (int m = 0; m < (nmaps ? nmaps : 1); ++m) {
+    const uint8_t* wmm = wm ? wm + (size_t)m * plane : nullptr;
+    const int64_t n_cand = spawn_enumerate(d.H, d.W, d.K, nullptr, nullptr, 0, SPAWN_TABLE_LIMIT, wmm);
+    if (n_cand < d.ns) {
+      delete h;
+      if (num_maps) return fail(SNK_E_INVALID, "wall map %d: only %lld spawn poses for %d snakes", m, (long long)n_cand, c->num_snakes);
+      return fail(SNK_E_INVALID, "only %lld spawn poses for %d snakes", (long long)n_cand, c->num_snakes);
+    }
+    if (n_cand > SPAWN_TABLE_LIMIT) {
+      delete h;
+      if (num_maps) return fail(SNK_E_INVALID, "wall map %d: more than %lld spawn poses for snake_length %d", m,
+                                (long long)SPAWN_TABLE_LIMIT, c->snake_length);
+      return fail(SNK_E_INVALID, "more than %lld spawn poses for a %dx%d grid and snake_length %d (the reference enumerates "
+                  "them on every reset; here the table would not fit)", (long long)SPAWN_TABLE_LIMIT, c->height, c->width, c->snake_length);
+    }
+    if ((int64_t)table.size() + n_cand > SPAWN_TABLE_LIMIT) {
+      delete h;
+      return fail(SNK_E_INVALID, "wall maps 0..%d: more than %lld spawn poses together (%lld MB of tables)", m,
+                  (long long)SPAWN_TABLE_LIMIT, (long long)(SPAWN_TABLE_LIMIT * 8 >> 20));
+    }
+    map_tab.push_back(make_uint2((uint32_t)table.size(), (uint32_t)n_cand));
+    table.resize(table.size() + (size_t)n_cand);
+    spawn_enumerate(d.H, d.W, d.K, table.data() + map_tab.back().x, nullptr, n_cand, 0, wmm);
   }
-  std::vector<uint64_t> table((size_t)n_cand);
-  spawn_enumerate(d.H, d.W, d.K, table.data(), nullptr, n_cand, 0, wm);
-  d.n_cand = (uint32_t)n_cand;
+  d.n_cand = map_tab[0].y;
+  std::vector<uint8_t> ids;
+  if (num_maps) {
+    // next_map: the caller's assignment, or global env id modulo the number of maps (a sharded run equals one run)
+    ids.resize((size_t)d.N);
+    for (int e = 0; e < d.N; ++e) {
+      if (map_ids_host && map_ids_host[e] >= num_maps) {
+        delete h;
+        return fail(SNK_E_INVALID, "map_ids[%d] = %d names no map (num_maps %d)", e, map_ids_host[e], num_maps);
+      }
+      ids[e] = map_ids_host ? map_ids_host[e] : (uint8_t)((c->env_id_offset + (uint64_t)e) % (uint64_t)num_maps);
+    }
+    h->num_maps = num_maps;
+    uint64_t dg = fnv1a(0xCBF29CE484222325ull, walls.data(), walls.size());
+    h->pool_digest = fnv1a(dg, map_tab.data(), map_tab.size() * sizeof(uint2));
+  }
 
   // tile shape: a tile is 32/G environments (G = num_snakes rounded up to a power of two).  Large
   // batches: every warp owns a tile, the CTA's warps share only the encode tables.  Small batches or
@@ -288,11 +353,21 @@ static int create_impl(const snk_config* c, const uint8_t* walls_host, snk_env**
   CUH(cudaMalloc(&h->stats, STAT_COUNT * sizeof(double)));
   CUH(cudaMalloc(&h->replay_off, ((size_t)d.N + 1) * sizeof(int64_t)));
   CUH(cudaMemcpy(h->spawn, table.data(), table.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
-  if (wm) {
+  if (num_maps) {
+    // the pool serves the resets and (compact records) the tile loads, which paint each grid from its own map
+    CUH(cudaMalloc(&h->maps, walls.size()));
+    CUH(cudaMemcpy(h->maps, walls.data(), walls.size(), cudaMemcpyHostToDevice));
+    CUH(cudaMalloc(&h->map_tab, map_tab.size() * sizeof(uint2)));
+    CUH(cudaMemcpy(h->map_tab, map_tab.data(), map_tab.size() * sizeof(uint2), cudaMemcpyHostToDevice));
+    CUH(cudaMalloc(&h->next_map, ids.size()));
+    CUH(cudaMalloc(&h->cur_map, ids.size()));
+    CUH(cudaMemcpy(h->next_map, ids.data(), ids.size(), cudaMemcpyHostToDevice));
+    CUH(cudaMemcpy(h->cur_map, ids.data(), ids.size(), cudaMemcpyHostToDevice));
+  } else if (wm) {
     CUH(cudaMalloc(&h->wall_map, walls.size()));
     CUH(cudaMemcpy(h->wall_map, walls.data(), walls.size(), cudaMemcpyHostToDevice));
   }
-  {
+  if (!num_maps) {
     // the wall layout every reset starts from: make_grid's walled box (core/grid_util.py:14-20) or the custom map,
     // padded to 16 bytes.  Compact records: it is also what the grid every record implies starts from -- as many
     // copies as the widest tile has environments, so ONE bulk copy paints a tile's grids
@@ -344,6 +419,7 @@ extern "C" int snk_destroy(snk_env* h) {
   DeviceGuard guard(h->device);
   cudaFree(h->recs); cudaFree(h->hist); cudaFree(h->spawn); cudaFree(h->replay); cudaFree(h->replay_off);
   cudaFree(h->err); cudaFree(h->stats); cudaFree(h->enc_blob); cudaFree(h->wall_map); cudaFree(h->base_grid);
+  cudaFree(h->maps); cudaFree(h->map_tab); cudaFree(h->next_map); cudaFree(h->cur_map);
   cudaFree(h->h_actions); cudaFree(h->h_obs); cudaFree(h->h_rew); cudaFree(h->h_done);
   cudaFree(h->h_fin); cudaFree(h->h_rank); cudaFree(h->h_scores); cudaFree(h->h_counts);
   cudaFree(h->small_dev);
@@ -365,6 +441,14 @@ extern "C" int snk_obs_shape(const snk_env* h, int32_t out[4]) {
 }
 extern "C" size_t snk_obs_bytes(const snk_env* h) { return h ? (size_t)h->d.N * h->d.obs_env_bytes : 0; }
 extern "C" int snk_num_envs(const snk_env* h) { return h ? h->d.N : 0; }
+extern "C" int snk_num_maps(const snk_env* h) { return h ? h->num_maps : 0; }
+
+extern "C" int snk_map_ids_dev(snk_env* h, uint8_t** next_dev, uint8_t** cur_dev) {
+  if (!h || !next_dev || !cur_dev) return fail(SNK_E_INVALID, "null argument");
+  if (!h->num_maps) return fail(SNK_E_STATE, "handle has no wall-map pool (create it with snk_create_maps)");
+  *next_dev = h->next_map; *cur_dev = h->cur_map;
+  return SNK_OK;
+}
 
 extern "C" size_t snk_algorithmic_bytes_per_env_step(const snk_env* h) {
   if (!h) return 0;
@@ -937,7 +1021,8 @@ extern "C" int snk_get_state(snk_env* h, const snk_state_view* out, void* stream
   if (!h || !out) return fail(SNK_E_INVALID, "null argument");
   if (out->cells && out->max_cells < 1) return fail(SNK_E_INVALID, "max_cells must be >= 1 when cells is given");
   ON_DEVICE(h);
-  CU(launch_get_state(h->d, h->recs, h->base_grid, to_view(out), (cudaStream_t)stream));
+  const MapView mv = {h->maps, h->cur_map, nullptr, h->num_maps};
+  CU(launch_get_state(h->d, h->recs, h->base_grid, mv, h->err, to_view(out), (cudaStream_t)stream));
   note_user_stream(h, (cudaStream_t)stream);
   return SNK_OK;
 }
@@ -948,7 +1033,8 @@ extern "C" int snk_set_state(snk_env* h, const snk_state_view* in, uint8_t* obs_
     return fail(SNK_E_INVALID, "set_state needs grid, alive, dir, cells, length, alive_counter, episode_length");
   if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
   ON_DEVICE(h);
-  CU(launch_set_state(h->d, h->recs, h->base_grid, h->err, to_view(in), (cudaStream_t)stream));
+  const MapView mv = {h->maps, h->next_map, h->cur_map, h->num_maps};
+  CU(launch_set_state(h->d, h->recs, h->base_grid, mv, h->err, to_view(in), (cudaStream_t)stream));
   KParams p = base_params(h);
   p.mode = MODE_ENCODE; p.obs = obs_dev;
   p.vec16 = check_vec16(h, obs_dev);
@@ -961,11 +1047,17 @@ extern "C" int snk_set_state(snk_env* h, const snk_state_view* in, uint8_t* obs_
 // ---- exact checkpoint: the raw records (grid, snakes, counters, Philox event, replay cursor, statistics),
 // the frame histories and the rollout statistics vector, byte for byte
 static const uint64_t CKPT_MAGIC = 0x0031544B434B4E53ull;     // "SNKCKT1"
+// A handle with a wall-map pool writes its own magic and appends the pool's digest, next_map and cur_map, so its blob
+// and that of a handle without a pool never load into each other.
+static const uint64_t CKPT_MAGIC_POOL = 0x0031504B434B4E53ull;  // "SNKCKP1"
 struct CkptHeader { uint64_t magic; int32_t N, H, W, ns, K, V, fs, dig, rec_bytes, hist_env_bytes; double env_steps; };   // rec_bytes: per env in HBM
+
+static size_t ckpt_pool_bytes(const snk_env* h) { return h->num_maps ? sizeof(uint64_t) + 2 * (size_t)h->d.N : 0; }
 
 extern "C" size_t snk_checkpoint_bytes(const snk_env* h) {
   if (!h) return 0;
-  return sizeof(CkptHeader) + (size_t)h->d.N * ((size_t)h->d.hbm_rec_bytes + (size_t)h->d.hist_env_bytes) + STAT_COUNT * sizeof(double);
+  return sizeof(CkptHeader) + (size_t)h->d.N * ((size_t)h->d.hbm_rec_bytes + (size_t)h->d.hist_env_bytes) + STAT_COUNT * sizeof(double) +
+         ckpt_pool_bytes(h);
 }
 
 extern "C" int snk_checkpoint_save(snk_env* h, void* blob_host, size_t bytes) {
@@ -975,11 +1067,18 @@ extern "C" int snk_checkpoint_save(snk_env* h, void* blob_host, size_t bytes) {
   CU(cudaDeviceSynchronize());
   const Dims& d = h->d;
   uint8_t* out = (uint8_t*)blob_host;
-  CkptHeader hd = {CKPT_MAGIC, d.N, d.H, d.W, d.ns, d.K, d.V, d.fs, d.dig | (d.compact << 1), d.hbm_rec_bytes, d.hist_env_bytes, 0.0};
+  CkptHeader hd = {h->num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC, d.N, d.H, d.W, d.ns, d.K, d.V, d.fs, d.dig | (d.compact << 1),
+                   d.hbm_rec_bytes, d.hist_env_bytes, 0.0};
   memcpy(out, &hd, sizeof hd); out += sizeof hd;
   CU(cudaMemcpy(out, h->recs, (size_t)d.N * d.hbm_rec_bytes, cudaMemcpyDeviceToHost)); out += (size_t)d.N * d.hbm_rec_bytes;
   if (d.hist_env_bytes) { CU(cudaMemcpy(out, h->hist, (size_t)d.N * d.hist_env_bytes, cudaMemcpyDeviceToHost)); out += (size_t)d.N * d.hist_env_bytes; }
   CU(cudaMemcpy(out, h->stats, STAT_COUNT * sizeof(double), cudaMemcpyDeviceToHost));
+  if (h->num_maps) {
+    out += STAT_COUNT * sizeof(double);
+    memcpy(out, &h->pool_digest, sizeof(uint64_t)); out += sizeof(uint64_t);
+    CU(cudaMemcpy(out, h->next_map, (size_t)d.N, cudaMemcpyDeviceToHost)); out += d.N;
+    CU(cudaMemcpy(out, h->cur_map, (size_t)d.N, cudaMemcpyDeviceToHost));
+  }
   return SNK_OK;
 }
 
@@ -990,14 +1089,30 @@ extern "C" int snk_checkpoint_load(snk_env* h, const void* blob_host, size_t byt
   const uint8_t* in = (const uint8_t*)blob_host;
   CkptHeader hd;
   memcpy(&hd, in, sizeof hd); in += sizeof hd;
-  if (hd.magic != CKPT_MAGIC || hd.N != d.N || hd.H != d.H || hd.W != d.W || hd.ns != d.ns || hd.K != d.K || hd.V != d.V ||
+  if (hd.magic != (h->num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC) && (hd.magic == CKPT_MAGIC || hd.magic == CKPT_MAGIC_POOL))
+    return fail(SNK_E_INVALID, h->num_maps ? "checkpoint was written by a handle without a wall-map pool"
+                                           : "checkpoint was written by a handle with a wall-map pool");
+  if (hd.magic != (h->num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC) || hd.N != d.N || hd.H != d.H || hd.W != d.W || hd.ns != d.ns || hd.K != d.K || hd.V != d.V ||
       hd.fs != d.fs || hd.dig != (d.dig | (d.compact << 1)) || hd.rec_bytes != d.hbm_rec_bytes || hd.hist_env_bytes != d.hist_env_bytes)
     return fail(SNK_E_INVALID, "checkpoint was written by a handle of a different shape");
+  const uint8_t* pool_part = in + (size_t)d.N * ((size_t)d.hbm_rec_bytes + (size_t)d.hist_env_bytes) + STAT_COUNT * sizeof(double);
+  if (h->num_maps) {
+    uint64_t digest;
+    memcpy(&digest, pool_part, sizeof digest);
+    if (digest != h->pool_digest) return fail(SNK_E_INVALID, "checkpoint was written by a handle with a different wall-map pool");
+    const uint8_t* cur = pool_part + sizeof(uint64_t) + d.N;
+    for (int e = 0; e < d.N; ++e)
+      if (cur[e] >= h->num_maps) return fail(SNK_E_INVALID, "checkpoint: cur_map[%d] = %d names no map", e, cur[e]);
+  }
   ON_DEVICE(h);
   CU(cudaDeviceSynchronize());
   CU(cudaMemcpy(h->recs, in, (size_t)d.N * d.hbm_rec_bytes, cudaMemcpyHostToDevice)); in += (size_t)d.N * d.hbm_rec_bytes;
   if (d.hist_env_bytes) { CU(cudaMemcpy(h->hist, in, (size_t)d.N * d.hist_env_bytes, cudaMemcpyHostToDevice)); in += (size_t)d.N * d.hist_env_bytes; }
   CU(cudaMemcpy(h->stats, in, STAT_COUNT * sizeof(double), cudaMemcpyHostToDevice));
+  if (h->num_maps) {
+    CU(cudaMemcpy(h->next_map, pool_part + sizeof(uint64_t), (size_t)d.N, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(h->cur_map, pool_part + sizeof(uint64_t) + d.N, (size_t)d.N, cudaMemcpyHostToDevice));
+  }
   h->was_reset = true;
   return SNK_OK;
 }

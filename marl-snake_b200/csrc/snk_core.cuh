@@ -26,8 +26,9 @@ enum : int { RNG_PHILOX = 0, RNG_REPLAY = 1 };
 enum : uint32_t { ERR_BAD_ACTION = 1, ERR_REPLAY_UNDERRUN = 2, ERR_REPLAY_RANGE = 4, ERR_SPAWN_GIVEUP = 8,
                   ERR_INTERNAL = 16,       // a bounds / alignment check of the debug build (-DSNK_DEBUG_CHECKS) failed
                   ERR_TMA_TIMEOUT = 32,    // a record tile's bulk copy did not land within two seconds; tile skipped
-                  ERR_STATE = 64 };        // compact records: set_state grid is not walls + fruits + live snakes, or more
+                  ERR_STATE = 64,          // compact records: set_state grid is not walls + fruits + live snakes, or more
                                            // fruit cells than the record has slots for
+                  ERR_MAP_RANGE = 128 };   // wall-map pool: a map id was not below the number of maps; map 0 was used
 enum : int { DRAW_STEP_FRUIT = 0, DRAW_SPAWN = 1, DRAW_RESET_FRUIT = 2 };
 enum : int { STAT_EPISODES = 0, STAT_RETURN, STAT_EP_STEPS, STAT_FRUITS, STAT_KILLS, STAT_DEATHS,
              STAT_ENV_STEPS, STAT_COUNT = 8 };

@@ -241,21 +241,39 @@ __device__ __forceinline__ void dirp_set_atomic(uint8_t* dirp, int c, int v) {
   atomicOr(w, (uint32_t)v << sh);
 }
 
+// Wall-map pool: the map id `m` read from a caller-written array, checked.  An id that is not a map raises the sticky
+// ERR_MAP_RANGE bit and reads as map 0, so a bad id never leads to a read outside the pool.
+__device__ __forceinline__ uint32_t checked_map(const KParams& p, uint32_t m) {
+  if (m >= (uint32_t)p.num_maps) { atomicOr(p.err, ERR_MAP_RANGE); m = 0u; }
+  return m;
+}
+
 // SnakeEnv.reset for one environment record in shared memory      envs/snake_env.py:131-159, 576-596
+// kPool: the handle has a wall-map pool; the environment's next_map picks the layout and the spawn table, and becomes
+// its cur_map.
+template <bool kPool>
 __device__ __noinline__ void reset_env_warp(const KParams& p, uint8_t* g, uint8_t* vb, uint32_t env_local) {
   const Dims& d = p.d;
   const Rec r = rec_view2(g, vb + d.off_c0, d);
   const uint32_t lane = lane_id();
   // values read inside loops live in registers (see place_fruits_warp); what a rare branch reads once stays in `p`
   const int ns = d.ns, K = d.K, W = d.W, H = d.H, rng_mode = d.rng_mode;
-  const uint32_t n_cand = d.n_cand, inv_row_words = p.inv_row_words;
-  const uint64_t* const spawn = p.spawn;
+  uint32_t m = 0;
+  if constexpr (kPool) {
+    if (lane == 0) {
+      m = checked_map(p, p.next_map[env_local]);
+      p.cur_map[env_local] = (uint8_t)m;
+    }
+    m = __shfl_sync(0xffffffffu, m, 0);
+  }
+  const uint32_t n_cand = kPool ? p.map_tab[m].y : d.n_cand, inv_row_words = p.inv_row_words;
+  const uint64_t* const spawn = kPool ? p.spawn + p.map_tab[m].x : p.spawn;
   SNK_R(0);
   if (d.compact) for (int j = (int)lane; j < d.fcap; j += 32) r.fruit[j] = 0;
   // make_grid: walled empty box (core/grid_util.py:14-20), one grid row at a time so no division is needed --
-  // or the handle's custom wall layout (snk_create_map), copied word by word from its L2-resident plane
-  if (p.wall_map) {
-    const uint32_t* const wm = p.wall_map;
+  // or the handle's custom wall layout (snk_create_map, or the pool's map), copied word by word from its L2-resident plane
+  if (kPool || p.wall_map) {
+    const uint32_t* const wm = kPool ? reinterpret_cast<const uint32_t*>(p.pool + (size_t)m * d.off_c0) : p.wall_map;
     const int HW = d.HW, nfull = HW >> 2;
     uint32_t* gw = reinterpret_cast<uint32_t*>(r.grid);
     for (int j = (int)lane; j < nfull; j += 32) gw[j] = __ldg(wm + j);
@@ -670,7 +688,7 @@ __device__ __forceinline__ void expand_tile(const KParams& p, const SH& sh, cons
 
 // ---- one warp: rules + terminal info + rollout statistics + rare events for a tile ----------------
 // Leaves per-environment flags in s_flag[] (F_RESET / F_INIT / F_SKIP).
-template <class SH>
+template <bool kPool, class SH>
 __device__ __forceinline__ void tile_rules(const KParams& p, const SH& sh, const TilePtr& tp, int e0, int ne,
                                            uint8_t* s_flag, uint32_t action, int t) {
   const Dims& d = p.d;
@@ -755,7 +773,7 @@ __device__ __forceinline__ void tile_rules(const KParams& p, const SH& sh, const
     const int qf = __shfl_sync(FULL, fruit, src);
     const int qflag = __shfl_sync(FULL, (int)flag, src);
     if (qf) place_fruits_warp(p, tp.G(q), tp.VB(q), (uint32_t)(e0 + q), qf, DRAW_STEP_FRUIT);
-    if (qflag & F_RESET) reset_env_warp(p, tp.G(q), tp.VB(q), (uint32_t)(e0 + q));
+    if (qflag & F_RESET) reset_env_warp<kPool>(p, tp.G(q), tp.VB(q), (uint32_t)(e0 + q));
   }
   __syncwarp();
 }
@@ -1308,11 +1326,16 @@ __device__ __forceinline__ void encode_env_stacked(const KParams& p, const SH& s
 //         slower on a 131 072-env shard (profiles/r02_ab_tiles3.txt); the launch picks by batch size (KParams::bigreg).
 //         Only while the observation writes are bound by DRAM: into a compressible block (snk_alloc_obs) the capped
 //         instance is 11 % faster at cfg5 (0.671 against 0.758 ms, profiles/r03_retune.txt), and the step picks it.
-// Warp-private instances of variants 0 and 1 are capped at 64 registers (eight 128-thread CTAs per SM).
+//       4, 5, 6 variants 0, 1, 2 of a handle with a wall-map pool (snk_create_maps, KParams::pool): compact tiles paint
+//         each environment's grid from its own map, resets pick the map from next_map.  Handles without a pool run
+//         variants 0..3, which hold none of that code.
+// Warp-private instances of variants 0, 1, 4 and 5 are capped at 64 registers (eight 128-thread CTAs per SM).
 template <int kNS, int kW, int kOH, int kOW, int kFS, bool kCoop, int kEnc, int kVar>
-__global__ void __launch_bounds__(kCoop ? SNK_MAX_THREADS_COOP : SNK_MAX_THREADS, (!kCoop && kVar <= 1) ? 8 : (!kCoop && kVar == 3) ? 1 : 0)
+__global__ void __launch_bounds__(kCoop ? SNK_MAX_THREADS_COOP : SNK_MAX_THREADS, (!kCoop && (kVar & 3) <= 1) ? 8 : (!kCoop && kVar == 3) ? 1 : 0)
 snk_tile_kernel(const __grid_constant__ KParams p) {
-  constexpr bool kBits = kVar == 1 || kVar == 2, kMulti = kVar == 2;
+  constexpr bool kPool = kVar >= 4;
+  constexpr int kV = kPool ? kVar - 4 : kVar;             // the variant apart from the pool
+  constexpr bool kBits = kV == 1 || kV == 2, kMulti = kV == 2;
   uint8_t* const bits_out = kBits ? p.bits : nullptr;
   extern __shared__ __align__(16) uint8_t smem[];
   const Dims& d = p.d;
@@ -1373,9 +1396,21 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
         mbar_expect_tx(mbar, tile_load_bytes + grid_load_bytes + hist_load_bytes + (blob_by_tma ? (uint32_t)p.enc_copy_bytes : 0u));
         if (p.l2_keep) bulk_load_hint(rec32, p.recs + (size_t)e0 * d.hbm_rec_bytes, tile_load_bytes, mbar, l2_policy_evict_last(p.l2_keep_frac));
         else bulk_load(rec32, p.recs + (size_t)e0 * d.hbm_rec_bytes, tile_load_bytes, mbar);
-        if (grid_load_bytes) bulk_load((uint32_t)__cvta_generic_to_shared(s_rec), p.base_grid, grid_load_bytes, mbar);
+        if (!kPool && grid_load_bytes) bulk_load((uint32_t)__cvta_generic_to_shared(s_rec), p.base_grid, grid_load_bytes, mbar);
         if (hist_load_bytes) bulk_load((uint32_t)__cvta_generic_to_shared(s_hist), p.hist + (size_t)e0 * d.hist_env_bytes, hist_load_bytes, mbar);
         if (blob_by_tma) bulk_load((uint32_t)__cvta_generic_to_shared(s_lut), p.enc_blob, (uint32_t)p.enc_copy_bytes, mbar);
+      }
+    }
+    if constexpr (kPool) {
+      // one bulk copy per environment from its own map, issued by the environment's lane of the electing warp once
+      // the barrier is armed (the same expect_tx total as the single-layout copy)
+      if (grid_load_bytes && (!kCoop || warp == 0)) {
+        __syncwarp();
+        if ((int)lane < ne) {
+          const uint32_t m = checked_map(p, p.cur_map[e0 + (int)lane]);
+          bulk_load((uint32_t)__cvta_generic_to_shared(s_rec) + lane * (uint32_t)d.off_c0, p.pool + (size_t)m * d.off_c0,
+                    (uint32_t)d.off_c0, mbar);
+        }
       }
     }
   } else {
@@ -1387,7 +1422,14 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
     const uint4* gsrc = reinterpret_cast<const uint4*>(p.base_grid);
     uint4* gdst = reinterpret_cast<uint4*>(s_rec);
     const int g16 = (int)(grid_load_bytes >> 4);
-    if (kCoop) { for (int k = tid; k < g16; k += nt) gdst[k] = __ldg(gsrc + k); }
+    if constexpr (kPool) {       // unit k of the tile's grids is unit k % (off_c0 / 16) of environment k / (off_c0 / 16)'s map
+      const int u16 = d.off_c0 >> 4;
+      for (int k = kCoop ? tid : (int)lane; k < g16; k += kCoop ? nt : 32) {
+        const int q = k / u16;
+        const uint32_t m = checked_map(p, p.cur_map[e0 + q]);
+        gdst[k] = __ldg(reinterpret_cast<const uint4*>(p.pool + (size_t)m * d.off_c0) + (k - q * u16));
+      }
+    } else if (kCoop) { for (int k = tid; k < g16; k += nt) gdst[k] = __ldg(gsrc + k); }
     else { for (int k = (int)lane; k < g16; k += 32) gdst[k] = __ldg(gsrc + k); }
     const uint4* hsrc = reinterpret_cast<const uint4*>(p.hist + (size_t)e0 * d.hist_env_bytes);
     uint4* hdst = reinterpret_cast<uint4*>(s_hist);
@@ -1453,7 +1495,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
       action = (g < ne && i < ns) ? __ldg(p.actions + ((size_t)t * d.N + e0 + g) * ns + i) : 0u;
     }
     if (d.compact && t == 0 && ne > 0) expand_tile(p, sh, tp, ne);
-    if (ne > 0) tile_rules(p, sh, tp, e0, ne, s_flag, action, t);
+    if (ne > 0) tile_rules<kPool>(p, sh, tp, e0, ne, s_flag, action, t);
     if (kEnc == ENC_REG && ne > 0) {           // crop origin + out-of-grid rows / columns of every viewer of the tile
       const int g = (int)lane / G, i = (int)lane - g * G;
       if (g < ne && i < ns) s_view[lane] = make_viewer_word(p, sh, tp.VB(g), i);
@@ -1533,7 +1575,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
     } else if (render) {
       // viewer pairs (encode_env_pairs): warp-private ENC_REG tiles writing NHWC bytes only, odd window, even
       // viewer count, 16-byte aligned environment blocks
-      constexpr bool kPairable = kEnc == ENC_REG && !kCoop && !(kVar == 1) && (kOH * kOW == 0 || ((kOH * kOW) & 1)) &&
+      constexpr bool kPairable = kEnc == ENC_REG && !kCoop && !(kV == 1) && (kOH * kOW == 0 || ((kOH * kOW) & 1)) &&
                                  (kNS == 0 || (kNS & 1) == 0);
       const bool pairs = kPairable && obs_t && !bits_t && p.vec16 && (ohw & 1) && (ns & 1) == 0;
       if (kEnc == ENC_REG && !cw_ready) { cw = pairs ? make_pair_cell_words(sh) : make_cell_words(sh, sh.view_bits()); cw_ready = true; }
@@ -1641,12 +1683,23 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
 }
 
 // ---- state export / import (parity + checkpoint interface; thread per environment) ----------------
-// Compact handles keep no grid in HBM: `base_grid` is the handle's wall layout, the caller's array receives the rebuilt
-// grid (walls + fruit slots + live bodies walked from the tail).  r.grid is never dereferenced for them.
+// Compact handles keep no grid in HBM: `base_grid` (or, with a wall-map pool, the pool slot of the environment's cur_map)
+// is the wall layout, the caller's array receives the rebuilt grid (walls + fruit slots + live bodies walked from the
+// tail).  r.grid is never dereferenced for them.
+__device__ __forceinline__ const uint8_t* env_walls(const Dims& d, const uint8_t* base_grid, const MapView& mv, int e,
+                                                    uint32_t* err) {
+  if (!mv.pool) return base_grid;
+  uint32_t m = mv.map_ids[e];
+  if (m >= (uint32_t)mv.num_maps) { atomicOr(err, ERR_MAP_RANGE); m = 0u; }
+  if (mv.cur_out) mv.cur_out[e] = (uint8_t)m;
+  return mv.pool + (size_t)m * d.off_c0;
+}
+
 __global__ void snk_get_state_kernel(const Dims d, const uint8_t* __restrict__ recs, const uint8_t* __restrict__ base_grid,
-                                     StateView sv) {
+                                     const MapView mv, uint32_t* err, StateView sv) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= d.N) return;
+  base_grid = env_walls(d, base_grid, mv, e, err);
   uint8_t* hb = const_cast<uint8_t*>(recs) + (size_t)e * d.hbm_rec_bytes;
   Rec r = rec_view2(hb, hb + d.hbm_c0, d);
   if (sv.grid && !d.compact) for (int c = 0; c < d.HW; ++c) sv.grid[(size_t)e * d.HW + c] = (uint8_t)cell_code(d, r.grid[c]);
@@ -1690,12 +1743,19 @@ __global__ void snk_get_state_kernel(const Dims d, const uint8_t* __restrict__ r
 }
 
 __global__ void snk_set_state_kernel(const Dims d, uint8_t* __restrict__ recs, const uint8_t* __restrict__ base_grid,
-                                     uint32_t* __restrict__ err, StateView sv) {
+                                     const MapView mv, uint32_t* __restrict__ err, StateView sv) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= d.N) return;
+  base_grid = env_walls(d, base_grid, mv, e, err);      // set_state starts an episode on next_map, as a reset does
   uint8_t* hb = recs + (size_t)e * d.hbm_rec_bytes;
   Rec r = rec_view2(hb, hb + d.hbm_c0, d);
   if (!d.compact) for (int c = 0; c < d.HW; ++c) r.grid[c] = sv.grid[(size_t)e * d.HW + c];
+  if (!d.compact && mv.pool) {
+    // a wall-map pool names the layout of every episode (cur_map): the grid's walls must be exactly that map's
+    bool bad = false;
+    for (int c = 0; c < d.HW; ++c) bad |= (sv.grid[(size_t)e * d.HW + c] == (uint8_t)WALL) != (base_grid[c] == (uint8_t)WALL);
+    if (bad) atomicOr(err, ERR_STATE);
+  }
   if (d.compact) {
     // the record stores the fruit cells and the bodies; whatever else the caller's grid holds must be what they imply
     const uint8_t* in = sv.grid + (size_t)e * d.HW;
@@ -1903,6 +1963,11 @@ static cudaError_t launch_variant(const KParams& p, int threads, size_t smem_byt
 
 template <int kNS, int kW, int kOH, int kOW, int kFS, bool kCoop, int kEnc>
 static cudaError_t launch_instance(const KParams& p, int threads, size_t smem_bytes, cudaStream_t stream) {
+  if (p.pool) {                 // wall-map pool: variants 4 / 5 / 6 (no uncapped pool instance is built)
+    if (p.T > 1) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 6>(p, threads, smem_bytes, stream);
+    if (p.bits) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 5>(p, threads, smem_bytes, stream);
+    return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 4>(p, threads, smem_bytes, stream);
+  }
   if (p.T > 1) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 2>(p, threads, smem_bytes, stream);
   if (p.bits) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 1>(p, threads, smem_bytes, stream);
   if constexpr (!kCoop) {
@@ -1944,12 +2009,14 @@ cudaError_t launch_tile_kernel(const KParams& p, int threads, size_t smem_bytes,
   }
 }
 
-cudaError_t launch_get_state(const Dims& d, const uint8_t* recs, const uint8_t* base_grid, const StateView& sv, cudaStream_t s) {
-  snk_get_state_kernel<<<(d.N + 127) / 128, 128, 0, s>>>(d, recs, base_grid, sv);
+cudaError_t launch_get_state(const Dims& d, const uint8_t* recs, const uint8_t* base_grid, const MapView& mv, uint32_t* err,
+                             const StateView& sv, cudaStream_t s) {
+  snk_get_state_kernel<<<(d.N + 127) / 128, 128, 0, s>>>(d, recs, base_grid, mv, err, sv);
   return cudaGetLastError();
 }
-cudaError_t launch_set_state(const Dims& d, uint8_t* recs, const uint8_t* base_grid, uint32_t* err, const StateView& sv, cudaStream_t s) {
-  snk_set_state_kernel<<<(d.N + 127) / 128, 128, 0, s>>>(d, recs, base_grid, err, sv);
+cudaError_t launch_set_state(const Dims& d, uint8_t* recs, const uint8_t* base_grid, const MapView& mv, uint32_t* err,
+                             const StateView& sv, cudaStream_t s) {
+  snk_set_state_kernel<<<(d.N + 127) / 128, 128, 0, s>>>(d, recs, base_grid, mv, err, sv);
   return cudaGetLastError();
 }
 cudaError_t launch_pack_obs(const uint8_t* obs, uint8_t* bits, size_t n_units, cudaStream_t s) {

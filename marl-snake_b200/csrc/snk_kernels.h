@@ -73,6 +73,12 @@ struct KParams {
   int32_t bigreg;              // warp-private tiles, batch many waves deep: run the instance compiled without a register cap
   int32_t T;                   // steps per launch (snk_step_many; frame_stack 1).  actions / rewards / dones / extras are
   int32_t obs_every_step;      //   [T, ...]; obs / bits are [T, ...] when obs_every_step, else the last step's block only
+  // wall-map pool (snk_create_maps); pool == null for every other handle, which then runs the instances without it
+  const uint8_t* pool;         // [num_maps][off_c0] wall layouts (cell codes EMPTY / WALL, zero padded)
+  const uint2* map_tab;        // [num_maps] {first pose in `spawn`, number of poses} of each map's spawn table
+  const uint8_t* next_map;     // [N] map a reset of env e starts from (written by the caller)
+  uint8_t* cur_map;            // [N] map of env e's current episode (written by every reset)
+  int32_t num_maps;
 };
 
 struct StateView {
@@ -89,8 +95,13 @@ size_t pad_plane_bytes(const Dims& d, int tile_envs);     // ENC_PAD: padded pla
 size_t encode_blob_bytes(const Dims& d, size_t* tab_off, size_t* lutb_off);
 void encode_blob_fill(const Dims& d, uint8_t* out);
 cudaError_t launch_tile_kernel(const KParams& p, int threads, size_t smem_bytes, cudaStream_t stream);
-cudaError_t launch_get_state(const Dims& d, const uint8_t* recs, const uint8_t* base_grid, const StateView& sv, cudaStream_t s);
-cudaError_t launch_set_state(const Dims& d, uint8_t* recs, const uint8_t* base_grid, uint32_t* err, const StateView& sv, cudaStream_t s);
+// Wall layout of each environment: base_grid for every environment, or -- wall-map pool -- pool slot map_ids[e]
+// (cur_map for get_state, next_map for set_state, which also copies it to cur_map)
+struct MapView { const uint8_t* pool; const uint8_t* map_ids; uint8_t* cur_out; int32_t num_maps; };
+cudaError_t launch_get_state(const Dims& d, const uint8_t* recs, const uint8_t* base_grid, const MapView& mv, uint32_t* err,
+                             const StateView& sv, cudaStream_t s);
+cudaError_t launch_set_state(const Dims& d, uint8_t* recs, const uint8_t* base_grid, const MapView& mv, uint32_t* err,
+                             const StateView& sv, cudaStream_t s);
 cudaError_t launch_init_records(const Dims& d, uint8_t* recs, cudaStream_t s);
 // obs: n_units * 8 bytes of 0/1 (16-byte aligned) -> bits: n_units bytes, bit c = byte c of the unit
 cudaError_t launch_pack_obs(const uint8_t* obs, uint8_t* bits, size_t n_units, cudaStream_t s);

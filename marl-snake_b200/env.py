@@ -33,13 +33,35 @@ class SnakeBatch:
     def __init__(self, num_envs, height=20, width=20, num_snakes=4, snake_length=3, vision_range=None,
                  frame_stack=1, observer='snake', reward_dict=None, num_fruits=None,
                  max_episode_steps=DEFAULT_MAX_EPISODE_STEPS, device=0, seed=0, rng='philox',
-                 auto_reset=True, env_id_offset=0, done_mode='all', wall_map=None, **ignored):
+                 auto_reset=True, env_id_offset=0, done_mode='all', wall_map=None, wall_maps=None, map_ids=None,
+                 **ignored):
+        """wall_map: one custom wall layout for every env.  wall_maps: a pool of layouts of one shape (a list of arrays or
+        map paths, or an [M, H, W] array; 1 <= M <= 256); each env starts every episode on the map its `next_maps`
+        entry names at that reset (see next_maps / current_maps).  map_ids: initial next_maps (M ids), default
+        (env_id_offset + e) % M."""
         reward_dict = DEFAULT_REWARD_DICT if reward_dict is None else reward_dict
         self.wall_map = None
+        self.wall_maps = None
+        if wall_map is not None and wall_maps is not None:
+            raise ValueError('give either wall_map (one layout) or wall_maps (a pool of layouts), not both')
         if wall_map is not None:                      # custom wall layout: the map decides the grid shape
             from .grid_util import as_wall_plane
             self.wall_map = as_wall_plane(wall_map)
             height, width = self.wall_map.shape
+        if wall_maps is not None:                     # wall-map pool: the maps decide the grid shape
+            from .grid_util import as_wall_plane
+            maps = [wall_maps] if isinstance(wall_maps, (str, bytes)) or hasattr(wall_maps, '__fspath__') else wall_maps
+            if isinstance(maps, np.ndarray) and maps.ndim == 3 or isinstance(maps, torch.Tensor) and maps.dim() == 3:
+                maps = list(np.asarray(maps.cpu() if isinstance(maps, torch.Tensor) else maps))
+            planes = [as_wall_plane(m) for m in maps]
+            if not 1 <= len(planes) <= _lib.SNK_MAX_MAPS:
+                raise ValueError(f'wall_maps must hold 1..{_lib.SNK_MAX_MAPS} layouts, got {len(planes)}')
+            if len({p.shape for p in planes}) != 1:
+                raise ValueError(f'every map of wall_maps must have one shape, got {sorted({p.shape for p in planes})}')
+            self.wall_maps = np.ascontiguousarray(np.stack(planes))
+            height, width = self.wall_maps.shape[1:]
+        elif map_ids is not None:
+            raise ValueError('map_ids needs wall_maps')
         if reward_dict.keys() != DEFAULT_REWARD_DICT.keys():                      # snake_env.py:77-80
             raise KeyError(f'reward dict keys must correspond to {DEFAULT_REWARD_DICT.keys()}')
         if observer not in ('snake', 'human'):
@@ -76,7 +98,17 @@ class SnakeBatch:
                         reward_time=float(reward_dict['time']))
         self._h = C.c_void_p()
         with torch.cuda.device(self.device):
-            if self.wall_map is None:
+            if self.wall_maps is not None:
+                ids = None
+                if map_ids is not None:
+                    ids = np.asarray(map_ids.cpu() if isinstance(map_ids, torch.Tensor) else map_ids).reshape(-1)
+                    if ids.size != self.num_envs or ids.min(initial=0) < 0 or ids.max(initial=0) >= len(self.wall_maps):
+                        raise ValueError(f'map_ids must hold one id in 0..{len(self.wall_maps) - 1} per environment')
+                    ids = np.ascontiguousarray(ids, dtype=np.uint8)
+                check(lib.snk_create_maps(C.byref(cfg), len(self.wall_maps), self.wall_maps.ctypes.data_as(C.c_void_p),
+                                          ids.ctypes.data_as(C.c_void_p) if ids is not None else None,
+                                          C.byref(self._h)))
+            elif self.wall_map is None:
                 check(lib.snk_create(C.byref(cfg), C.byref(self._h)))
             else:
                 check(lib.snk_create_map(C.byref(cfg), self.wall_map.ctypes.data_as(C.c_void_p), C.byref(self._h)))
@@ -108,6 +140,16 @@ class SnakeBatch:
         self._mutations = 0
         self._obs_stale = 'construction (no reset yet)'
         self._rollout_alive = self._rollout_age = self._rollout_mark = None
+        self.num_maps = int(lib.snk_num_maps(self._h))
+        self.next_maps = self.current_maps = None
+        if self.num_maps:
+            nxt, cur = C.c_void_p(), C.c_void_p()
+            check(lib.snk_map_ids_dev(self._h, C.byref(nxt), C.byref(cur)))
+            # views of the handle's own uint8 [N] id arrays, valid until close().  next_maps[e]: the map env e's next
+            # reset starts from (rewrite it freely, e.g. next_maps.random_(0, num_maps) after every step);
+            # current_maps[e]: the map of env e's current episode, set from next_maps by every reset
+            self.next_maps = _tensor_from_ptr(nxt.value, N, torch.uint8, dev)
+            self.current_maps = _tensor_from_ptr(cur.value, N, torch.uint8, dev)
 
     @property
     def obs_compressed(self):
@@ -320,6 +362,8 @@ class SnakeBatch:
         view = SnkStateView(**{k: v.data_ptr() for k, v in st.items()}, max_cells=int(max_cells or 0))
         check(lib.snk_get_state(self._h, C.byref(view), self._stream()))
         st['grid'] = st['grid'].view(N, H, W)
+        if self.num_maps:
+            st['map'] = self.current_maps.clone()           # the wall map of each env's current episode
         return st
 
     def set_state(self, grid, alive, dir, length, cells, alive_counter, episode_length=None):
@@ -429,8 +473,8 @@ def _tensor_from_ptr(ptr, n, dtype, device):
         pass
     h = _Holder()
     itemsize = torch.empty((), dtype=dtype).element_size()
-    h.__cuda_array_interface__ = dict(shape=(n,), typestr={8: '<f8', 4: '<f4'}[itemsize], data=(ptr, False),
-                                      version=2)
+    typestr = '|u1' if dtype == torch.uint8 else {8: '<f8', 4: '<f4'}[itemsize]
+    h.__cuda_array_interface__ = dict(shape=(n,), typestr=typestr, data=(ptr, False), version=2)
     return torch.as_tensor(h, device=device)
 
 
