@@ -197,6 +197,23 @@ int snk_step_many(snk_env* env, int32_t num_steps, const uint8_t* actions_dev, u
                   int32_t obs_every_step, double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* extra,
                   void* stream);
 
+/* GLOBAL STATE for centralized critics and mixers (MAPPO, QMIX, ...): the three calls above, plus grid_dev, uint8
+ * [N, H*W] row-major -- the format of snk_state_view.grid, i.e. the reference's SnakeEnv.grid (cell codes
+ * type + 10 * owner, no direction bits).  Row e is env e's grid as the returned observation was encoded from it: for
+ * an env that auto-reset in this step, the grid of the new episode; after a masked reset, every env's row (the
+ * others' unchanged grids); with a wall-map pool, on the walls of the env's cur_map.  The step kernel stores the rows
+ * from shared memory as it stores the records, so no second launch reads the records again.  obs_dev, bits_dev and
+ * grid_dev may each be NULL, in any combination; grid_dev may have any alignment (16-byte aligned is fastest).
+ * snk_step_many_grid: grid_dev is [T, N, H*W] when obs_every_step != 0, else the last step's [N, H*W].  With grid_dev
+ * NULL each call equals its counterpart. */
+int snk_reset_grid(snk_env* env, const uint8_t* mask_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
+                   void* stream);
+int snk_step_grid(snk_env* env, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
+                  double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* extra, void* stream);
+int snk_step_many_grid(snk_env* env, int32_t num_steps, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev,
+                       uint8_t* grid_dev, int32_t obs_every_step, double* rewards_dev, uint8_t* dones_dev,
+                       const snk_step_extra* extra, void* stream);
+
 /* Same call with HOST buffers (the reference's step() takes and returns host objects,
  * snake_env.py:414): copies actions in, steps, copies obs / rewards / dones out and synchronises.
  * Pinned buffers make the copies asynchronous to the host until the final synchronise.  obs_host may

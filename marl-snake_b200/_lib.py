@@ -69,6 +69,11 @@ PROTOTYPES = {
                                 C.POINTER(SnkStepExtra), C.c_void_p]),
     'snk_step_many': (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
                                 C.c_void_p, C.POINTER(SnkStepExtra), C.c_void_p]),
+    'snk_reset_grid': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'snk_step_grid': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.POINTER(SnkStepExtra), C.c_void_p]),
+    'snk_step_many_grid': (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                     C.c_void_p, C.c_void_p, C.POINTER(SnkStepExtra), C.c_void_p]),
     'snk_step_host': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     'snk_step_host_info': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.POINTER(SnkStepExtra)]),

@@ -489,10 +489,11 @@ extern "C" int snk_note_stream(snk_env* h, void* stream) {
   return SNK_OK;
 }
 
-static int reset_impl(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, uint8_t* bits_dev, cudaStream_t stream) {
+static int reset_impl(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
+                      cudaStream_t stream) {
   if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
   KParams p = base_params(h);
-  p.mode = MODE_RESET; p.mask = mask_dev; p.obs = obs_dev; p.bits = bits_dev;
+  p.mode = MODE_RESET; p.mask = mask_dev; p.obs = obs_dev; p.bits = bits_dev; p.grid_out = grid_dev;
   p.vec16 = check_vec16(h, obs_dev);
   CU(launch_tile_kernel(p, h->threads, h->smem_bytes, stream));
   note_user_stream(h, stream);
@@ -500,15 +501,15 @@ static int reset_impl(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, uin
   return SNK_OK;
 }
 
-static int step_impl(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, double* rewards_dev,
-                     uint8_t* dones_dev, const snk_step_extra* x, cudaStream_t stream) {
+static int step_impl(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
+                     double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* x, cudaStream_t stream) {
   if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
   if (!h->was_reset) return fail(SNK_E_STATE, "step before reset");
   if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
   if ((uintptr_t)rewards_dev & 7) return fail(SNK_E_INVALID, "rewards must be 8-byte aligned");
   KParams p = base_params(h);
   p.mode = MODE_STEP;
-  p.actions = actions_dev; p.obs = obs_dev; p.bits = bits_dev; p.rew = rewards_dev; p.done = dones_dev;
+  p.actions = actions_dev; p.obs = obs_dev; p.bits = bits_dev; p.grid_out = grid_dev; p.rew = rewards_dev; p.done = dones_dev;
   if (x) {
     p.fin = x->finished; p.rank = x->rank; p.ep_scores = x->episode_scores;
     p.ep_steps = x->episode_steps; p.ep_fruits = x->episode_fruits; p.ep_kills = x->episode_kills;
@@ -517,7 +518,9 @@ static int step_impl(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, u
   // An observation block in compressible memory costs the step far less DRAM time, and the step is then bound by the
   // latency of its rule phase: the 64-register instance, with twice the resident warps, is the faster one there
   // (cfg5, 1 048 576 envs on a B200 at 1000 W: 0.671 ms against 0.758 ms uncapped; profiles/r03_retune.txt).
-  if (p.bigreg && obs_dev && in_compressible_block(obs_dev)) p.bigreg = 0;
+  // (A step that writes the global state runs a capped instance in any case: the grid variants have no uncapped one.)
+  const uint8_t* out_dev = obs_dev ? obs_dev : grid_dev;
+  if (p.bigreg && out_dev && in_compressible_block(out_dev)) p.bigreg = 0;
   CU(launch_tile_kernel(p, h->threads, h->smem_bytes, stream));
   note_user_stream(h, stream);
   return SNK_OK;
@@ -525,8 +528,8 @@ static int step_impl(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, u
 
 // T steps in one call.  frame_stack 1: ONE launch, every tile's records stay in shared memory for all T steps.
 // frame_stack > 1 (the frame history is written per step): T ordinary launches -- same results, same arrays.
-static int step_many_impl(snk_env* h, int T, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, int every,
-                          double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* x, cudaStream_t stream) {
+static int step_many_impl(snk_env* h, int T, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
+                          int every, double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* x, cudaStream_t stream) {
   if (T < 1 || T > 65536) return fail(SNK_E_INVALID, "num_steps must be in 1..65536");
   const Dims& d = h->d;
   const size_t nn = (size_t)d.N * d.ns;
@@ -539,7 +542,7 @@ static int step_many_impl(snk_env* h, int T, const uint8_t* actions_dev, uint8_t
     const bool many = T > 1;
     if (many) p.E = h->many_tile_envs;
     p.mode = MODE_STEP; p.T = T; p.obs_every_step = every ? 1 : 0;
-    p.actions = actions_dev; p.obs = obs_dev; p.bits = bits_dev; p.rew = rewards_dev; p.done = dones_dev;
+    p.actions = actions_dev; p.obs = obs_dev; p.bits = bits_dev; p.grid_out = grid_dev; p.rew = rewards_dev; p.done = dones_dev;
     p.vec16 = check_vec16(h, obs_dev);          // the per-step blocks of obs_every_step are whole environment blocks apart
     if (x) {
       p.fin = x->finished; p.rank = x->rank; p.ep_scores = x->episode_scores;
@@ -563,7 +566,8 @@ static int step_many_impl(snk_env* h, int T, const uint8_t* actions_dev, uint8_t
     const bool render = every || t == T - 1;
     uint8_t* o = (obs_dev && render) ? obs_dev + (every ? (size_t)t * d.N * d.obs_env_bytes : 0) : nullptr;
     uint8_t* b = (bits_dev && render) ? bits_dev + (every ? (size_t)t * d.N * d.stage_env_bytes : 0) : nullptr;
-    int rc = step_impl(h, actions_dev + t * nn, o, b, rewards_dev + t * nn, dones_dev + t * nn, x ? &xt : nullptr, stream);
+    uint8_t* g = (grid_dev && render) ? grid_dev + (every ? (size_t)t * d.N * d.HW : 0) : nullptr;
+    int rc = step_impl(h, actions_dev + t * nn, o, b, g, rewards_dev + t * nn, dones_dev + t * nn, x ? &xt : nullptr, stream);
     if (rc) return rc;
   }
   return SNK_OK;
@@ -575,33 +579,58 @@ extern "C" int snk_step_many(snk_env* h, int32_t num_steps, const uint8_t* actio
   if (!h) return fail(SNK_E_INVALID, "null handle");
   if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
   ON_DEVICE(h);
-  return step_many_impl(h, num_steps, actions_dev, obs_dev, bits_dev, obs_every_step, rewards_dev, dones_dev, x, (cudaStream_t)stream);
+  return step_many_impl(h, num_steps, actions_dev, obs_dev, bits_dev, nullptr, obs_every_step, rewards_dev, dones_dev, x,
+                        (cudaStream_t)stream);
+}
+
+extern "C" int snk_step_many_grid(snk_env* h, int32_t num_steps, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev,
+                                  uint8_t* grid_dev, int32_t obs_every_step, double* rewards_dev, uint8_t* dones_dev,
+                                  const snk_step_extra* x, void* stream) {
+  if (!h) return fail(SNK_E_INVALID, "null handle");
+  if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
+  ON_DEVICE(h);
+  return step_many_impl(h, num_steps, actions_dev, obs_dev, bits_dev, grid_dev, obs_every_step, rewards_dev, dones_dev, x,
+                        (cudaStream_t)stream);
 }
 
 extern "C" int snk_reset(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, void* stream) {
   if (!h) return fail(SNK_E_INVALID, "null handle");
   ON_DEVICE(h);
-  return reset_impl(h, mask_dev, obs_dev, nullptr, (cudaStream_t)stream);
+  return reset_impl(h, mask_dev, obs_dev, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int snk_reset_bits(snk_env* h, const uint8_t* mask_dev, uint8_t* bits_dev, void* stream) {
   if (!h) return fail(SNK_E_INVALID, "null handle");
   ON_DEVICE(h);
-  return reset_impl(h, mask_dev, nullptr, bits_dev, (cudaStream_t)stream);
+  return reset_impl(h, mask_dev, nullptr, bits_dev, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int snk_reset_grid(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
+                              void* stream) {
+  if (!h) return fail(SNK_E_INVALID, "null handle");
+  ON_DEVICE(h);
+  return reset_impl(h, mask_dev, obs_dev, bits_dev, grid_dev, (cudaStream_t)stream);
 }
 
 extern "C" int snk_step(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, double* rewards_dev,
                         uint8_t* dones_dev, const snk_step_extra* x, void* stream) {
   if (!h) return fail(SNK_E_INVALID, "null handle");
   ON_DEVICE(h);
-  return step_impl(h, actions_dev, obs_dev, nullptr, rewards_dev, dones_dev, x, (cudaStream_t)stream);
+  return step_impl(h, actions_dev, obs_dev, nullptr, nullptr, rewards_dev, dones_dev, x, (cudaStream_t)stream);
 }
 
 extern "C" int snk_step_bits(snk_env* h, const uint8_t* actions_dev, uint8_t* bits_dev, double* rewards_dev,
                              uint8_t* dones_dev, const snk_step_extra* x, void* stream) {
   if (!h) return fail(SNK_E_INVALID, "null handle");
   ON_DEVICE(h);
-  return step_impl(h, actions_dev, nullptr, bits_dev, rewards_dev, dones_dev, x, (cudaStream_t)stream);
+  return step_impl(h, actions_dev, nullptr, bits_dev, nullptr, rewards_dev, dones_dev, x, (cudaStream_t)stream);
+}
+
+extern "C" int snk_step_grid(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
+                             double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* x, void* stream) {
+  if (!h) return fail(SNK_E_INVALID, "null handle");
+  ON_DEVICE(h);
+  return step_impl(h, actions_dev, obs_dev, bits_dev, grid_dev, rewards_dev, dones_dev, x, (cudaStream_t)stream);
 }
 
 static bool packed(const snk_env* h) { return h->xfer_mode == XFER_PACKED; }
@@ -707,7 +736,7 @@ static int step_host_small(snk_env* h, const SmallLayout& L, const uint8_t* acti
     xd.finished = dv + L.fin; xd.rank = (int32_t*)(dv + L.rank); xd.episode_scores = (double*)(dv + L.scores);
     xd.episode_steps = (int32_t*)(dv + L.counts); xd.episode_fruits = xd.episode_steps + nn; xd.episode_kills = xd.episode_fruits + nn;
   }
-  int rc = step_impl(h, dv + L.act, obs_host ? dv + L.obs : nullptr, nullptr, (double*)(dv + L.rew), dv + L.done, xh ? &xd : nullptr, s);
+  int rc = step_impl(h, dv + L.act, obs_host ? dv + L.obs : nullptr, nullptr, nullptr, (double*)(dv + L.rew), dv + L.done, xh ? &xd : nullptr, s);
   if (rc) return rc;
   const size_t lo = obs_host ? L.obs : L.rew, hi = xh ? L.total : L.fin;
   if (!zero_copy) CU(cudaMemcpyAsync(hv + lo, dv + lo, hi - lo, cudaMemcpyDeviceToHost, s));
@@ -758,7 +787,7 @@ extern "C" int snk_step_host_info(snk_env* h, const uint8_t* actions_host, uint8
     if (xh->episode_kills) xd.episode_kills = h->h_counts + 2 * nn;
   }
   CU(cudaMemcpyAsync(h->h_actions, actions_host, nn, cudaMemcpyHostToDevice, s));
-  rc = step_impl(h, h->h_actions, obs_host && !as_bits ? h->h_obs : nullptr, as_bits ? h->d_bits : nullptr, h->h_rew, h->h_done,
+  rc = step_impl(h, h->h_actions, obs_host && !as_bits ? h->h_obs : nullptr, as_bits ? h->d_bits : nullptr, nullptr, h->h_rew, h->h_done,
                  xh ? &xd : nullptr, s);
   if (rc) return rc;
   CU(cudaMemcpyAsync(rewards_host, h->h_rew, nn * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -787,7 +816,7 @@ extern "C" int snk_step_host_bits(snk_env* h, const uint8_t* actions_host, uint8
   const size_t nn = (size_t)d.N * d.ns, units = (size_t)d.N * d.stage_env_bytes;
   cudaStream_t s = h->own_stream;
   CU(cudaMemcpyAsync(h->h_actions, actions_host, nn, cudaMemcpyHostToDevice, s));
-  rc = step_impl(h, h->h_actions, nullptr, h->d_bits, h->h_rew, h->h_done, nullptr, s);   // channel bits straight from the encode
+  rc = step_impl(h, h->h_actions, nullptr, h->d_bits, nullptr, h->h_rew, h->h_done, nullptr, s);   // channel bits straight from the encode
   if (rc) return rc;
   CU(cudaMemcpyAsync(rewards_host, h->h_rew, nn * sizeof(double), cudaMemcpyDeviceToHost, s));
   CU(cudaMemcpyAsync(dones_host, h->h_done, nn, cudaMemcpyDeviceToHost, s));
@@ -810,7 +839,7 @@ extern "C" int snk_reset_host(snk_env* h, uint8_t* obs_host) {
   rc = own_stream_after_user_work(h);
   if (rc) return rc;
   cudaStream_t s = h->own_stream;
-  rc = reset_impl(h, nullptr, obs_host && !as_bits ? h->h_obs : nullptr, as_bits ? h->d_bits : nullptr, s);
+  rc = reset_impl(h, nullptr, obs_host && !as_bits ? h->h_obs : nullptr, as_bits ? h->d_bits : nullptr, nullptr, s);
   if (rc) return rc;
   if (obs_host) return obs_to_host(h, obs_host, s);
   CU(cudaStreamSynchronize(s));

@@ -1312,6 +1312,38 @@ __device__ __forceinline__ void encode_env_stacked(const KParams& p, const SH& s
   __syncwarp();
 }
 
+// ---- global state output (KParams::grid_out): the tile's final grids -> rows e0 .. e0+ne-1 of [N, H*W] -------------
+// bulk: compact records with H*W a multiple of 16 (off_c0 == H*W, so the tile's grids are ONE contiguous block, and
+// they carry no direction bits) and a 16-byte aligned output: one bulk copy by the tile's elected thread, after the
+// rule warp's fence.proxy.async; the issuer waits for its shared-memory reads before the CTA exits or the next step's
+// rules run.  Otherwise plain stores of cell codes (full records: stride rec_bytes, direction bits masked off).
+template <bool kCoop>
+__device__ __forceinline__ void store_grid_rows(const KParams& p, const TilePtr& tp, int e0, int ne, uint8_t* out,
+                                                bool bulk, bool elected) {
+  const Dims& d = p.d;
+  uint8_t* const rows = out + (size_t)e0 * d.HW;
+  if (bulk) {
+    if (elected) bulk_store(rows, (uint32_t)__cvta_generic_to_shared(tp.g), (uint32_t)(ne * d.HW));
+    return;
+  }
+  const int first = kCoop ? (int)threadIdx.x : (int)lane_id(), step = kCoop ? (int)blockDim.x : 32;
+  if (((d.HW | (int)reinterpret_cast<uintptr_t>(rows)) & 15) == 0) {
+    const uint32_t cm4 = (uint32_t)d.code_mask * 0x01010101u;
+    const int n16 = d.HW >> 4;
+    for (int k = first; k < ne * n16; k += step) {
+      const int q = k / n16;
+      uint4 v = reinterpret_cast<const uint4*>(tp.G(q))[k - q * n16];
+      v.x &= cm4; v.y &= cm4; v.z &= cm4; v.w &= cm4;
+      reinterpret_cast<uint4*>(rows)[k] = v;
+    }
+  } else {
+    for (int k = first; k < ne * d.HW; k += step) {
+      const int q = k / d.HW;
+      rows[k] = (uint8_t)cell_code(d, tp.G(q)[k - q * d.HW]);
+    }
+  }
+}
+
 // ---- the fused step / reset / encode kernel -------------------------------------------------------
 // kCoop = false: every warp owns its own tile (records in a private shared-memory slice), no block
 //                barrier after the table copy -- the mode for large batches.
@@ -1329,12 +1361,15 @@ __device__ __forceinline__ void encode_env_stacked(const KParams& p, const SH& s
 //       4, 5, 6 variants 0, 1, 2 of a handle with a wall-map pool (snk_create_maps, KParams::pool): compact tiles paint
 //         each environment's grid from its own map, resets pick the map from next_map.  Handles without a pool run
 //         variants 0..3, which hold none of that code.
-// Warp-private instances of variants 0, 1, 4 and 5 are capped at 64 registers (eight 128-thread CTAs per SM).
+//       8, 10 (12, 14 with a pool) variants 0 and 2 that also write the global state (KParams::grid_out): 8 / 12 the
+//         plain step with or without its NHWC observation, 10 / 14 everything else (channel bits, several steps).  Calls
+//         without grid_out run the variants above, which hold none of that code.
+// Warp-private instances of variants 0, 1, 4, 5, 8 and 12 are capped at 64 registers (eight 128-thread CTAs per SM).
 template <int kNS, int kW, int kOH, int kOW, int kFS, bool kCoop, int kEnc, int kVar>
 __global__ void __launch_bounds__(kCoop ? SNK_MAX_THREADS_COOP : SNK_MAX_THREADS, (!kCoop && (kVar & 3) <= 1) ? 8 : (!kCoop && kVar == 3) ? 1 : 0)
 snk_tile_kernel(const __grid_constant__ KParams p) {
-  constexpr bool kPool = kVar >= 4;
-  constexpr int kV = kPool ? kVar - 4 : kVar;             // the variant apart from the pool
+  constexpr bool kPool = (kVar & 4) != 0, kGrid = (kVar & 8) != 0;
+  constexpr int kV = kVar & 3;                            // the variant apart from the pool and the global state
   constexpr bool kBits = kV == 1 || kV == 2, kMulti = kV == 2;
   uint8_t* const bits_out = kBits ? p.bits : nullptr;
   extern __shared__ __align__(16) uint8_t smem[];
@@ -1486,9 +1521,13 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
   const int T = (kMulti && fs == 1 && p.mode == MODE_STEP) ? p.T : 1;
   CellWords cw;
   bool cw_ready = false;
+  const bool grid_bulk = kGrid && p.use_tma && d.compact && (d.HW & 15) == 0 && (reinterpret_cast<uintptr_t>(p.grid_out) & 15) == 0;
 #pragma unroll 1
   for (int t = 0; t < T; ++t) {
   const bool last = t == T - 1;
+  // this step's global state rows (every step of a multi-step launch, or only the last one, as the observation)
+  uint8_t* const grid_t = (kGrid && p.grid_out && (last || (kMulti && p.obs_every_step)))
+                              ? p.grid_out + ((kMulti && p.obs_every_step) ? (size_t)t * d.N * d.HW : 0) : nullptr;
   if (!kCoop || warp == 0) {
     if (t > 0) {
       const int g = (int)lane / G, i = (int)lane - g * G;
@@ -1508,13 +1547,16 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
         s_view[lane] = (uint32_t)((r0 + d.V) * sh.pad_pitch() + c0 + sh.pad_left());
       }
     }
-    if (p.use_tma && last) fence_proxy_async();   // the rules' shared-memory writes -> visible to the bulk store
+    if (p.use_tma && (last || (kGrid && grid_t))) fence_proxy_async();   // the rules' shared-memory writes -> visible to the bulk stores
     __syncwarp();
   }
   SNK_T(t_ruled);
   if (kCoop) __syncthreads();
   SNK_T(t_synced);
   if (ne == 0) return;
+  if constexpr (kGrid) {
+    if (grid_t) store_grid_rows<kCoop>(p, tp, e0, ne, grid_t, grid_bulk, elected);
+  }
 
   if (fs == 1) {
     // ---- write the records back: shared -> HBM (nothing below modifies them).  The bulk store runs
@@ -1632,6 +1674,9 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
       }
     }
     if (!last) {                                // the next step's rules rewrite the records and viewer words
+      if constexpr (kGrid) {                    // ... and the grids: this step's bulk store must have read them
+        if (grid_bulk && grid_t && elected) bulk_store_wait_read();
+      }
       if (kCoop) __syncthreads(); else __syncwarp();
       continue;
     }
@@ -1963,6 +2008,13 @@ static cudaError_t launch_variant(const KParams& p, int threads, size_t smem_byt
 
 template <int kNS, int kW, int kOH, int kOW, int kFS, bool kCoop, int kEnc>
 static cudaError_t launch_instance(const KParams& p, int threads, size_t smem_bytes, cudaStream_t stream) {
+  if (p.grid_out) {             // global state: variants 8 / 10, with a pool 12 / 14 (no uncapped copy like variant 3)
+    const bool general = p.T > 1 || p.bits;
+    if (p.pool) return general ? launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 14>(p, threads, smem_bytes, stream)
+                               : launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 12>(p, threads, smem_bytes, stream);
+    return general ? launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 10>(p, threads, smem_bytes, stream)
+                   : launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 8>(p, threads, smem_bytes, stream);
+  }
   if (p.pool) {                 // wall-map pool: variants 4 / 5 / 6 (no uncapped pool instance is built)
     if (p.T > 1) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 6>(p, threads, smem_bytes, stream);
     if (p.bits) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 5>(p, threads, smem_bytes, stream);

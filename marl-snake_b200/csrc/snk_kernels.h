@@ -79,6 +79,9 @@ struct KParams {
   const uint8_t* next_map;     // [N] map a reset of env e starts from (written by the caller)
   uint8_t* cur_map;            // [N] map of env e's current episode (written by every reset)
   int32_t num_maps;
+  // global state (snk_*_grid): [N, H*W] cell codes of every environment's grid as the observation was encoded from it
+  // ([T, N, H*W] when obs_every_step), or null -- and then the instances without it run
+  uint8_t* grid_out;
 };
 
 struct StateView {

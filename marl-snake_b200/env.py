@@ -34,11 +34,11 @@ class SnakeBatch:
                  frame_stack=1, observer='snake', reward_dict=None, num_fruits=None,
                  max_episode_steps=DEFAULT_MAX_EPISODE_STEPS, device=0, seed=0, rng='philox',
                  auto_reset=True, env_id_offset=0, done_mode='all', wall_map=None, wall_maps=None, map_ids=None,
-                 **ignored):
+                 global_state=False, **ignored):
         """wall_map: one custom wall layout for every env.  wall_maps: a pool of layouts of one shape (a list of arrays or
         map paths, or an [M, H, W] array; 1 <= M <= 256); each env starts every episode on the map its `next_maps`
         entry names at that reset (see next_maps / current_maps).  map_ids: initial next_maps (M ids), default
-        (env_id_offset + e) % M."""
+        (env_id_offset + e) % M.  global_state: keep `global_state` current (see there)."""
         reward_dict = DEFAULT_REWARD_DICT if reward_dict is None else reward_dict
         self.wall_map = None
         self.wall_maps = None
@@ -150,6 +150,15 @@ class SnakeBatch:
             # current_maps[e]: the map of env e's current episode, set from next_maps by every reset
             self.next_maps = _tensor_from_ptr(nxt.value, N, torch.uint8, dev)
             self.current_maps = _tensor_from_ptr(cur.value, N, torch.uint8, dev)
+        # global state for centralized critics: uint8 [N, H, W], every env's grid as cell codes (type + 10 * owner, the
+        # reference's SnakeEnv.grid) as the current observation was encoded from it -- after an auto-reset the new
+        # episode's grid.  The step kernel writes it beside the observation (snk_step_grid); like next_maps it is the
+        # batch's own buffer, overwritten by the next call.  None unless global_state=True.
+        self.global_state = None
+        if global_state:
+            H, W = self.grid_shape
+            self._gs_block = _ObsBlock(dev.index, N * H * W)     # mostly zero bytes: compressible, as the observation
+            self.global_state = torch.as_tensor(self._gs_block, device=dev).view(N, H, W)
 
     @property
     def obs_compressed(self):
@@ -195,10 +204,16 @@ class SnakeBatch:
         with torch.cuda.device(self.device):
             if bits:
                 out = self._bits_buffer()
-                check(lib.snk_reset_bits(self._h, _ptr(mask), _ptr(out), self._stream()))
+                if self.global_state is not None:
+                    check(lib.snk_reset_grid(self._h, _ptr(mask), None, _ptr(out), _ptr(self.global_state), self._stream()))
+                else:
+                    check(lib.snk_reset_bits(self._h, _ptr(mask), _ptr(out), self._stream()))
             else:
                 out = self._obs
-                check(lib.snk_reset(self._h, _ptr(mask), _ptr(out), self._stream()))
+                if self.global_state is not None:
+                    check(lib.snk_reset_grid(self._h, _ptr(mask), _ptr(out), None, _ptr(self.global_state), self._stream()))
+                else:
+                    check(lib.snk_reset(self._h, _ptr(mask), _ptr(out), self._stream()))
         # a masked reset rewrites the observation of the selected envs only: the others keep theirs
         self._mutated('reset(bits=True)' if bits else (None if mask is None else False))
         return out.clone() if copy else out
@@ -211,8 +226,12 @@ class SnakeBatch:
                 or actions.numel() != self.num_envs * self.num_snakes:
             raise ValueError('actions must be a contiguous uint8 CUDA tensor of shape [num_envs, num_snakes]')
         out = self._bits_buffer()
-        check(lib.snk_step_bits(self._h, _ptr(actions), _ptr(out), _ptr(self._rew), _ptr(self._done),
-                                C.byref(self._extra) if want_info else None, self._stream()))
+        if self.global_state is not None:
+            check(lib.snk_step_grid(self._h, _ptr(actions), None, _ptr(out), _ptr(self.global_state), _ptr(self._rew),
+                                    _ptr(self._done), C.byref(self._extra) if want_info else None, self._stream()))
+        else:
+            check(lib.snk_step_bits(self._h, _ptr(actions), _ptr(out), _ptr(self._rew), _ptr(self._done),
+                                    C.byref(self._extra) if want_info else None, self._stream()))
         self._mutated('step_bits')
         info = {}
         if want_info:
@@ -232,8 +251,13 @@ class SnakeBatch:
         if actions.dtype != torch.uint8 or actions.device != self.device or not actions.is_contiguous() \
                 or actions.numel() != self.num_envs * self.num_snakes:
             raise ValueError('actions must be a contiguous uint8 CUDA tensor of shape [num_envs, num_snakes]')
-        check(lib.snk_step(self._h, _ptr(actions), _ptr(self._obs if want_obs else None), _ptr(self._rew),
-                           _ptr(self._done), C.byref(self._extra) if want_info else None, self._stream()))
+        if self.global_state is not None:
+            check(lib.snk_step_grid(self._h, _ptr(actions), _ptr(self._obs if want_obs else None), None,
+                                    _ptr(self.global_state), _ptr(self._rew), _ptr(self._done),
+                                    C.byref(self._extra) if want_info else None, self._stream()))
+        else:
+            check(lib.snk_step(self._h, _ptr(actions), _ptr(self._obs if want_obs else None), _ptr(self._rew),
+                               _ptr(self._done), C.byref(self._extra) if want_info else None, self._stream()))
         self._mutated(None if want_obs else 'step(want_obs=False)')
         info = {}
         if want_info:
@@ -246,11 +270,12 @@ class SnakeBatch:
                    {k: v.clone() for k, v in info.items()})
         return out
 
-    def step_many(self, actions, obs=None, rewards=None, dones=None, bits=None, finished=None):
+    def step_many(self, actions, obs=None, rewards=None, dones=None, bits=None, finished=None, global_state=None):
         """T steps in one call (snk_step_many) for open-loop action streams.  actions: uint8 CUDA [T, N, ns].
-        rewards f64 / dones uint8 [T, N, ns] are allocated when not given.  obs (uint8) / bits: a [T, N, ...] tensor
-        receives every step's block, an [N, ...] tensor only the last step's; None skips that output.  finished:
-        optional uint8 [T, N].  Returns (obs, rewards, dones, bits).  Bit-identical to T calls of step()."""
+        rewards f64 / dones uint8 [T, N, ns] are allocated when not given.  obs (uint8) / bits / global_state (uint8
+        [.., N, H, W]): a [T, N, ...] tensor receives every step's block, an [N, ...] tensor only the last step's; None
+        skips that output.  finished: optional uint8 [T, N].  Returns (obs, rewards, dones, bits).  Bit-identical to T
+        calls of step().  A batch created with global_state=True keeps its `global_state` current either way."""
         N, ns = self.num_envs, self.num_snakes
         if actions.dtype != torch.uint8 or actions.device != self.device or not actions.is_contiguous() \
                 or actions.dim() != 3 or tuple(actions.shape[1:]) != (N, ns):
@@ -266,7 +291,8 @@ class SnakeBatch:
                 raise ValueError(f'{name} must be a contiguous {str(dtype)[6:]} CUDA tensor of shape '
                                  '[T, num_envs, num_snakes]')
         every = None
-        for name, buf, shape in (('obs', obs, self.obs_shape), ('bits', bits, self.bits_shape)):
+        for name, buf, shape in (('obs', obs, self.obs_shape), ('bits', bits, self.bits_shape),
+                                 ('global_state', global_state, self.grid_shape)):
             if buf is None:
                 continue
             if buf.dtype != torch.uint8 or buf.device != self.device or not buf.is_contiguous():
@@ -278,7 +304,7 @@ class SnakeBatch:
             else:
                 raise ValueError(f'{name} must have shape [T, N, ...] (every step) or [N, ...] (last step only)')
             if every is not None and every != e:
-                raise ValueError('obs and bits must both hold every step or both hold the last step only')
+                raise ValueError('obs, bits and global_state must all hold every step or all hold the last step only')
             every = e
         extra = None
         if finished is not None:
@@ -286,8 +312,21 @@ class SnakeBatch:
                     or not finished.is_contiguous():
                 raise ValueError('finished must be a contiguous uint8 CUDA tensor of shape [T, N]')
             extra = SnkStepExtra(finished.data_ptr(), 0, 0, 0, 0, 0)
-        check(lib.snk_step_many(self._h, T, _ptr(actions), _ptr(obs), _ptr(bits), int(bool(every)), _ptr(rewards),
-                                _ptr(dones), C.byref(extra) if extra is not None else None, self._stream()))
+        grid = global_state
+        if grid is None and self.global_state is not None and not every:
+            grid = self.global_state                        # the last step's rows straight into the batch's buffer
+        if grid is not None:
+            check(lib.snk_step_many_grid(self._h, T, _ptr(actions), _ptr(obs), _ptr(bits), _ptr(grid), int(bool(every)),
+                                         _ptr(rewards), _ptr(dones), C.byref(extra) if extra is not None else None,
+                                         self._stream()))
+        else:
+            check(lib.snk_step_many(self._h, T, _ptr(actions), _ptr(obs), _ptr(bits), int(bool(every)), _ptr(rewards),
+                                    _ptr(dones), C.byref(extra) if extra is not None else None, self._stream()))
+        if self.global_state is not None and grid is not self.global_state:
+            if grid is not None:
+                self.global_state.copy_(grid[-1] if every else grid)
+            else:                                           # obs / bits of every step, no caller grid: rebuild it
+                self._refresh_global_state()
         self._mutated('step_many')
         return obs, rewards, dones, bits
 
@@ -297,6 +336,7 @@ class SnakeBatch:
         check(lib.snk_step_host(self._h, C.c_void_p(actions.data_ptr()),
                                 C.c_void_p(obs.data_ptr()) if obs is not None else C.c_void_p(0),
                                 C.c_void_p(rewards.data_ptr()), C.c_void_p(dones.data_ptr())))
+        self._refresh_global_state()
         self._mutated('step_host')
 
     def step_host_info(self, actions, obs, rewards, dones, finished=None, rank=None, episode_scores=None,
@@ -311,6 +351,7 @@ class SnakeBatch:
         check(lib.snk_step_host_info(self._h, C.c_void_p(actions.data_ptr()),
                                      C.c_void_p(obs.data_ptr()) if obs is not None else C.c_void_p(0),
                                      C.c_void_p(rewards.data_ptr()), C.c_void_p(dones.data_ptr()), C.byref(xh)))
+        self._refresh_global_state()
         self._mutated('step_host_info')
 
     def step_host_bits(self, actions, bits, rewards, dones):
@@ -318,10 +359,12 @@ class SnakeBatch:
         bits -- one byte per (cell, frame) -- and nothing is widened on the host."""
         check(lib.snk_step_host_bits(self._h, C.c_void_p(actions.data_ptr()), C.c_void_p(bits.data_ptr()),
                                      C.c_void_p(rewards.data_ptr()), C.c_void_p(dones.data_ptr())))
+        self._refresh_global_state()
         self._mutated('step_host_bits')
 
     def reset_host(self, obs):
         check(lib.snk_reset_host(self._h, C.c_void_p(obs.data_ptr()) if obs is not None else C.c_void_p(0)))
+        self._refresh_global_state()
         self._mutated('reset_host')
 
     def set_host_transport(self, mode, threads=0):
@@ -348,6 +391,13 @@ class SnakeBatch:
         return out
 
     # ---- parity / checkpoint interface ---------------------------------------------------------------
+    def _refresh_global_state(self):
+        """After a call that changes the state without writing `global_state` (set_state, load_checkpoint, the
+        host-buffer calls): one snk_get_state launch that fills only the grid."""
+        if self.global_state is not None:
+            view = SnkStateView(grid=self.global_state.data_ptr())
+            check(lib.snk_get_state(self._h, C.byref(view), self._stream()))
+
     def get_state(self, max_cells=None):
         N, ns, dev = self.num_envs, self.num_snakes, self.device
         H, W = self.grid_shape
@@ -387,6 +437,7 @@ class SnakeBatch:
                     episode_length=t(episode_length, torch.int32, (N,)))
         view = SnkStateView(**{k: v.data_ptr() for k, v in keep.items()}, max_cells=cells.shape[-1])
         check(lib.snk_set_state(self._h, C.byref(view), _ptr(self._obs), self._stream()))
+        self._refresh_global_state()
         torch.cuda.current_stream(self.device).synchronize()      # `keep` must outlive the kernels
         self._mutated(None)
         return self._obs
@@ -402,6 +453,7 @@ class SnakeBatch:
     def load_checkpoint(self, blob):
         blob = np.ascontiguousarray(blob, dtype=np.uint8)
         check(lib.snk_checkpoint_load(self._h, blob.ctypes.data_as(C.c_void_p), blob.size))
+        self._refresh_global_state()
         self._mutated('load_checkpoint')
 
     def set_replay(self, draws_per_env):
