@@ -1364,6 +1364,9 @@ __device__ __forceinline__ void store_grid_rows(const KParams& p, const TilePtr&
 //       8, 10 (12, 14 with a pool) variants 0 and 2 that also write the global state (KParams::grid_out): 8 / 12 the
 //         plain step with or without its NHWC observation, 10 / 14 everything else (channel bits, several steps).  Calls
 //         without grid_out run the variants above, which hold none of that code.
+//       Specialised shapes (launch_tile_kernel) are built only in the tile modes their defaults select, and those with
+//       frame_stack > 1 without variants 2 and 6 (snk_step_many runs one launch per step there); the generic instances
+//       have every variant, and serve the calls a forced mode sends past a specialisation.
 // Warp-private instances of variants 0, 1, 4, 5, 8 and 12 are capped at 64 registers (eight 128-thread CTAs per SM).
 template <int kNS, int kW, int kOH, int kOW, int kFS, bool kCoop, int kEnc, int kVar>
 __global__ void __launch_bounds__(kCoop ? SNK_MAX_THREADS_COOP : SNK_MAX_THREADS, (!kCoop && (kVar & 3) <= 1) ? 8 : (!kCoop && kVar == 3) ? 1 : 0)
@@ -2015,12 +2018,15 @@ static cudaError_t launch_instance(const KParams& p, int threads, size_t smem_by
     return general ? launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 10>(p, threads, smem_bytes, stream)
                    : launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 8>(p, threads, smem_bytes, stream);
   }
-  if (p.pool) {                 // wall-map pool: variants 4 / 5 / 6 (no uncapped pool instance is built)
-    if (p.T > 1) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 6>(p, threads, smem_bytes, stream);
+  if (p.T > 1) {                // several steps per launch: variants 2 / 6
+    if constexpr (kFS > 1) return cudaErrorInvalidValue;     // step_many_impl steps frame stacks one launch at a time
+    else return p.pool ? launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 6>(p, threads, smem_bytes, stream)
+                       : launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 2>(p, threads, smem_bytes, stream);
+  }
+  if (p.pool) {                 // wall-map pool: variants 4 / 5 (no uncapped pool instance is built)
     if (p.bits) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 5>(p, threads, smem_bytes, stream);
     return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 4>(p, threads, smem_bytes, stream);
   }
-  if (p.T > 1) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 2>(p, threads, smem_bytes, stream);
   if (p.bits) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 1>(p, threads, smem_bytes, stream);
   if constexpr (!kCoop) {
     if (p.bigreg) return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 3>(p, threads, smem_bytes, stream);
@@ -2028,36 +2034,40 @@ static cudaError_t launch_instance(const KParams& p, int threads, size_t smem_by
   return launch_variant<kNS, kW, kOH, kOW, kFS, kCoop, kEnc, 0>(p, threads, smem_bytes, stream);
 }
 
-template <int kNS, int kW, int kOH, int kOW, int kFS, int kEnc>
-static cudaError_t launch_mode(const KParams& p, int threads, size_t smem_bytes, cudaStream_t stream) {
-  if constexpr (kEnc == ENC_PAD) {          // cooperative tiles only (encode_flavour)
-    if (!p.coop) return cudaErrorInvalidValue;
-    return launch_instance<kNS, kW, kOH, kOW, kFS, true, kEnc>(p, threads, smem_bytes, stream);
-  } else {
-    return p.coop ? launch_instance<kNS, kW, kOH, kOW, kFS, true, kEnc>(p, threads, smem_bytes, stream)
-                  : launch_instance<kNS, kW, kOH, kOW, kFS, false, kEnc>(p, threads, smem_bytes, stream);
+// The tile modes a set of instances is built for (bit 0 cooperative, bit 1 warp-private).
+enum : int { TILES_COOP = 1, TILES_WARP = 2, TILES_BOTH = 3 };
+static bool serves(int tiles, int coop) { return (tiles & (coop ? TILES_COOP : TILES_WARP)) != 0; }
+
+template <int kNS, int kW, int kOH, int kOW, int kFS, int kEnc, int kTiles>
+static cudaError_t launch_tiles(const KParams& p, int threads, size_t smem_bytes, cudaStream_t stream) {
+  if constexpr ((kTiles & TILES_COOP) != 0) {
+    if (p.coop) return launch_instance<kNS, kW, kOH, kOW, kFS, true, kEnc>(p, threads, smem_bytes, stream);
   }
+  if constexpr ((kTiles & TILES_WARP) != 0) {
+    if (!p.coop) return launch_instance<kNS, kW, kOH, kOW, kFS, false, kEnc>(p, threads, smem_bytes, stream);
+  }
+  return cudaErrorInvalidValue;             // the generic ENC_PAD set without coop: encode_flavour never gives that
 }
 
-// Specialised instances for the BASELINE shapes; everything else runs a generic instance of its flavour.
+// Specialised instances for the BASELINE shapes, in the tile modes create_impl's defaults give them; every other
+// call, forced modes included, runs the generic instance of its flavour.
 cudaError_t launch_tile_kernel(const KParams& p, int threads, size_t smem_bytes, cudaStream_t stream) {
   const Dims& d = p.d;
   const bool generic = p.force_generic != 0;
-#define SNK_TRY(NS, W_, OH, OW, FS, ENC)                                                                    \
-  if (!generic && d.ns == NS && d.W == W_ && d.oh == OH && d.ow == OW && d.fs == FS && p.enc_flavour == ENC) \
-    return launch_mode<NS, W_, OH, OW, FS, ENC>(p, threads, smem_bytes, stream);
-  SNK_TRY(4, 20, 11, 11, 1, ENC_REG)        // cfg1 / cfg5: 20x20, 4 snakes, vision 5
-  SNK_TRY(4, 20, 11, 11, 1, ENC_LEGACY)
-  SNK_TRY(4, 20, 20, 20, 1, ENC_DIRECT)     // cfg2: full-grid observation
-  SNK_TRY(4, 20, 11, 11, 4, ENC_LEGACY)     // cfg3: frame_stack 4
-  SNK_TRY(16, 64, 15, 15, 1, ENC_PAD)       // cfg4: 64x64, 16 snakes, vision 7
-  SNK_TRY(16, 64, 15, 15, 1, ENC_LEGACY)
+#define SNK_TRY(NS, W_, OH, OW, FS, ENC, TILES)                                                             \
+  if (!generic && d.ns == NS && d.W == W_ && d.oh == OH && d.ow == OW && d.fs == FS && p.enc_flavour == ENC && \
+      serves(TILES, p.coop))                                                                                 \
+    return launch_tiles<NS, W_, OH, OW, FS, ENC, TILES>(p, threads, smem_bytes, stream);
+  SNK_TRY(4, 20, 11, 11, 1, ENC_REG, TILES_BOTH)      // cfg1 / cfg5: 20x20, 4 snakes, vision 5
+  SNK_TRY(4, 20, 20, 20, 1, ENC_DIRECT, TILES_BOTH)   // cfg2: full-grid observation
+  SNK_TRY(4, 20, 11, 11, 4, ENC_LEGACY, TILES_COOP)   // cfg3: frame_stack 4 (create_impl: d.fs > 1 picks coop)
+  SNK_TRY(16, 64, 15, 15, 1, ENC_PAD, TILES_COOP)     // cfg4: 64x64, 16 snakes, vision 7 (create_impl: ENC_PAD picks coop)
 #undef SNK_TRY
   switch (p.enc_flavour) {
-    case ENC_REG: return launch_mode<0, 0, 0, 0, 0, ENC_REG>(p, threads, smem_bytes, stream);
-    case ENC_DIRECT: return launch_mode<0, 0, 0, 0, 0, ENC_DIRECT>(p, threads, smem_bytes, stream);
-    case ENC_PAD: return launch_mode<0, 0, 0, 0, 0, ENC_PAD>(p, threads, smem_bytes, stream);
-    default: return launch_mode<0, 0, 0, 0, 0, ENC_LEGACY>(p, threads, smem_bytes, stream);
+    case ENC_REG: return launch_tiles<0, 0, 0, 0, 0, ENC_REG, TILES_BOTH>(p, threads, smem_bytes, stream);
+    case ENC_DIRECT: return launch_tiles<0, 0, 0, 0, 0, ENC_DIRECT, TILES_BOTH>(p, threads, smem_bytes, stream);
+    case ENC_PAD: return launch_tiles<0, 0, 0, 0, 0, ENC_PAD, TILES_COOP>(p, threads, smem_bytes, stream);
+    default: return launch_tiles<0, 0, 0, 0, 0, ENC_LEGACY, TILES_BOTH>(p, threads, smem_bytes, stream);
   }
 }
 

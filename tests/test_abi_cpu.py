@@ -4,6 +4,8 @@ reference's dfs_sweep_empty enumeration (golden tables)."""
 import ctypes as C
 import os
 import re
+import shutil
+import subprocess
 
 import numpy as np
 import pytest
@@ -122,33 +124,54 @@ def test_reference_import_paths_resolve():
         sys.modules.update(saved)
 
 
-def test_hot_kernel_instances_keep_their_register_budget():
-    """The occupancy of the benchmarked kernel instances is part of the measured numbers: the rare-event functions
-    (fruit placement, reset) are out of line, and what they keep live raises the register count of EVERY instance
-    (a four-words-per-load fruit scan once took cfg2 from 48 to 62 and cfg5 from 88 to 102 registers -- 0.756 -> 0.836 ms).
-    cuobjdump reads the counts from the in-tree library; no GPU needed."""
-    import re
-    import shutil
-    import subprocess
+def _tile_kernels():
+    """(registers, stack bytes) of every snk_tile_kernel instance of the in-tree library, keyed by its template
+    arguments (ns, W, oh, ow, fs, coop, enc, variant; 0 for a generic dimension).  cuobjdump reads them; no GPU needed."""
     if not shutil.which('cuobjdump'):
         pytest.skip('cuobjdump not on PATH')
     import marl_snake_b200 as m
     out = subprocess.run(['cuobjdump', '-res-usage', m.LIB_PATH], capture_output=True, text=True, timeout=300).stdout
-    regs = {}
-    for name, reg, stack in re.findall(r'Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+)', out):
-        regs[name] = (int(reg), int(stack))
+    found = re.findall(r'Function \S*snk_tile_kernelILi(\d+)ELi(\d+)ELi(\d+)ELi(\d+)ELi(\d+)ELb(\d)ELi(\d+)ELi(\d+)EE\S*:'
+                       r'\s*\n\s*REG:(\d+) STACK:(\d+)', out)
+    tiles = {tuple(int(a) for a in f[:8]): (int(f[8]), int(f[9])) for f in found}
+    assert len(tiles) == len(found)
+    return tiles
 
-    def instance(ns, w, oh, ow, fs, coop, enc, var):
-        key = f'snk_tile_kernelILi{ns}ELi{w}ELi{oh}ELi{ow}ELi{fs}ELb{coop}ELi{enc}ELi{var}EE'
-        hits = [v for k, v in regs.items() if key in k]
-        assert len(hits) == 1, key
-        return hits[0]
+
+def test_hot_kernel_instances_keep_their_register_budget():
+    """The occupancy of the benchmarked kernel instances is part of the measured numbers: the rare-event functions
+    (fruit placement, reset) are out of line, and what they keep live raises the register count of EVERY instance
+    (a four-words-per-load fruit scan once took cfg2 from 48 to 62 and cfg5 from 88 to 102 registers -- 0.756 -> 0.836 ms)."""
+    tiles = _tile_kernels()
     budget = {                                    # (registers, stack bytes) ceilings
-        'cfg5 warp-private, capped': (instance(4, 20, 11, 11, 1, 0, 1, 0), (64, 16)),
-        'cfg5 warp-private, uncapped (the bench line)': (instance(4, 20, 11, 11, 1, 0, 1, 3), (88, 0)),
-        'cfg2 cooperative': (instance(4, 20, 20, 20, 1, 1, 2, 0), (48, 16)),
-        'cfg3 cooperative': (instance(4, 20, 11, 11, 4, 1, 0, 0), (64, 0)),
-        'cfg4 cooperative': (instance(16, 64, 15, 15, 1, 1, 3, 0), (64, 0)),
+        'cfg5 warp-private, capped': (tiles[4, 20, 11, 11, 1, 0, 1, 0], (64, 16)),
+        'cfg5 warp-private, uncapped (the bench line)': (tiles[4, 20, 11, 11, 1, 0, 1, 3], (88, 0)),
+        'cfg2 cooperative': (tiles[4, 20, 20, 20, 1, 1, 2, 0], (48, 16)),
+        'cfg3 cooperative': (tiles[4, 20, 11, 11, 4, 1, 0, 0], (64, 0)),
+        'cfg4 cooperative': (tiles[16, 64, 15, 15, 1, 1, 3, 0], (64, 0)),
     }
     for what, ((reg, stack), (max_reg, max_stack)) in budget.items():
         assert reg <= max_reg and stack <= max_stack, (what, reg, stack)
+
+
+def test_grid_instances_keep_the_register_budget():
+    """The cfg5 step with the global state runs its own instance (variant 8): still the viewer-pair encode within 64
+    registers and a small stack.  Every instance a default launch selects is there with its budget, and no specialised
+    instance that only a forced tile mode or encode could reach: those calls run the generic instance of their flavour."""
+    tiles = _tile_kernels()
+    reg, stack = tiles[4, 20, 11, 11, 1, 0, 1, 8]
+    assert reg <= 64 and stack <= 16, (reg, stack)
+    assert tiles[4, 20, 11, 11, 1, 0, 1, 0] == (64, 8)
+    assert tiles[4, 20, 11, 11, 1, 0, 1, 3] == (88, 0)
+    for var in (0, 1, 2, 4, 5, 6, 8, 10, 12, 14):
+        assert (4, 20, 11, 11, 1, 1, 1, var) in tiles            # the cooperative ones
+    assert not [k for k in tiles if k[:5] == (4, 20, 11, 11, 1) and k[6] == 0], 'cfg5 ENC_LEGACY'
+    assert not [k for k in tiles if k[:5] == (16, 64, 15, 15, 1) and k[6] == 0], 'cfg4 ENC_LEGACY'
+    assert not [k for k in tiles if k[:5] == (4, 20, 11, 11, 4) and k[5] == 0], 'cfg3 warp-private'
+    assert not [k for k in tiles if k[:5] == (4, 20, 11, 11, 4) and k[7] in (2, 6)], 'cfg3 several steps per launch'
+    per_var = {}
+    for k in tiles:
+        per_var[k[7]] = per_var.get(k[7], 0) + 1
+    # generic REG, DIRECT and LEGACY in both tile modes and PAD cooperative (7), cfg5 REG and cfg2 DIRECT in both (4),
+    # cfg3 LEGACY and cfg4 PAD cooperative (2, cfg3 without variants 2 and 6); variant 3 exists warp-private only
+    assert per_var == {0: 13, 1: 13, 2: 12, 3: 5, 4: 13, 5: 13, 6: 12, 8: 13, 10: 13, 12: 13, 14: 13}, per_var

@@ -3,9 +3,6 @@ kernel writes every env's grid, as cell codes, beside the observation.  Checked 
 grids (golden rollouts and scenarios), against the oracle in Philox mode, against get_state() at full size, and for
 leaving every other output byte for byte as it was."""
 import ctypes as C
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
@@ -345,32 +342,3 @@ def test_graph_replay_and_stale_calls():
     b.reset_host(obs)
     assert_grid_is_state(b, 'reset_host')
     assert a.device_errors() == 0 and b.device_errors() == 0
-
-
-def test_grid_instances_keep_the_register_budget():
-    """The cfg5 step with the global state runs its own instance (variant 8): still the viewer-pair encode within 64
-    registers and a small stack.  The instances of the calls without it are all still there, with their budgets."""
-    if not shutil.which('cuobjdump'):
-        pytest.skip('cuobjdump not on PATH')
-    import marl_snake_b200 as m
-    out = subprocess.run(['cuobjdump', '-res-usage', m.LIB_PATH], capture_output=True, text=True, timeout=300).stdout
-    regs = {name: (int(r), int(s)) for name, r, s in re.findall(r'Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+)', out)}
-
-    def instance(ns, w, oh, ow, fs, coop, enc, var):
-        key = f'snk_tile_kernelILi{ns}ELi{w}ELi{oh}ELi{ow}ELi{fs}ELb{coop}ELi{enc}ELi{var}EE'
-        hits = [v for k, v in regs.items() if key in k]
-        assert len(hits) == 1, key
-        return hits[0]
-    reg, stack = instance(4, 20, 11, 11, 1, 0, 1, 8)
-    assert reg <= 64 and stack <= 16, (reg, stack)
-    assert instance(4, 20, 11, 11, 1, 0, 1, 0) == (64, 8)
-    assert instance(4, 20, 11, 11, 1, 0, 1, 3) == (88, 0)
-    for var in (0, 1, 2, 4, 5, 6, 8, 10, 12, 14):
-        instance(4, 20, 11, 11, 1, 1, 1, var)                    # the cooperative ones
-    per_var = {}
-    for k in regs:
-        v = re.search(r'snk_tile_kernelI.*ELi(\d+)EEEv', k)
-        if v:
-            per_var[int(v.group(1))] = per_var.get(int(v.group(1)), 0) + 1
-    # the parent's instances (variants 0..6), and one grid twin per instance of variants 0, 2, 4 and 6
-    assert per_var == {0: 18, 1: 18, 2: 18, 3: 8, 4: 18, 5: 18, 6: 18, 8: 18, 10: 18, 12: 18, 14: 18}, per_var

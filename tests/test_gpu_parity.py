@@ -875,12 +875,12 @@ BITS_CASES = [
     (dict(num_snakes=4, vision_range=5), 700, {'SNK_COOP': '1'}),                     # register encode, cooperative
     (dict(num_snakes=4), 300, {}),                                                    # full-grid (direct) encode
     (dict(num_snakes=3, vision_range=2, frame_stack=3), 811, {}),                     # stacked
-    (dict(num_snakes=4, vision_range=5, frame_stack=4), 130, {'SNK_COOP': '0'}),      # stacked, specialised fs 4
+    (dict(num_snakes=4, vision_range=5, frame_stack=4), 130, {'SNK_COOP': '0'}),      # cfg3 shape warp-private: generic
     (dict(height=64, width=64, num_snakes=16, snake_length=5, vision_range=7), 40, {}),          # padded-plane encode, dual LUT
-    (dict(height=64, width=64, num_snakes=16, snake_length=5, vision_range=7), 40, {'SNK_ENC_NOPAD': '1'}),   # table encode, dual LUT
+    (dict(height=64, width=64, num_snakes=16, snake_length=5, vision_range=7), 40, {'SNK_ENC_NOPAD': '1'}),   # table encode, dual LUT, generic
     (dict(height=24, width=24, num_snakes=9, snake_length=3, vision_range=9), 50, {}),            # window > 16: index arithmetic
     (dict(height=32, width=32, num_snakes=8, snake_length=4, vision_range=6), 90, {'SNK_COOP': '1'}),   # padded plane, per-viewer LUT
-    (dict(num_snakes=4, vision_range=5), 400, {'SNK_ENC_LEGACY': '1'}),               # table encode, per-viewer LUT
+    (dict(num_snakes=4, vision_range=5), 400, {'SNK_ENC_LEGACY': '1'}),               # table encode, per-viewer LUT, generic
     (dict(height=13, width=11, num_snakes=2, vision_range=3), 77, {'SNK_FORCE_GENERIC': '1'}),
 ]
 

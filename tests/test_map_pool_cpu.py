@@ -21,7 +21,7 @@ def create_maps(maps, num_envs=4, ids=None, **kw):
     h = C.c_void_p()
     ids_p = None if ids is None else np.ascontiguousarray(ids, dtype=np.uint8).ctypes.data_as(C.c_void_p)
     rc = m.lib.snk_create_maps(C.byref(cfg), len(maps), maps.ctypes.data_as(C.c_void_p), ids_p, C.byref(h))
-    msg = m.lib.snk_last_error().decode()
+    msg = m.lib.snk_last_error().decode() if rc else ''    # a successful call leaves the last failure's message
     if rc == 0:
         m.lib.snk_destroy(h)
     return rc, msg
