@@ -53,38 +53,43 @@ struct DeviceGuard {
       return fail(SNK_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__); \
   } while (0)
 
+// The terminal-info outputs of snk_step_extra, in its field order: element size, and [N, ns] (per snake) or [N].
+constexpr int N_EXTRA = 6;
+struct ExtraOut { size_t elem; bool per_snake; };
+static const ExtraOut EXTRA_OUT[N_EXTRA] = {{1, false}, {sizeof(int32_t), true}, {sizeof(double), true},
+                                            {sizeof(int32_t), true}, {sizeof(int32_t), true}, {sizeof(int32_t), true}};
+static_assert(sizeof(snk_step_extra) == N_EXTRA * sizeof(void*), "EXTRA_OUT describes every field of snk_step_extra");
+static size_t extra_bytes(const Dims& d, int i) { return EXTRA_OUT[i].elem * d.N * (EXTRA_OUT[i].per_snake ? d.ns : 1); }
+// snk_step_extra as the array of its pointers (null x: all null), and back
+struct ExtraPtrs { uint8_t* p[N_EXTRA]; };
+static ExtraPtrs extra_ptrs(const snk_step_extra* x) {
+  ExtraPtrs a = {};
+  if (x) memcpy(a.p, x, sizeof *x);
+  return a;
+}
+static snk_step_extra extra_struct(const ExtraPtrs& a) {
+  snk_step_extra x;
+  memcpy(&x, a.p, sizeof x);
+  return x;
+}
+
 struct snk_env {
-  Dims d;
+  // The launch template: the shape, the resident device buffers and every launch decision of create_impl.  A launch
+  // copies it and fills in its own I/O.  (Its `pool` is the wall-map pool, not the widening pool below.)
+  KParams kp = {};
   int device = 0;
-  int tile_envs = 0, threads = 0;
+  int threads = 0;
   size_t smem_bytes = 0;
   int many_tile_envs = 0, many_threads = 0;      // tile shape of multi-step launches (snk_step_many, cooperative tiles)
   size_t many_smem_bytes = 0;
-  uint8_t* recs = nullptr;
-  uint8_t* hist = nullptr;
-  uint64_t* spawn = nullptr;
-  uint32_t* wall_map = nullptr;                  // custom wall layout (snk_create_map): H*W cell codes, padded to words
-  uint8_t* base_grid = nullptr;                  // compact records: the wall layout, one copy per environment of a tile
-  // wall-map pool (snk_create_maps): num_maps layouts of off_c0 bytes, each map's part of `spawn`, the per-env map ids
-  int num_maps = 0;                              // 0: no pool
-  uint8_t* maps = nullptr;
-  uint2* map_tab = nullptr;
-  uint8_t* next_map = nullptr;
-  uint8_t* cur_map = nullptr;
   uint64_t pool_digest = 0;                      // layouts + spawn-table sizes: a checkpoint only loads into the same pool
-  int32_t* replay = nullptr;
-  int64_t* replay_off = nullptr;
-  uint32_t* err = nullptr;
-  double* stats = nullptr;
-  uint8_t* enc_blob = nullptr;
-  int enc_blob_bytes = 0, enc_tab_off = 0, enc_lutb_off = 0, use_tab = 0;
   // ordering between the caller's streams (device-pointer calls) and own_stream (host-buffer calls)
   cudaStream_t last_user_stream = nullptr;
   bool user_work_pending = false;
   cudaEvent_t user_ev = nullptr;
-  // device mirrors used by the *_host entry points
+  // device mirrors used by the *_host entry points; h_extra in EXTRA_OUT order
   uint8_t* h_actions = nullptr; uint8_t* h_obs = nullptr; double* h_rew = nullptr; uint8_t* h_done = nullptr;
-  uint8_t* h_fin = nullptr; int32_t* h_rank = nullptr; double* h_scores = nullptr; int32_t* h_counts = nullptr;   // [3][N, ns]
+  uint8_t* h_extra[N_EXTRA] = {};
   // few environments: every output of a host-buffer step lives in ONE device block mirrored by ONE pinned host
   // block, so the step costs one copy in, one launch, one copy out (the latency-bound drop-in mode)
   uint8_t* small_dev = nullptr; uint8_t* small_host = nullptr; uint8_t* small_map = nullptr;
@@ -96,8 +101,6 @@ struct snk_env {
   WidenPool* pool = nullptr;
   cudaEvent_t chunk_ev[XFER_MAX_CHUNKS] = {};
   int n_chunk_ev = 0;
-  int force_generic = 0, coop = 0, lut_dual = 0, use_tma = 0, enc_flavour = 0, pdl = 1, bigreg = 0, l2_keep = 0;
-  float l2_keep_frac = 1.0f;
   bool was_reset = false;
 };
 
@@ -109,32 +112,13 @@ static int env_int(const char* name, int dflt) {
   return (s && *s) ? atoi(s) : dflt;
 }
 
-static KParams base_params(const snk_env* h) {
-  KParams p;
-  memset(&p, 0, sizeof p);
-  p.d = h->d;
-  p.recs = h->recs; p.hist = h->hist; p.spawn = h->spawn; p.wall_map = h->wall_map; p.base_grid = h->base_grid;
-  p.replay = h->replay; p.replay_off = h->replay_off;
-  p.err = h->err; p.stats = h->stats;
-  p.E = h->tile_envs;
-  p.force_generic = h->force_generic;
-  p.enc_blob = h->enc_blob; p.enc_blob_bytes = h->enc_blob_bytes; p.enc_tab_off = h->enc_tab_off; p.use_tab = h->use_tab;
-  p.enc_lutb_off = h->enc_lutb_off;
-  p.lut_dual = h->lut_dual; p.coop = h->coop; p.use_tma = h->use_tma; p.pdl = h->pdl; p.bigreg = h->bigreg; p.l2_keep = h->l2_keep; p.l2_keep_frac = h->l2_keep_frac;
-  p.T = 1;
-  if (h->num_maps) {
-    p.pool = h->maps; p.map_tab = h->map_tab; p.next_map = h->next_map; p.cur_map = h->cur_map; p.num_maps = h->num_maps;
-    p.bigreg = 0;                                // pool handles run the capped instances (no uncapped pool instance is built)
-  }
-  p.enc_flavour = h->enc_flavour;
-  p.enc_copy_bytes = (h->enc_flavour == ENC_LEGACY) ? h->enc_blob_bytes : h->enc_tab_off;     // LUT only
-  {
-    const uint64_t one = (uint64_t)1 << 32;
-    const uint64_t wpr = (uint64_t)(h->d.W >> 2 > 1 ? h->d.W >> 2 : 2), nw = (uint64_t)h->d.H * wpr;
-    p.inv_grid_words = (uint32_t)((one + nw - 1) / nw);
-    p.inv_row_words = (uint32_t)((one + wpr - 1) / wpr);
-  }
-  return p;
+// cudaMalloc of `bytes` filled from host memory; dst may be a pointer to const (the template's read-only buffers)
+template <typename T>
+static cudaError_t upload(T*& dst, const void* src, size_t bytes) {
+  void* p = nullptr;
+  const cudaError_t e = cudaMalloc(&p, bytes);
+  dst = static_cast<T*>(p);
+  return e != cudaSuccess ? e : cudaMemcpy(p, src, bytes, cudaMemcpyHostToDevice);
 }
 
 // num_maps == 0: snk_create (walls_host null) or snk_create_map (one layout, no pool); num_maps >= 1: a wall-map pool of
@@ -173,7 +157,7 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
 
   snk_env* h = new (std::nothrow) snk_env();
   if (!h) return fail(SNK_E_NOMEM, "out of host memory");
-  Dims& d = h->d;
+  Dims& d = h->kp.d;
   memset(&d, 0, sizeof d);
   d.N = c->num_envs; d.H = c->height; d.W = c->width; d.ns = c->num_snakes; d.K = c->snake_length;
   d.V = c->vision_range; d.fs = c->frame_stack; d.nfruits = nfruits;
@@ -251,7 +235,7 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
       }
       ids[e] = map_ids_host ? map_ids_host[e] : (uint8_t)((c->env_id_offset + (uint64_t)e) % (uint64_t)num_maps);
     }
-    h->num_maps = num_maps;
+    h->kp.num_maps = num_maps;
     uint64_t dg = fnv1a(0xCBF29CE484222325ull, walls.data(), walls.size());
     h->pool_digest = fnv1a(dg, map_tab.data(), map_tab.size() * sizeof(uint2));
   }
@@ -312,7 +296,7 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
   if (env_int("SNK_TILE_ENVS", 0) <= 0)
     while (EPW > 1 && tile_smem_bytes(d, coop ? threads / 32 : 1, coop != 0, EPW) > 100 * 1024) EPW >>= 1;
   while (threads > 32 && tile_smem_bytes(d, threads / 32, coop != 0, EPW) > 200 * 1024) threads -= 32;
-  h->tile_envs = EPW; h->threads = threads; h->coop = coop;
+  h->kp.E = EPW; h->threads = threads; h->kp.coop = coop;
   {
     // snk_step_many: every CTA lives for the whole launch, so the grid should be ONE resident wave -- as many
     // environments per cooperative tile as the rule warp has lane groups (fewer, longer-lived CTAs), more warps to
@@ -324,18 +308,27 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
     h->many_tile_envs = me; h->many_threads = mt;
     h->many_smem_bytes = tile_smem_bytes(d, mt / 32, coop != 0, me);
   }
-  h->force_generic = env_int("SNK_FORCE_GENERIC", 0);
-  h->use_tma = env_int("SNK_TMA", 1);
-  h->pdl = env_int("SNK_PDL", 1);
+  h->kp.force_generic = env_int("SNK_FORCE_GENERIC", 0);
+  h->kp.use_tma = env_int("SNK_TMA", 1);
+  h->kp.pdl = env_int("SNK_PDL", 1);
   h->small_zero_copy = env_int("SNK_SMALL_ZEROCOPY", 1);
-  h->l2_keep = env_int("SNK_L2_KEEP", d.fs > 1 ? 1 : 0);
-  h->l2_keep_frac = (float)env_int("SNK_L2_KEEP_PCT", 100) / 100.0f;
+  h->kp.l2_keep = env_int("SNK_L2_KEEP", d.fs > 1 ? 1 : 0);
+  h->kp.l2_keep_frac = (float)env_int("SNK_L2_KEEP_PCT", 100) / 100.0f;
   {
     // the uncapped-register instance of the warp-private kernel once the batch is many waves deep (a step that writes
-    // its observation into a compressible block runs the capped one all the same: see step_impl)
+    // its observation into a compressible block runs the capped one all the same: see step_impl).  Pool handles run
+    // the capped instances: no uncapped pool instance is built.
     const int64_t tiles = ((int64_t)d.N + EPW - 1) / EPW;
-    h->bigreg = (!coop && tiles >= (int64_t)env_int("SNK_BIGREG_TILES", 24576)) ? 1 : 0;
+    h->kp.bigreg = (!coop && !num_maps && tiles >= (int64_t)env_int("SNK_BIGREG_TILES", 24576)) ? 1 : 0;
   }
+  {
+    // ENC_PAD: ceil(2^32 / words) of a grid and of a row (at least two words a row)
+    const uint64_t one = (uint64_t)1 << 32;
+    const uint64_t wpr = (uint64_t)(d.W >> 2 > 1 ? d.W >> 2 : 2), nw = (uint64_t)d.H * wpr;
+    h->kp.inv_grid_words = (uint32_t)((one + nw - 1) / nw);
+    h->kp.inv_row_words = (uint32_t)((one + wpr - 1) / wpr);
+  }
+  h->kp.T = 1;
   h->smem_bytes = tile_smem_bytes(d, threads / 32, coop != 0, EPW);
   if (h->smem_bytes > 227 * 1024) {
     const size_t need = h->smem_bytes;
@@ -346,57 +339,51 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
   DeviceGuard guard(c->device);
   if (guard.err != cudaSuccess) { delete h; return fail(SNK_E_CUDA, "cudaSetDevice(%d): %s", c->device, cudaGetErrorString(guard.err)); }
 #define CUH(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { int rc = fail(SNK_E_CUDA, "%s failed: %s", #call, cudaGetErrorString(_e)); snk_destroy(h); return rc; } } while (0)
-  CUH(cudaMalloc(&h->recs, (size_t)d.N * d.hbm_rec_bytes));
-  if (d.hist_env_bytes) CUH(cudaMalloc(&h->hist, (size_t)d.N * d.hist_env_bytes));
-  CUH(cudaMalloc(&h->spawn, table.size() * sizeof(uint64_t)));
-  CUH(cudaMalloc(&h->err, sizeof(uint32_t)));
-  CUH(cudaMalloc(&h->stats, STAT_COUNT * sizeof(double)));
-  CUH(cudaMalloc(&h->replay_off, ((size_t)d.N + 1) * sizeof(int64_t)));
-  CUH(cudaMemcpy(h->spawn, table.data(), table.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
+  CUH(cudaMalloc(&h->kp.recs, (size_t)d.N * d.hbm_rec_bytes));
+  if (d.hist_env_bytes) CUH(cudaMalloc(&h->kp.hist, (size_t)d.N * d.hist_env_bytes));
+  CUH(upload(h->kp.spawn, table.data(), table.size() * sizeof(uint64_t)));
+  CUH(cudaMalloc(&h->kp.err, sizeof(uint32_t)));
+  CUH(cudaMalloc(&h->kp.stats, STAT_COUNT * sizeof(double)));
+  CUH(cudaMalloc((void**)&h->kp.replay_off, ((size_t)d.N + 1) * sizeof(int64_t)));
   if (num_maps) {
     // the pool serves the resets and (compact records) the tile loads, which paint each grid from its own map
-    CUH(cudaMalloc(&h->maps, walls.size()));
-    CUH(cudaMemcpy(h->maps, walls.data(), walls.size(), cudaMemcpyHostToDevice));
-    CUH(cudaMalloc(&h->map_tab, map_tab.size() * sizeof(uint2)));
-    CUH(cudaMemcpy(h->map_tab, map_tab.data(), map_tab.size() * sizeof(uint2), cudaMemcpyHostToDevice));
-    CUH(cudaMalloc(&h->next_map, ids.size()));
-    CUH(cudaMalloc(&h->cur_map, ids.size()));
-    CUH(cudaMemcpy(h->next_map, ids.data(), ids.size(), cudaMemcpyHostToDevice));
-    CUH(cudaMemcpy(h->cur_map, ids.data(), ids.size(), cudaMemcpyHostToDevice));
+    CUH(upload(h->kp.pool, walls.data(), walls.size()));
+    CUH(upload(h->kp.map_tab, map_tab.data(), map_tab.size() * sizeof(uint2)));
+    CUH(upload(h->kp.next_map, ids.data(), ids.size()));
+    CUH(upload(h->kp.cur_map, ids.data(), ids.size()));
   } else if (wm) {
-    CUH(cudaMalloc(&h->wall_map, walls.size()));
-    CUH(cudaMemcpy(h->wall_map, walls.data(), walls.size(), cudaMemcpyHostToDevice));
+    CUH(upload(h->kp.wall_map, walls.data(), walls.size()));
   }
   if (!num_maps) {
     // the wall layout every reset starts from: make_grid's walled box (core/grid_util.py:14-20) or the custom map,
     // padded to 16 bytes.  Compact records: it is also what the grid every record implies starts from -- as many
     // copies as the widest tile has environments, so ONE bulk copy paints a tile's grids
-    const int copies = !d.compact ? 1 : h->tile_envs > h->many_tile_envs ? h->tile_envs : h->many_tile_envs;
+    const int copies = !d.compact ? 1 : h->kp.E > h->many_tile_envs ? h->kp.E : h->many_tile_envs;
     std::vector<uint8_t> tpl((size_t)copies * d.off_c0, 0);
     for (int i = 0; i < d.HW; ++i) tpl[i] = wm ? wm[i] : wall_or_empty(i, d.H, d.W);
     for (int k = 1; k < copies; ++k) memcpy(tpl.data() + (size_t)k * d.off_c0, tpl.data(), (size_t)d.off_c0);
-    CUH(cudaMalloc(&h->base_grid, tpl.size()));
-    CUH(cudaMemcpy(h->base_grid, tpl.data(), tpl.size(), cudaMemcpyHostToDevice));
+    CUH(upload(h->kp.base_grid, tpl.data(), tpl.size()));
   }
   {
     size_t tab_off = 0, lutb_off = 0;
     const size_t nb = encode_blob_bytes(d, &tab_off, &lutb_off);
     std::vector<uint8_t> blob(nb, 0);
     encode_blob_fill(d, blob.data());
-    CUH(cudaMalloc(&h->enc_blob, nb));
-    CUH(cudaMemcpy(h->enc_blob, blob.data(), nb, cudaMemcpyHostToDevice));
-    h->enc_blob_bytes = (int)nb; h->enc_tab_off = (int)tab_off; h->enc_lutb_off = (int)lutb_off;
-    h->lut_dual = encode_lut_dual(d) ? 1 : 0;
-    h->use_tab = encode_uses_table(d) && (h->lut_dual || !env_int("SNK_NO_TABLE", 0)) ? 1 : 0;
+    CUH(upload(h->kp.enc_blob, blob.data(), nb));
+    KParams& p = h->kp;
+    p.enc_blob_bytes = (int)nb; p.enc_tab_off = (int)tab_off; p.enc_lutb_off = (int)lutb_off;
+    p.lut_dual = encode_lut_dual(d) ? 1 : 0;
+    p.use_tab = encode_uses_table(d) && (p.lut_dual || !env_int("SNK_NO_TABLE", 0)) ? 1 : 0;
     // SNK_ENC_LEGACY=1 / SNK_ENC_NOPAD=1: A/B switches (the cooperative ENC_PAD encode falls back to what warp-private
     // tiles of the same shape run)
-    h->enc_flavour = env_int("SNK_ENC_LEGACY", 0) ? ENC_LEGACY : encode_flavour(d, coop != 0 && !env_int("SNK_ENC_NOPAD", 0));
+    p.enc_flavour = env_int("SNK_ENC_LEGACY", 0) ? ENC_LEGACY : encode_flavour(d, coop != 0 && !env_int("SNK_ENC_NOPAD", 0));
+    p.enc_copy_bytes = (p.enc_flavour == ENC_LEGACY) ? p.enc_blob_bytes : p.enc_tab_off;     // LUT only
   }
-  CUH(cudaMemset(h->err, 0, sizeof(uint32_t)));
-  CUH(cudaMemset(h->stats, 0, STAT_COUNT * sizeof(double)));
-  CUH(cudaMemset(h->replay_off, 0, ((size_t)d.N + 1) * sizeof(int64_t)));
-  if (d.hist_env_bytes) CUH(cudaMemset(h->hist, 0, (size_t)d.N * d.hist_env_bytes));
-  CUH(launch_init_records(d, h->recs, nullptr));
+  CUH(cudaMemset(h->kp.err, 0, sizeof(uint32_t)));
+  CUH(cudaMemset(h->kp.stats, 0, STAT_COUNT * sizeof(double)));
+  CUH(cudaMemset((void*)h->kp.replay_off, 0, ((size_t)d.N + 1) * sizeof(int64_t)));
+  if (d.hist_env_bytes) CUH(cudaMemset(h->kp.hist, 0, (size_t)d.N * d.hist_env_bytes));
+  CUH(launch_init_records(d, h->kp.recs, nullptr));
   CUH(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
   CUH(cudaEventCreateWithFlags(&h->user_ev, cudaEventDisableTiming));
   CUH(cudaDeviceSynchronize());
@@ -417,11 +404,12 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
 extern "C" int snk_destroy(snk_env* h) {
   if (!h) return SNK_OK;
   DeviceGuard guard(h->device);
-  cudaFree(h->recs); cudaFree(h->hist); cudaFree(h->spawn); cudaFree(h->replay); cudaFree(h->replay_off);
-  cudaFree(h->err); cudaFree(h->stats); cudaFree(h->enc_blob); cudaFree(h->wall_map); cudaFree(h->base_grid);
-  cudaFree(h->maps); cudaFree(h->map_tab); cudaFree(h->next_map); cudaFree(h->cur_map);
+  const KParams& p = h->kp;
+  const void* bufs[] = {p.recs, p.hist, p.spawn, p.replay, p.replay_off, p.err, p.stats, p.enc_blob, p.wall_map, p.base_grid,
+                        p.pool, p.map_tab, p.next_map, p.cur_map};
+  for (const void* b : bufs) cudaFree(const_cast<void*>(b));
   cudaFree(h->h_actions); cudaFree(h->h_obs); cudaFree(h->h_rew); cudaFree(h->h_done);
-  cudaFree(h->h_fin); cudaFree(h->h_rank); cudaFree(h->h_scores); cudaFree(h->h_counts);
+  for (uint8_t* b : h->h_extra) cudaFree(b);
   cudaFree(h->small_dev);
   if (h->small_host) cudaFreeHost(h->small_host);
   cudaFree(h->d_bits);
@@ -436,33 +424,28 @@ extern "C" int snk_destroy(snk_env* h) {
 
 extern "C" int snk_obs_shape(const snk_env* h, int32_t out[4]) {
   if (!h || !out) return fail(SNK_E_INVALID, "null argument");
-  out[0] = h->d.ns; out[1] = h->d.oh; out[2] = h->d.ow; out[3] = 8 * h->d.fs;
+  out[0] = h->kp.d.ns; out[1] = h->kp.d.oh; out[2] = h->kp.d.ow; out[3] = 8 * h->kp.d.fs;
   return SNK_OK;
 }
-extern "C" size_t snk_obs_bytes(const snk_env* h) { return h ? (size_t)h->d.N * h->d.obs_env_bytes : 0; }
-extern "C" int snk_num_envs(const snk_env* h) { return h ? h->d.N : 0; }
-extern "C" int snk_num_maps(const snk_env* h) { return h ? h->num_maps : 0; }
+extern "C" size_t snk_obs_bytes(const snk_env* h) { return h ? (size_t)h->kp.d.N * h->kp.d.obs_env_bytes : 0; }
+extern "C" int snk_num_envs(const snk_env* h) { return h ? h->kp.d.N : 0; }
+extern "C" int snk_num_maps(const snk_env* h) { return h ? h->kp.num_maps : 0; }
 
 extern "C" int snk_map_ids_dev(snk_env* h, uint8_t** next_dev, uint8_t** cur_dev) {
   if (!h || !next_dev || !cur_dev) return fail(SNK_E_INVALID, "null argument");
-  if (!h->num_maps) return fail(SNK_E_STATE, "handle has no wall-map pool (create it with snk_create_maps)");
-  *next_dev = h->next_map; *cur_dev = h->cur_map;
+  if (!h->kp.num_maps) return fail(SNK_E_STATE, "handle has no wall-map pool (create it with snk_create_maps)");
+  *next_dev = const_cast<uint8_t*>(h->kp.next_map); *cur_dev = h->kp.cur_map;
   return SNK_OK;
 }
 
 extern "C" size_t snk_algorithmic_bytes_per_env_step(const snk_env* h) {
   if (!h) return 0;
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   // state record read + write, frame history (read fs-1 rows, write 1), observation write,
   // actions in, rewards (f64) and dones out.
   size_t b = 2 * (size_t)d.hbm_rec_bytes + (size_t)d.obs_env_bytes + (size_t)d.ns * (1 + 8 + 1);
   if (d.fs > 1) b += (size_t)d.ns * d.fs * d.ohw;
   return b;
-}
-
-static int check_vec16(const snk_env* h, const uint8_t* obs) {
-  if (!obs) return 0;
-  return (((uintptr_t)obs & 15) == 0 && h->d.obs_env_bytes % 16 == 0) ? 1 : 0;    // every env block 16-byte aligned
 }
 
 // Device-pointer calls only enqueue work on the caller's stream.  The host-buffer calls run on the handle's own
@@ -489,12 +472,35 @@ extern "C" int snk_note_stream(snk_env* h, void* stream) {
   return SNK_OK;
 }
 
+// The parameters of one launch: the handle's template plus the call's I/O, once the pointers pass their checks.  A step
+// needs actions, rewards and dones and a reset before it; a reset and the encode of set_state take none of the three.
+// With T steps, actions / rewards / dones / extras are [T, ...], and obs / bits / grid too when `every`.
+static int call_params(snk_env* h, KParams& p, int mode, const uint8_t* actions, uint8_t* obs, uint8_t* bits, uint8_t* grid,
+                       double* rew, uint8_t* done, const snk_step_extra* x, int T = 1, int every = 0) {
+  if (mode == MODE_STEP) {
+    if (!actions || !rew || !done) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
+    if (!h->was_reset) return fail(SNK_E_STATE, "step before reset");
+  }
+  if (obs && ((uintptr_t)obs & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
+  if ((uintptr_t)rew & 7) return fail(SNK_E_INVALID, "rewards must be 8-byte aligned");
+  p = h->kp;
+  p.mode = mode; p.T = T; p.obs_every_step = every ? 1 : 0;
+  p.actions = actions; p.obs = obs; p.bits = bits; p.grid_out = grid; p.rew = rew; p.done = done;
+  if (x) {
+    p.fin = x->finished; p.rank = x->rank; p.ep_scores = x->episode_scores;
+    p.ep_steps = x->episode_steps; p.ep_fruits = x->episode_fruits; p.ep_kills = x->episode_kills;
+  }
+  // every env block 16-byte aligned (the per-step blocks of `every` are whole env blocks apart)
+  p.vec16 = (obs && ((uintptr_t)obs & 15) == 0 && h->kp.d.obs_env_bytes % 16 == 0) ? 1 : 0;
+  return SNK_OK;
+}
+
 static int reset_impl(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
                       cudaStream_t stream) {
-  if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
-  KParams p = base_params(h);
-  p.mode = MODE_RESET; p.mask = mask_dev; p.obs = obs_dev; p.bits = bits_dev; p.grid_out = grid_dev;
-  p.vec16 = check_vec16(h, obs_dev);
+  KParams p;
+  const int rc = call_params(h, p, MODE_RESET, nullptr, obs_dev, bits_dev, grid_dev, nullptr, nullptr, nullptr);
+  if (rc) return rc;
+  p.mask = mask_dev;
   CU(launch_tile_kernel(p, h->threads, h->smem_bytes, stream));
   note_user_stream(h, stream);
   h->was_reset = true;
@@ -503,18 +509,9 @@ static int reset_impl(snk_env* h, const uint8_t* mask_dev, uint8_t* obs_dev, uin
 
 static int step_impl(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
                      double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* x, cudaStream_t stream) {
-  if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
-  if (!h->was_reset) return fail(SNK_E_STATE, "step before reset");
-  if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
-  if ((uintptr_t)rewards_dev & 7) return fail(SNK_E_INVALID, "rewards must be 8-byte aligned");
-  KParams p = base_params(h);
-  p.mode = MODE_STEP;
-  p.actions = actions_dev; p.obs = obs_dev; p.bits = bits_dev; p.grid_out = grid_dev; p.rew = rewards_dev; p.done = dones_dev;
-  if (x) {
-    p.fin = x->finished; p.rank = x->rank; p.ep_scores = x->episode_scores;
-    p.ep_steps = x->episode_steps; p.ep_fruits = x->episode_fruits; p.ep_kills = x->episode_kills;
-  }
-  p.vec16 = check_vec16(h, obs_dev);
+  KParams p;
+  const int rc = call_params(h, p, MODE_STEP, actions_dev, obs_dev, bits_dev, grid_dev, rewards_dev, dones_dev, x);
+  if (rc) return rc;
   // An observation block in compressible memory costs the step far less DRAM time, and the step is then bound by the
   // latency of its rule phase: the 64-register instance, with twice the resident warps, is the faster one there
   // (cfg5, 1 048 576 envs on a B200 at 1000 W: 0.671 ms against 0.758 ms uncapped; profiles/r03_retune.txt).
@@ -530,39 +527,25 @@ static int step_impl(snk_env* h, const uint8_t* actions_dev, uint8_t* obs_dev, u
 // frame_stack > 1 (the frame history is written per step): T ordinary launches -- same results, same arrays.
 static int step_many_impl(snk_env* h, int T, const uint8_t* actions_dev, uint8_t* obs_dev, uint8_t* bits_dev, uint8_t* grid_dev,
                           int every, double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* x, cudaStream_t stream) {
+  if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
   if (T < 1 || T > 65536) return fail(SNK_E_INVALID, "num_steps must be in 1..65536");
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   const size_t nn = (size_t)d.N * d.ns;
   if (d.fs == 1) {
-    if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
-    if (!h->was_reset) return fail(SNK_E_STATE, "step before reset");
-    if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
-    if ((uintptr_t)rewards_dev & 7) return fail(SNK_E_INVALID, "rewards must be 8-byte aligned");
-    KParams p = base_params(h);
+    KParams p;
+    const int rc = call_params(h, p, MODE_STEP, actions_dev, obs_dev, bits_dev, grid_dev, rewards_dev, dones_dev, x, T, every);
+    if (rc) return rc;
     const bool many = T > 1;
     if (many) p.E = h->many_tile_envs;
-    p.mode = MODE_STEP; p.T = T; p.obs_every_step = every ? 1 : 0;
-    p.actions = actions_dev; p.obs = obs_dev; p.bits = bits_dev; p.grid_out = grid_dev; p.rew = rewards_dev; p.done = dones_dev;
-    p.vec16 = check_vec16(h, obs_dev);          // the per-step blocks of obs_every_step are whole environment blocks apart
-    if (x) {
-      p.fin = x->finished; p.rank = x->rank; p.ep_scores = x->episode_scores;
-      p.ep_steps = x->episode_steps; p.ep_fruits = x->episode_fruits; p.ep_kills = x->episode_kills;
-    }
     CU(launch_tile_kernel(p, many ? h->many_threads : h->threads, many ? h->many_smem_bytes : h->smem_bytes, stream));
     note_user_stream(h, stream);
     return SNK_OK;
   }
   for (int t = 0; t < T; ++t) {
-    snk_step_extra xt;
-    memset(&xt, 0, sizeof xt);
-    if (x) {
-      if (x->finished) xt.finished = x->finished + (size_t)t * d.N;
-      if (x->rank) xt.rank = x->rank + t * nn;
-      if (x->episode_scores) xt.episode_scores = x->episode_scores + t * nn;
-      if (x->episode_steps) xt.episode_steps = x->episode_steps + t * nn;
-      if (x->episode_fruits) xt.episode_fruits = x->episode_fruits + t * nn;
-      if (x->episode_kills) xt.episode_kills = x->episode_kills + t * nn;
-    }
+    ExtraPtrs xp = extra_ptrs(x);
+    for (int i = 0; i < N_EXTRA; ++i)
+      if (xp.p[i]) xp.p[i] += t * extra_bytes(d, i);
+    const snk_step_extra xt = extra_struct(xp);
     const bool render = every || t == T - 1;
     uint8_t* o = (obs_dev && render) ? obs_dev + (every ? (size_t)t * d.N * d.obs_env_bytes : 0) : nullptr;
     uint8_t* b = (bits_dev && render) ? bits_dev + (every ? (size_t)t * d.N * d.stage_env_bytes : 0) : nullptr;
@@ -577,7 +560,6 @@ extern "C" int snk_step_many(snk_env* h, int32_t num_steps, const uint8_t* actio
                              int32_t obs_every_step, double* rewards_dev, uint8_t* dones_dev, const snk_step_extra* x,
                              void* stream) {
   if (!h) return fail(SNK_E_INVALID, "null handle");
-  if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
   ON_DEVICE(h);
   return step_many_impl(h, num_steps, actions_dev, obs_dev, bits_dev, nullptr, obs_every_step, rewards_dev, dones_dev, x,
                         (cudaStream_t)stream);
@@ -587,7 +569,6 @@ extern "C" int snk_step_many_grid(snk_env* h, int32_t num_steps, const uint8_t* 
                                   uint8_t* grid_dev, int32_t obs_every_step, double* rewards_dev, uint8_t* dones_dev,
                                   const snk_step_extra* x, void* stream) {
   if (!h) return fail(SNK_E_INVALID, "null handle");
-  if (!actions_dev || !rewards_dev || !dones_dev) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
   ON_DEVICE(h);
   return step_many_impl(h, num_steps, actions_dev, obs_dev, bits_dev, grid_dev, obs_every_step, rewards_dev, dones_dev, x,
                         (cudaStream_t)stream);
@@ -638,7 +619,7 @@ static bool packed(const snk_env* h) { return h->xfer_mode == XFER_PACKED; }
 // Device mirrors of the host-buffer calls.  The NHWC mirror (N * obs bytes) exists only for the raw transport;
 // the packed transport has the step kernel emit channel bits straight into d_bits (an eighth of the bytes).
 static int ensure_mirrors(snk_env* h, bool want_obs, bool want_bits) {
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   if (!h->h_actions) CU(cudaMalloc(&h->h_actions, (size_t)d.N * d.ns));
   if (want_obs && !h->h_obs) CU(cudaMalloc(&h->h_obs, (size_t)d.N * d.obs_env_bytes));
   if (want_bits && !h->d_bits) CU(cudaMalloc(&h->d_bits, (size_t)d.N * d.stage_env_bytes));
@@ -651,7 +632,7 @@ static int ensure_mirrors(snk_env* h, bool want_obs, bool want_bits) {
 // Packed: the kernel already wrote channel bits into d_bits; D2H in chunks, widen each chunk on the host pool as
 // soon as its copy lands while the next chunks are still on the link.  Returns with the host buffer complete.
 static int obs_to_host(snk_env* h, uint8_t* obs_host, cudaStream_t s) {
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   const size_t total = (size_t)d.N * d.obs_env_bytes;
   if (!packed(h)) {
     CU(cudaMemcpyAsync(obs_host, h->h_obs, total, cudaMemcpyDeviceToHost, s));
@@ -690,7 +671,7 @@ static int obs_to_host(snk_env* h, uint8_t* obs_host, cudaStream_t s) {
 }
 
 // Layout of the single output block used for small batches (all offsets 16-byte aligned).
-struct SmallLayout { size_t act, obs, rew, done, fin, rank, scores, counts, total; };
+struct SmallLayout { size_t act, obs, rew, done, extra[N_EXTRA], total; };
 static SmallLayout small_layout(const Dims& d) {
   auto up = [](size_t x) { return (x + 15) & ~(size_t)15; };
   const size_t nn = (size_t)d.N * d.ns;
@@ -699,17 +680,17 @@ static SmallLayout small_layout(const Dims& d) {
   L.obs = up(nn);
   L.rew = L.obs + up((size_t)d.N * d.obs_env_bytes);
   L.done = L.rew + up(nn * sizeof(double));
-  L.fin = L.done + up(nn);
-  L.rank = L.fin + up((size_t)d.N);
-  L.scores = L.rank + up(nn * sizeof(int32_t));
-  L.counts = L.scores + up(nn * sizeof(double));
-  L.total = L.counts + up(3 * nn * sizeof(int32_t));
+  L.total = L.done + up(nn);
+  for (int i = 0; i < N_EXTRA; ++i) {
+    L.extra[i] = L.total;
+    L.total += up(extra_bytes(d, i));
+  }
   return L;
 }
 
 static int step_host_small(snk_env* h, const SmallLayout& L, const uint8_t* actions_host, uint8_t* obs_host,
                            double* rewards_host, uint8_t* dones_host, const snk_step_extra* xh) {
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   const size_t nn = (size_t)d.N * d.ns;
   cudaStream_t s = h->own_stream;
   // Zero-copy (default): the block is pinned host memory mapped into the device's address space; the kernel reads
@@ -730,28 +711,20 @@ static int step_host_small(snk_env* h, const SmallLayout& L, const uint8_t* acti
   memcpy(hv + L.act, actions_host, nn);
   { int rc0 = own_stream_after_user_work(h); if (rc0) return rc0; }
   if (!zero_copy) CU(cudaMemcpyAsync(dv + L.act, hv + L.act, nn, cudaMemcpyHostToDevice, s));
-  snk_step_extra xd;
-  memset(&xd, 0, sizeof xd);
-  if (xh) {
-    xd.finished = dv + L.fin; xd.rank = (int32_t*)(dv + L.rank); xd.episode_scores = (double*)(dv + L.scores);
-    xd.episode_steps = (int32_t*)(dv + L.counts); xd.episode_fruits = xd.episode_steps + nn; xd.episode_kills = xd.episode_fruits + nn;
-  }
+  ExtraPtrs xdp;                                 // with terminal info, the kernel writes all of it into the block
+  for (int i = 0; i < N_EXTRA; ++i) xdp.p[i] = dv + L.extra[i];
+  const snk_step_extra xd = extra_struct(xdp);
   int rc = step_impl(h, dv + L.act, obs_host ? dv + L.obs : nullptr, nullptr, nullptr, (double*)(dv + L.rew), dv + L.done, xh ? &xd : nullptr, s);
   if (rc) return rc;
-  const size_t lo = obs_host ? L.obs : L.rew, hi = xh ? L.total : L.fin;
+  const size_t lo = obs_host ? L.obs : L.rew, hi = xh ? L.total : L.extra[0];
   if (!zero_copy) CU(cudaMemcpyAsync(hv + lo, dv + lo, hi - lo, cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
   if (obs_host) memcpy(obs_host, hv + L.obs, (size_t)d.N * d.obs_env_bytes);
   memcpy(rewards_host, hv + L.rew, nn * sizeof(double));
   memcpy(dones_host, hv + L.done, nn);
-  if (xh) {
-    if (xh->finished) memcpy(xh->finished, hv + L.fin, (size_t)d.N);
-    if (xh->rank) memcpy(xh->rank, hv + L.rank, nn * sizeof(int32_t));
-    if (xh->episode_scores) memcpy(xh->episode_scores, hv + L.scores, nn * sizeof(double));
-    if (xh->episode_steps) memcpy(xh->episode_steps, hv + L.counts, nn * sizeof(int32_t));
-    if (xh->episode_fruits) memcpy(xh->episode_fruits, hv + L.counts + nn * sizeof(int32_t), nn * sizeof(int32_t));
-    if (xh->episode_kills) memcpy(xh->episode_kills, hv + L.counts + 2 * nn * sizeof(int32_t), nn * sizeof(int32_t));
-  }
+  const ExtraPtrs out = extra_ptrs(xh);
+  for (int i = 0; i < N_EXTRA; ++i)
+    if (out.p[i]) memcpy(out.p[i], hv + L.extra[i], extra_bytes(d, i));
   return SNK_OK;
 }
 
@@ -761,7 +734,7 @@ extern "C" int snk_step_host_info(snk_env* h, const uint8_t* actions_host, uint8
   if (!actions_host || !rewards_host || !dones_host) return fail(SNK_E_INVALID, "actions, rewards and dones are required");
   ON_DEVICE(h);
   {
-    const SmallLayout L = small_layout(h->d);
+    const SmallLayout L = small_layout(h->kp.d);
     if (L.total <= 64 * 1024) return step_host_small(h, L, actions_host, obs_host, rewards_host, dones_host, xh);
   }
   const bool as_bits = obs_host && packed(h);  // packed transport: the kernel emits channel bits, no NHWC block at all
@@ -769,35 +742,25 @@ extern "C" int snk_step_host_info(snk_env* h, const uint8_t* actions_host, uint8
   if (rc) return rc;
   rc = own_stream_after_user_work(h);
   if (rc) return rc;
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   const size_t nn = (size_t)d.N * d.ns;
   cudaStream_t s = h->own_stream;
-  snk_step_extra xd;
-  memset(&xd, 0, sizeof xd);
-  if (xh) {                                    // device mirrors of the terminal-info outputs the caller asked for
-    if (!h->h_fin) CU(cudaMalloc(&h->h_fin, (size_t)d.N));
-    if (!h->h_rank) CU(cudaMalloc(&h->h_rank, nn * sizeof(int32_t)));
-    if (!h->h_scores) CU(cudaMalloc(&h->h_scores, nn * sizeof(double)));
-    if (!h->h_counts) CU(cudaMalloc(&h->h_counts, 3 * nn * sizeof(int32_t)));
-    if (xh->finished) xd.finished = h->h_fin;
-    if (xh->rank) xd.rank = h->h_rank;
-    if (xh->episode_scores) xd.episode_scores = h->h_scores;
-    if (xh->episode_steps) xd.episode_steps = h->h_counts;
-    if (xh->episode_fruits) xd.episode_fruits = h->h_counts + nn;
-    if (xh->episode_kills) xd.episode_kills = h->h_counts + 2 * nn;
+  const ExtraPtrs out = extra_ptrs(xh);
+  ExtraPtrs dev = {};                          // device mirrors of the terminal-info outputs the caller asked for
+  for (int i = 0; i < N_EXTRA; ++i) {
+    if (!out.p[i]) continue;
+    if (!h->h_extra[i]) CU(cudaMalloc(&h->h_extra[i], extra_bytes(d, i)));
+    dev.p[i] = h->h_extra[i];
   }
+  const snk_step_extra xd = extra_struct(dev);
   CU(cudaMemcpyAsync(h->h_actions, actions_host, nn, cudaMemcpyHostToDevice, s));
   rc = step_impl(h, h->h_actions, obs_host && !as_bits ? h->h_obs : nullptr, as_bits ? h->d_bits : nullptr, nullptr, h->h_rew, h->h_done,
                  xh ? &xd : nullptr, s);
   if (rc) return rc;
   CU(cudaMemcpyAsync(rewards_host, h->h_rew, nn * sizeof(double), cudaMemcpyDeviceToHost, s));
   CU(cudaMemcpyAsync(dones_host, h->h_done, nn, cudaMemcpyDeviceToHost, s));
-  if (xd.finished) CU(cudaMemcpyAsync(xh->finished, xd.finished, (size_t)d.N, cudaMemcpyDeviceToHost, s));
-  if (xd.rank) CU(cudaMemcpyAsync(xh->rank, xd.rank, nn * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  if (xd.episode_scores) CU(cudaMemcpyAsync(xh->episode_scores, xd.episode_scores, nn * sizeof(double), cudaMemcpyDeviceToHost, s));
-  if (xd.episode_steps) CU(cudaMemcpyAsync(xh->episode_steps, xd.episode_steps, nn * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  if (xd.episode_fruits) CU(cudaMemcpyAsync(xh->episode_fruits, xd.episode_fruits, nn * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  if (xd.episode_kills) CU(cudaMemcpyAsync(xh->episode_kills, xd.episode_kills, nn * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  for (int i = 0; i < N_EXTRA; ++i)
+    if (dev.p[i]) CU(cudaMemcpyAsync(out.p[i], dev.p[i], extra_bytes(d, i), cudaMemcpyDeviceToHost, s));
   if (obs_host) return obs_to_host(h, obs_host, s);
   CU(cudaStreamSynchronize(s));
   return SNK_OK;
@@ -812,7 +775,7 @@ extern "C" int snk_step_host_bits(snk_env* h, const uint8_t* actions_host, uint8
   if (rc) return rc;
   rc = own_stream_after_user_work(h);
   if (rc) return rc;
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   const size_t nn = (size_t)d.N * d.ns, units = (size_t)d.N * d.stage_env_bytes;
   cudaStream_t s = h->own_stream;
   CU(cudaMemcpyAsync(h->h_actions, actions_host, nn, cudaMemcpyHostToDevice, s));
@@ -1050,8 +1013,8 @@ extern "C" int snk_get_state(snk_env* h, const snk_state_view* out, void* stream
   if (!h || !out) return fail(SNK_E_INVALID, "null argument");
   if (out->cells && out->max_cells < 1) return fail(SNK_E_INVALID, "max_cells must be >= 1 when cells is given");
   ON_DEVICE(h);
-  const MapView mv = {h->maps, h->cur_map, nullptr, h->num_maps};
-  CU(launch_get_state(h->d, h->recs, h->base_grid, mv, h->err, to_view(out), (cudaStream_t)stream));
+  const MapView mv = {h->kp.pool, h->kp.cur_map, nullptr, h->kp.num_maps};
+  CU(launch_get_state(h->kp.d, h->kp.recs, h->kp.base_grid, mv, h->kp.err, to_view(out), (cudaStream_t)stream));
   note_user_stream(h, (cudaStream_t)stream);
   return SNK_OK;
 }
@@ -1060,13 +1023,12 @@ extern "C" int snk_set_state(snk_env* h, const snk_state_view* in, uint8_t* obs_
   if (!h || !in) return fail(SNK_E_INVALID, "null argument");
   if (!in->grid || !in->alive || !in->dir || !in->cells || !in->length || !in->alive_counter || !in->episode_length || in->max_cells < 2)
     return fail(SNK_E_INVALID, "set_state needs grid, alive, dir, cells, length, alive_counter, episode_length");
-  if (obs_dev && ((uintptr_t)obs_dev & 7)) return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
+  KParams p;
+  const int rc = call_params(h, p, MODE_ENCODE, nullptr, obs_dev, nullptr, nullptr, nullptr, nullptr, nullptr);
+  if (rc) return rc;
   ON_DEVICE(h);
-  const MapView mv = {h->maps, h->next_map, h->cur_map, h->num_maps};
-  CU(launch_set_state(h->d, h->recs, h->base_grid, mv, h->err, to_view(in), (cudaStream_t)stream));
-  KParams p = base_params(h);
-  p.mode = MODE_ENCODE; p.obs = obs_dev;
-  p.vec16 = check_vec16(h, obs_dev);
+  const MapView mv = {h->kp.pool, h->kp.next_map, h->kp.cur_map, h->kp.num_maps};
+  CU(launch_set_state(h->kp.d, h->kp.recs, h->kp.base_grid, mv, h->kp.err, to_view(in), (cudaStream_t)stream));
   CU(launch_tile_kernel(p, h->threads, h->smem_bytes, (cudaStream_t)stream));
   note_user_stream(h, (cudaStream_t)stream);
   h->was_reset = true;
@@ -1081,11 +1043,11 @@ static const uint64_t CKPT_MAGIC = 0x0031544B434B4E53ull;     // "SNKCKT1"
 static const uint64_t CKPT_MAGIC_POOL = 0x0031504B434B4E53ull;  // "SNKCKP1"
 struct CkptHeader { uint64_t magic; int32_t N, H, W, ns, K, V, fs, dig, rec_bytes, hist_env_bytes; double env_steps; };   // rec_bytes: per env in HBM
 
-static size_t ckpt_pool_bytes(const snk_env* h) { return h->num_maps ? sizeof(uint64_t) + 2 * (size_t)h->d.N : 0; }
+static size_t ckpt_pool_bytes(const snk_env* h) { return h->kp.num_maps ? sizeof(uint64_t) + 2 * (size_t)h->kp.d.N : 0; }
 
 extern "C" size_t snk_checkpoint_bytes(const snk_env* h) {
   if (!h) return 0;
-  return sizeof(CkptHeader) + (size_t)h->d.N * ((size_t)h->d.hbm_rec_bytes + (size_t)h->d.hist_env_bytes) + STAT_COUNT * sizeof(double) +
+  return sizeof(CkptHeader) + (size_t)h->kp.d.N * ((size_t)h->kp.d.hbm_rec_bytes + (size_t)h->kp.d.hist_env_bytes) + STAT_COUNT * sizeof(double) +
          ckpt_pool_bytes(h);
 }
 
@@ -1094,19 +1056,19 @@ extern "C" int snk_checkpoint_save(snk_env* h, void* blob_host, size_t bytes) {
   if (bytes < snk_checkpoint_bytes(h)) return fail(SNK_E_INVALID, "checkpoint buffer too small: %zu < %zu", bytes, snk_checkpoint_bytes(h));
   ON_DEVICE(h);
   CU(cudaDeviceSynchronize());
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   uint8_t* out = (uint8_t*)blob_host;
-  CkptHeader hd = {h->num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC, d.N, d.H, d.W, d.ns, d.K, d.V, d.fs, d.dig | (d.compact << 1),
+  CkptHeader hd = {h->kp.num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC, d.N, d.H, d.W, d.ns, d.K, d.V, d.fs, d.dig | (d.compact << 1),
                    d.hbm_rec_bytes, d.hist_env_bytes, 0.0};
   memcpy(out, &hd, sizeof hd); out += sizeof hd;
-  CU(cudaMemcpy(out, h->recs, (size_t)d.N * d.hbm_rec_bytes, cudaMemcpyDeviceToHost)); out += (size_t)d.N * d.hbm_rec_bytes;
-  if (d.hist_env_bytes) { CU(cudaMemcpy(out, h->hist, (size_t)d.N * d.hist_env_bytes, cudaMemcpyDeviceToHost)); out += (size_t)d.N * d.hist_env_bytes; }
-  CU(cudaMemcpy(out, h->stats, STAT_COUNT * sizeof(double), cudaMemcpyDeviceToHost));
-  if (h->num_maps) {
+  CU(cudaMemcpy(out, h->kp.recs, (size_t)d.N * d.hbm_rec_bytes, cudaMemcpyDeviceToHost)); out += (size_t)d.N * d.hbm_rec_bytes;
+  if (d.hist_env_bytes) { CU(cudaMemcpy(out, h->kp.hist, (size_t)d.N * d.hist_env_bytes, cudaMemcpyDeviceToHost)); out += (size_t)d.N * d.hist_env_bytes; }
+  CU(cudaMemcpy(out, h->kp.stats, STAT_COUNT * sizeof(double), cudaMemcpyDeviceToHost));
+  if (h->kp.num_maps) {
     out += STAT_COUNT * sizeof(double);
     memcpy(out, &h->pool_digest, sizeof(uint64_t)); out += sizeof(uint64_t);
-    CU(cudaMemcpy(out, h->next_map, (size_t)d.N, cudaMemcpyDeviceToHost)); out += d.N;
-    CU(cudaMemcpy(out, h->cur_map, (size_t)d.N, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out, h->kp.next_map, (size_t)d.N, cudaMemcpyDeviceToHost)); out += d.N;
+    CU(cudaMemcpy(out, h->kp.cur_map, (size_t)d.N, cudaMemcpyDeviceToHost));
   }
   return SNK_OK;
 }
@@ -1114,33 +1076,33 @@ extern "C" int snk_checkpoint_save(snk_env* h, void* blob_host, size_t bytes) {
 extern "C" int snk_checkpoint_load(snk_env* h, const void* blob_host, size_t bytes) {
   if (!h || !blob_host) return fail(SNK_E_INVALID, "null argument");
   if (bytes < snk_checkpoint_bytes(h)) return fail(SNK_E_INVALID, "checkpoint too small for this handle");
-  const Dims& d = h->d;
+  const Dims& d = h->kp.d;
   const uint8_t* in = (const uint8_t*)blob_host;
   CkptHeader hd;
   memcpy(&hd, in, sizeof hd); in += sizeof hd;
-  if (hd.magic != (h->num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC) && (hd.magic == CKPT_MAGIC || hd.magic == CKPT_MAGIC_POOL))
-    return fail(SNK_E_INVALID, h->num_maps ? "checkpoint was written by a handle without a wall-map pool"
+  if (hd.magic != (h->kp.num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC) && (hd.magic == CKPT_MAGIC || hd.magic == CKPT_MAGIC_POOL))
+    return fail(SNK_E_INVALID, h->kp.num_maps ? "checkpoint was written by a handle without a wall-map pool"
                                            : "checkpoint was written by a handle with a wall-map pool");
-  if (hd.magic != (h->num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC) || hd.N != d.N || hd.H != d.H || hd.W != d.W || hd.ns != d.ns || hd.K != d.K || hd.V != d.V ||
+  if (hd.magic != (h->kp.num_maps ? CKPT_MAGIC_POOL : CKPT_MAGIC) || hd.N != d.N || hd.H != d.H || hd.W != d.W || hd.ns != d.ns || hd.K != d.K || hd.V != d.V ||
       hd.fs != d.fs || hd.dig != (d.dig | (d.compact << 1)) || hd.rec_bytes != d.hbm_rec_bytes || hd.hist_env_bytes != d.hist_env_bytes)
     return fail(SNK_E_INVALID, "checkpoint was written by a handle of a different shape");
   const uint8_t* pool_part = in + (size_t)d.N * ((size_t)d.hbm_rec_bytes + (size_t)d.hist_env_bytes) + STAT_COUNT * sizeof(double);
-  if (h->num_maps) {
+  if (h->kp.num_maps) {
     uint64_t digest;
     memcpy(&digest, pool_part, sizeof digest);
     if (digest != h->pool_digest) return fail(SNK_E_INVALID, "checkpoint was written by a handle with a different wall-map pool");
     const uint8_t* cur = pool_part + sizeof(uint64_t) + d.N;
     for (int e = 0; e < d.N; ++e)
-      if (cur[e] >= h->num_maps) return fail(SNK_E_INVALID, "checkpoint: cur_map[%d] = %d names no map", e, cur[e]);
+      if (cur[e] >= h->kp.num_maps) return fail(SNK_E_INVALID, "checkpoint: cur_map[%d] = %d names no map", e, cur[e]);
   }
   ON_DEVICE(h);
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(h->recs, in, (size_t)d.N * d.hbm_rec_bytes, cudaMemcpyHostToDevice)); in += (size_t)d.N * d.hbm_rec_bytes;
-  if (d.hist_env_bytes) { CU(cudaMemcpy(h->hist, in, (size_t)d.N * d.hist_env_bytes, cudaMemcpyHostToDevice)); in += (size_t)d.N * d.hist_env_bytes; }
-  CU(cudaMemcpy(h->stats, in, STAT_COUNT * sizeof(double), cudaMemcpyHostToDevice));
-  if (h->num_maps) {
-    CU(cudaMemcpy(h->next_map, pool_part + sizeof(uint64_t), (size_t)d.N, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(h->cur_map, pool_part + sizeof(uint64_t) + d.N, (size_t)d.N, cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(h->kp.recs, in, (size_t)d.N * d.hbm_rec_bytes, cudaMemcpyHostToDevice)); in += (size_t)d.N * d.hbm_rec_bytes;
+  if (d.hist_env_bytes) { CU(cudaMemcpy(h->kp.hist, in, (size_t)d.N * d.hist_env_bytes, cudaMemcpyHostToDevice)); in += (size_t)d.N * d.hist_env_bytes; }
+  CU(cudaMemcpy(h->kp.stats, in, STAT_COUNT * sizeof(double), cudaMemcpyHostToDevice));
+  if (h->kp.num_maps) {
+    CU(cudaMemcpy(const_cast<uint8_t*>(h->kp.next_map), pool_part + sizeof(uint64_t), (size_t)d.N, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(h->kp.cur_map, pool_part + sizeof(uint64_t) + d.N, (size_t)d.N, cudaMemcpyHostToDevice));
   }
   h->was_reset = true;
   return SNK_OK;
@@ -1148,22 +1110,24 @@ extern "C" int snk_checkpoint_load(snk_env* h, const void* blob_host, size_t byt
 
 extern "C" int snk_set_replay(snk_env* h, const int32_t* draws_host, const int64_t* offsets_host) {
   if (!h || !offsets_host) return fail(SNK_E_INVALID, "null argument");
-  if (h->d.rng_mode != RNG_REPLAY) return fail(SNK_E_STATE, "handle was not created with SNK_RNG_REPLAY");
+  if (h->kp.d.rng_mode != RNG_REPLAY) return fail(SNK_E_STATE, "handle was not created with SNK_RNG_REPLAY");
   ON_DEVICE(h);
-  const int N = h->d.N;
+  const int N = h->kp.d.N;
   const int64_t total = offsets_host[N];
   if (offsets_host[0] != 0 || total < 0) return fail(SNK_E_INVALID, "offsets must start at 0 and be non-decreasing");
   for (int e = 0; e < N; ++e) if (offsets_host[e + 1] < offsets_host[e]) return fail(SNK_E_INVALID, "offsets must be non-decreasing");
   CU(cudaDeviceSynchronize());
-  cudaFree(h->replay); h->replay = nullptr;
-  CU(cudaMalloc(&h->replay, (size_t)(total > 0 ? total : 1) * sizeof(int32_t)));
+  cudaFree(const_cast<int32_t*>(h->kp.replay)); h->kp.replay = nullptr;
+  int32_t* replay = nullptr;
+  CU(cudaMalloc(&replay, (size_t)(total > 0 ? total : 1) * sizeof(int32_t)));
+  h->kp.replay = replay;                         // every later launch copies the template, so it reads the new stream
   if (total > 0) {
     if (!draws_host) return fail(SNK_E_INVALID, "null draws");
-    CU(cudaMemcpy(h->replay, draws_host, (size_t)total * sizeof(int32_t), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(replay, draws_host, (size_t)total * sizeof(int32_t), cudaMemcpyHostToDevice));
   }
-  CU(cudaMemcpy(h->replay_off, offsets_host, ((size_t)N + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(const_cast<int64_t*>(h->kp.replay_off), offsets_host, ((size_t)N + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
   // cursors live in the records: zero them
-  CU(cudaMemset2D(h->recs + h->d.hbm_c0 + (h->d.off_hdr - h->d.off_c0) + offsetof(EnvHdr, cursor), (size_t)h->d.hbm_rec_bytes, 0,
+  CU(cudaMemset2D(h->kp.recs + h->kp.d.hbm_c0 + (h->kp.d.off_hdr - h->kp.d.off_c0) + offsetof(EnvHdr, cursor), (size_t)h->kp.d.hbm_rec_bytes, 0,
                   sizeof(uint32_t), (size_t)N));
   return SNK_OK;
 }
@@ -1172,9 +1136,9 @@ extern "C" int snk_replay_cursors(snk_env* h, int32_t* cursors_host) {
   if (!h || !cursors_host) return fail(SNK_E_INVALID, "null argument");
   ON_DEVICE(h);
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy2D(cursors_host, sizeof(int32_t), h->recs + h->d.hbm_c0 + (h->d.off_hdr - h->d.off_c0) + offsetof(EnvHdr, cursor),
-                  (size_t)h->d.hbm_rec_bytes,
-                  sizeof(int32_t), (size_t)h->d.N, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy2D(cursors_host, sizeof(int32_t), h->kp.recs + h->kp.d.hbm_c0 + (h->kp.d.off_hdr - h->kp.d.off_c0) + offsetof(EnvHdr, cursor),
+                  (size_t)h->kp.d.hbm_rec_bytes,
+                  sizeof(int32_t), (size_t)h->kp.d.N, cudaMemcpyDeviceToHost));
   return SNK_OK;
 }
 
@@ -1182,14 +1146,14 @@ extern "C" int snk_device_errors(snk_env* h, uint32_t* bits, int clear) {
   if (!h || !bits) return fail(SNK_E_INVALID, "null argument");
   ON_DEVICE(h);
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(bits, h->err, sizeof(uint32_t), cudaMemcpyDeviceToHost));
-  if (clear) CU(cudaMemset(h->err, 0, sizeof(uint32_t)));
+  CU(cudaMemcpy(bits, h->kp.err, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+  if (clear) CU(cudaMemset(h->kp.err, 0, sizeof(uint32_t)));
   return SNK_OK;
 }
 
 extern "C" int snk_stats_dev(snk_env* h, double** stats_dev) {
   if (!h || !stats_dev) return fail(SNK_E_INVALID, "null argument");
-  *stats_dev = h->stats;
+  *stats_dev = h->kp.stats;
   return SNK_OK;
 }
 
@@ -1197,8 +1161,8 @@ extern "C" int snk_stats(snk_env* h, double* out_host, int clear) {
   if (!h || !out_host) return fail(SNK_E_INVALID, "null argument");
   ON_DEVICE(h);
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(out_host, h->stats, STAT_COUNT * sizeof(double), cudaMemcpyDeviceToHost));
-  if (clear) CU(cudaMemset(h->stats, 0, STAT_COUNT * sizeof(double)));
+  CU(cudaMemcpy(out_host, h->kp.stats, STAT_COUNT * sizeof(double), cudaMemcpyDeviceToHost));
+  if (clear) CU(cudaMemset(h->kp.stats, 0, STAT_COUNT * sizeof(double)));
   return SNK_OK;
 }
 

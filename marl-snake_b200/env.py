@@ -202,18 +202,9 @@ class SnakeBatch:
                 raise ValueError('mask must have one entry per environment')
             mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
         with torch.cuda.device(self.device):
-            if bits:
-                out = self._bits_buffer()
-                if self.global_state is not None:
-                    check(lib.snk_reset_grid(self._h, _ptr(mask), None, _ptr(out), _ptr(self.global_state), self._stream()))
-                else:
-                    check(lib.snk_reset_bits(self._h, _ptr(mask), _ptr(out), self._stream()))
-            else:
-                out = self._obs
-                if self.global_state is not None:
-                    check(lib.snk_reset_grid(self._h, _ptr(mask), _ptr(out), None, _ptr(self.global_state), self._stream()))
-                else:
-                    check(lib.snk_reset(self._h, _ptr(mask), _ptr(out), self._stream()))
+            out = self._bits_buffer() if bits else self._obs
+            check(lib.snk_reset_grid(self._h, _ptr(mask), None if bits else _ptr(out), _ptr(out) if bits else None,
+                                     _ptr(self.global_state), self._stream()))
         # a masked reset rewrites the observation of the selected envs only: the others keep theirs
         self._mutated('reset(bits=True)' if bits else (None if mask is None else False))
         return out.clone() if copy else out
@@ -222,17 +213,25 @@ class SnakeBatch:
         """As step(), but the observation comes as channel bits: uint8 [N, ns, oh, ow, fs], one byte per window cell
         and frame, bit c = channel c (np.packbits(obs.reshape(..., fs, 8), -1, bitorder='little')).  The encode
         writes them directly -- no NHWC block, an eighth of the observation traffic; `unpack_obs` widens them."""
+        return self._step(actions, copy, want_info, bits=True)
+
+    def step(self, actions, copy=False, want_obs=True, want_info=True):
+        """actions: uint8 CUDA tensor [N, ns] in {0,1,2} (observer 'snake') or {0..4} ('human').  Returns (obs, rewards f64, dones bool, info)
+        where info holds per-env `finished` and, for finished envs, the terminal `rank` / `episode_*`
+        arrays the reference puts in its info dict (snake_env.py:396-410).  The returned tensors are
+        the batch's own buffers, overwritten by the next call unless copy=True."""
+        return self._step(actions, copy, want_info, want_obs=want_obs)
+
+    def _step(self, actions, copy, want_info, bits=False, want_obs=True):
+        """Body of step (observation, or none) and step_bits (channel bits)."""
         if actions.dtype != torch.uint8 or actions.device != self.device or not actions.is_contiguous() \
                 or actions.numel() != self.num_envs * self.num_snakes:
             raise ValueError('actions must be a contiguous uint8 CUDA tensor of shape [num_envs, num_snakes]')
-        out = self._bits_buffer()
-        if self.global_state is not None:
-            check(lib.snk_step_grid(self._h, _ptr(actions), None, _ptr(out), _ptr(self.global_state), _ptr(self._rew),
-                                    _ptr(self._done), C.byref(self._extra) if want_info else None, self._stream()))
-        else:
-            check(lib.snk_step_bits(self._h, _ptr(actions), _ptr(out), _ptr(self._rew), _ptr(self._done),
-                                    C.byref(self._extra) if want_info else None, self._stream()))
-        self._mutated('step_bits')
+        out = self._bits_buffer() if bits else self._obs if want_obs else None
+        check(lib.snk_step_grid(self._h, _ptr(actions), None if bits else _ptr(out), _ptr(out) if bits else None,
+                                _ptr(self.global_state), _ptr(self._rew), _ptr(self._done),
+                                C.byref(self._extra) if want_info else None, self._stream()))
+        self._mutated('step_bits' if bits else None if want_obs else 'step(want_obs=False)')
         info = {}
         if want_info:
             info = dict(finished=self._fin.view(torch.bool), rank=self._rank, episode_scores=self._ep_scores,
@@ -240,35 +239,9 @@ class SnakeBatch:
                         episode_kills=self._ep_kills)
         res = (out, self._rew, self._done.view(torch.bool), info)
         if copy:
-            res = (out.clone(), res[1].clone(), res[2].clone(), {k: v.clone() for k, v in info.items()})
-        return res
-
-    def step(self, actions, copy=False, want_obs=True, want_info=True):
-        """actions: uint8 CUDA tensor [N, ns] in {0,1,2} (observer 'snake') or {0..4} ('human').  Returns (obs, rewards f64, dones bool, info)
-        where info holds per-env `finished` and, for finished envs, the terminal `rank` / `episode_*`
-        arrays the reference puts in its info dict (snake_env.py:396-410).  The returned tensors are
-        the batch's own buffers, overwritten by the next call unless copy=True."""
-        if actions.dtype != torch.uint8 or actions.device != self.device or not actions.is_contiguous() \
-                or actions.numel() != self.num_envs * self.num_snakes:
-            raise ValueError('actions must be a contiguous uint8 CUDA tensor of shape [num_envs, num_snakes]')
-        if self.global_state is not None:
-            check(lib.snk_step_grid(self._h, _ptr(actions), _ptr(self._obs if want_obs else None), None,
-                                    _ptr(self.global_state), _ptr(self._rew), _ptr(self._done),
-                                    C.byref(self._extra) if want_info else None, self._stream()))
-        else:
-            check(lib.snk_step(self._h, _ptr(actions), _ptr(self._obs if want_obs else None), _ptr(self._rew),
-                               _ptr(self._done), C.byref(self._extra) if want_info else None, self._stream()))
-        self._mutated(None if want_obs else 'step(want_obs=False)')
-        info = {}
-        if want_info:
-            info = dict(finished=self._fin.view(torch.bool), rank=self._rank, episode_scores=self._ep_scores,
-                        episode_steps=self._ep_steps, episode_fruits=self._ep_fruits,
-                        episode_kills=self._ep_kills)
-        out = (self._obs if want_obs else None, self._rew, self._done.view(torch.bool), info)
-        if copy:
-            out = (None if out[0] is None else out[0].clone(), out[1].clone(), out[2].clone(),
+            res = (None if out is None else out.clone(), res[1].clone(), res[2].clone(),
                    {k: v.clone() for k, v in info.items()})
-        return out
+        return res
 
     def step_many(self, actions, obs=None, rewards=None, dones=None, bits=None, finished=None, global_state=None):
         """T steps in one call (snk_step_many) for open-loop action streams.  actions: uint8 CUDA [T, N, ns].
@@ -315,13 +288,9 @@ class SnakeBatch:
         grid = global_state
         if grid is None and self.global_state is not None and not every:
             grid = self.global_state                        # the last step's rows straight into the batch's buffer
-        if grid is not None:
-            check(lib.snk_step_many_grid(self._h, T, _ptr(actions), _ptr(obs), _ptr(bits), _ptr(grid), int(bool(every)),
-                                         _ptr(rewards), _ptr(dones), C.byref(extra) if extra is not None else None,
-                                         self._stream()))
-        else:
-            check(lib.snk_step_many(self._h, T, _ptr(actions), _ptr(obs), _ptr(bits), int(bool(every)), _ptr(rewards),
-                                    _ptr(dones), C.byref(extra) if extra is not None else None, self._stream()))
+        check(lib.snk_step_many_grid(self._h, T, _ptr(actions), _ptr(obs), _ptr(bits), _ptr(grid), int(bool(every)),
+                                     _ptr(rewards), _ptr(dones), C.byref(extra) if extra is not None else None,
+                                     self._stream()))
         if self.global_state is not None and grid is not self.global_state:
             if grid is not None:
                 self.global_state.copy_(grid[-1] if every else grid)
@@ -530,6 +499,43 @@ def _tensor_from_ptr(ptr, n, dtype, device):
     return torch.as_tensor(h, device=device)
 
 
+class _HostStepper:
+    """The host buffers of a batch's host-buffer calls: one C-ABI call per step (snk_step_host_info: actions in, step,
+    observation / rewards / dones / terminal info out, one synchronisation) or per reset (snk_reset_host).  `pinned`
+    page-locks the buffers, which lets the large transfers of a big batch run asynchronously."""
+
+    def __init__(self, batch, pinned=False):
+        N, ns = batch.num_envs, batch.num_snakes
+
+        def host(shape, dtype):
+            a = np.zeros(shape, dtype=dtype)
+            return torch.from_numpy(a).pin_memory().numpy() if pinned else a
+        self.act = host((N, ns), np.uint8)
+        self.obs = host((N,) + batch.obs_shape, np.uint8)
+        self.rew, self.done = host((N, ns), np.float64), host((N, ns), np.uint8)
+        self.fin, self.rank = host((N,), np.uint8), host((N, ns), np.int32)
+        self.scores, self.counts = host((N, ns), np.float64), host((3, N, ns), np.int32)
+        self._xh = SnkStepExtra(self.fin.ctypes.data, self.rank.ctypes.data, self.scores.ctypes.data,
+                                self.counts[0].ctypes.data, self.counts[1].ctypes.data, self.counts[2].ctypes.data)
+        # the buffers never move: their addresses (and the handle) are converted for ctypes once, not on every step
+        act, obs, rew, done = (x.ctypes.data_as(C.c_void_p) for x in (self.act, self.obs, self.rew, self.done))
+        self._step_args = (batch._h, act, obs, rew, done, C.byref(self._xh))
+        self._reset_args = (batch._h, obs)
+
+    def reset(self):
+        check(lib.snk_reset_host(*self._reset_args))
+
+    def step(self):
+        check(lib.snk_step_host_info(*self._step_args))
+
+    def info(self, e):
+        """The reference's terminal info dict of env e (snake_env.py:396-410); valid where fin[e] is set."""
+        return dict(rank=[int(r) for r in self.rank[e]], episode_scores=self.scores[e].copy(),
+                    episode_steps=self.counts[0, e].astype(np.float64),
+                    episode_fruits=self.counts[1, e].astype(np.float64),
+                    episode_kills=self.counts[2, e].astype(np.float64))
+
+
 class SnakeEnv:
     """Drop-in for the reference's SnakeEnv (one environment, host-side return types).
 
@@ -568,23 +574,7 @@ class SnakeEnv:
         self.obs_ch = b.obs_ch
         self.action_space = Discrete(len(self.action_dict) * self.num_snakes)             # snake_env.py:107-109
         self.observation_space = Box(self.low, self.high, b.obs_shape, np.uint8)          # snake_env.py:115-129
-        # host buffers of the single-environment call: one C-ABI call per step (snk_step_host_info: actions
-        # in, step, observation / rewards / dones / terminal info out, one synchronisation)
-        ns = self.num_snakes
-        self._h_act = np.zeros((1, ns), dtype=np.uint8)
-        self._h_obs = np.empty((1,) + b.obs_shape, dtype=np.uint8)
-        self._h_rew = np.empty((1, ns), dtype=np.float64)
-        self._h_done = np.empty((1, ns), dtype=np.uint8)
-        self._h_fin = np.zeros(1, dtype=np.uint8)
-        self._h_rank = np.zeros((1, ns), dtype=np.int32)
-        self._h_scores = np.zeros((1, ns), dtype=np.float64)
-        self._h_counts = np.zeros((3, 1, ns), dtype=np.int32)
-        self._xh = SnkStepExtra(self._h_fin.ctypes.data, self._h_rank.ctypes.data, self._h_scores.ctypes.data,
-                                self._h_counts[0].ctypes.data, self._h_counts[1].ctypes.data,
-                                self._h_counts[2].ctypes.data)
-        # the buffers never move: their addresses (and the handle) are converted for ctypes once, not on every step
-        self._step_args = (self._batch._h,) + tuple(x.ctypes.data_as(C.c_void_p) for x in
-                                                    (self._h_act, self._h_obs, self._h_rew, self._h_done)) + (C.byref(self._xh),)
+        self._host = _HostStepper(b)
 
     @property
     def unwrapped(self):
@@ -600,9 +590,9 @@ class SnakeEnv:
         self._batch.close()
 
     def reset(self):
-        check(lib.snk_reset_host(self._batch._h, self._h_obs.ctypes.data_as(C.c_void_p)))
+        self._host.reset()
         self.frame_buffer = []                                                            # snake_env.py:151
-        return self._h_obs[0].copy()
+        return self._host.obs[0].copy()
 
     def _alive_now(self):
         return self._batch.get_state()['alive'][0].cpu().numpy().astype(bool)
@@ -611,27 +601,22 @@ class SnakeEnv:
         if isinstance(actions, int):
             actions = [actions]
         assert len(actions) == self.num_snakes                                            # snake_env.py:313
-        alive = None
+        hs, alive = self._host, None
         for i, ac in enumerate(actions):
             if isinstance(ac, np.ndarray):
                 ac = ac.item()
             if self.observer == 'human':              # unknown actions keep the direction (:610-632)
-                self._h_act[0, i] = int(ac) if ac in (0, 1, 2, 3, 4) else 0
+                hs.act[0, i] = int(ac) if ac in (0, 1, 2, 3, 4) else 0
                 continue
             if ac not in self.action_dict:            # the reference looks the action up only for live snakes
                 alive = self._alive_now() if alive is None else alive
                 if alive[i]:
                     raise KeyError(ac)                                                    # snake_env.py:606
                 ac = 0
-            self._h_act[0, i] = int(ac)
-        check(lib.snk_step_host_info(*self._step_args))
-        info = {}
-        if self._h_fin[0]:
-            info['rank'] = [int(r) for r in self._h_rank[0]]
-            info['episode_scores'] = self._h_scores[0].copy()
-            for k, name in enumerate(('episode_steps', 'episode_fruits', 'episode_kills')):
-                info[name] = self._h_counts[k, 0].astype(np.float64)
-        return (self._h_obs[0].copy(), self._h_rew[0].tolist(), self._h_done[0].astype(bool).tolist(), info)
+            hs.act[0, i] = int(ac)
+        hs.step()
+        info = hs.info(0) if hs.fin[0] else {}
+        return (hs.obs[0].copy(), hs.rew[0].tolist(), hs.done[0].astype(bool).tolist(), info)
 
     @property
     def grid(self):

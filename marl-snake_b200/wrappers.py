@@ -4,13 +4,10 @@ marlenv/wrappers.py (make_snake :203-223, SingleAgent :84-105, SingleMultiAgent 
 The reference vectorises with one OS process per environment (gym AsyncVectorEnv, :211-212); here
 `num_envs > 1` is one `SnakeBatch` on the GPU with the reference worker's auto-reset rule (:138-146).
 """
-import ctypes as C
-
 import numpy as np
 import torch
 
-from ._lib import SnkStepExtra, check, lib
-from .env import SnakeBatch
+from .env import SnakeBatch, _HostStepper
 from .registration import make
 from .spaces import Box, Discrete
 
@@ -136,21 +133,7 @@ class VectorSnakeEnv:
         self.single_action_space = self.action_space = Discrete(len(self.action_dict))
         self._act = torch.zeros((num_envs, num_snakes), dtype=torch.uint8, device=b.device)
         if output != 'torch':
-            N, ns = num_envs, num_snakes
-
-            def host(shape, dtype):
-                return torch.zeros(shape, dtype=dtype).pin_memory().numpy()
-            self._h_act = host((N, ns), torch.uint8)
-            self._h_obs = host((N,) + b.obs_shape, torch.uint8)
-            self._h_rew, self._h_done = host((N, ns), torch.float64), host((N, ns), torch.uint8)
-            self._h_fin, self._h_rank = host((N,), torch.uint8), host((N, ns), torch.int32)
-            self._h_scores, self._h_counts = host((N, ns), torch.float64), host((3, N, ns), torch.int32)
-            self._xh = SnkStepExtra(self._h_fin.ctypes.data, self._h_rank.ctypes.data, self._h_scores.ctypes.data,
-                                    self._h_counts[0].ctypes.data, self._h_counts[1].ctypes.data,
-                                    self._h_counts[2].ctypes.data)
-            # the buffers never move: convert their addresses for ctypes once, not on every step
-            self._step_args = (b._h,) + tuple(x.ctypes.data_as(C.c_void_p) for x in
-                                              (self._h_act, self._h_obs, self._h_rew, self._h_done)) + (C.byref(self._xh),)
+            self._host = _HostStepper(b, pinned=True)
 
     def _squeeze(self, x):
         return x[:, 0] if self.num_snakes == 1 else x
@@ -162,8 +145,8 @@ class VectorSnakeEnv:
     def reset(self):
         if self.output == 'torch':
             return self._squeeze(self.batch.reset())
-        check(lib.snk_reset_host(self.batch._h, self._h_obs.ctypes.data_as(C.c_void_p)))
-        return self._out(self._h_obs)
+        self._host.reset()
+        return self._out(self._host.obs)
 
     def step(self, actions):
         if self.output == 'torch':
@@ -185,16 +168,14 @@ class VectorSnakeEnv:
             a = np.where((a < 0) | (a > 2), 0, a)
         elif self.batch.observer == 'human':
             a = np.where((a < 0) | (a > 4), 0, a)
-        self._h_act[...] = a
-        check(lib.snk_step_host_info(*self._step_args))
+        hs = self._host
+        hs.act[...] = a
+        hs.step()
         infos = [{} for _ in range(self.num_envs)]
-        if self.num_snakes > 1 and self._h_fin.any():
-            for e in np.nonzero(self._h_fin)[0]:
-                infos[e] = dict(rank=[int(r) for r in self._h_rank[e]], episode_scores=self._h_scores[e].copy(),
-                                episode_steps=self._h_counts[0, e].astype(np.float64),
-                                episode_fruits=self._h_counts[1, e].astype(np.float64),
-                                episode_kills=self._h_counts[2, e].astype(np.float64))
-        return self._out(self._h_obs), self._out(self._h_rew), self._out(self._h_done.view(np.bool_)), tuple(infos)
+        if self.num_snakes > 1 and hs.fin.any():
+            for e in np.nonzero(hs.fin)[0]:
+                infos[e] = hs.info(e)
+        return self._out(hs.obs), self._out(hs.rew), self._out(hs.done.view(np.bool_)), tuple(infos)
 
     def close(self):
         self.batch.close()
