@@ -243,8 +243,8 @@ __device__ __forceinline__ void dirp_set_atomic(uint8_t* dirp, int c, int v) {
 
 // Wall-map pool: the map id `m` read from a caller-written array, checked.  An id that is not a map raises the sticky
 // ERR_MAP_RANGE bit and reads as map 0, so a bad id never leads to a read outside the pool.
-__device__ __forceinline__ uint32_t checked_map(const KParams& p, uint32_t m) {
-  if (m >= (uint32_t)p.num_maps) { atomicOr(p.err, ERR_MAP_RANGE); m = 0u; }
+__device__ __forceinline__ uint32_t checked_map(uint32_t m, int num_maps, uint32_t* err) {
+  if (m >= (uint32_t)num_maps) { atomicOr(err, ERR_MAP_RANGE); m = 0u; }
   return m;
 }
 
@@ -261,7 +261,7 @@ __device__ __noinline__ void reset_env_warp(const KParams& p, uint8_t* g, uint8_
   uint32_t m = 0;
   if constexpr (kPool) {
     if (lane == 0) {
-      m = checked_map(p, p.next_map[env_local]);
+      m = checked_map(p.next_map[env_local], p.num_maps, p.err);
       p.cur_map[env_local] = (uint8_t)m;
     }
     m = __shfl_sync(0xffffffffu, m, 0);
@@ -414,6 +414,15 @@ __device__ __forceinline__ void st_cs_64(void* p, uint2 a) {
   SNK_CHECK_OBS(p, 8);
   __stcs(reinterpret_cast<uint2*>(p), a);
 }
+// One 16-byte unit of a viewer block at dst: window cells a and b, 8 bytes each.  A block of an odd cell count is only
+// 8-byte aligned, so the unit at either end of it may hold one cell; has_a / has_b say which cells lie in the block.
+// A lane's second unit never starts before the block, so its callers pass has_a = true rather than a test the
+// compiler cannot fold.
+__device__ __forceinline__ void st_cs_unit(uint8_t* dst, bool has_a, bool has_b, uint2 a, uint2 b) {
+  if (has_a && has_b) st_cs_128(dst, a, b);
+  else if (has_a) st_cs_64(dst, a);
+  else st_cs_64(dst + 8, b);
+}
 
 // Channel-bit output (snk_step_bits): one byte per window cell, bit c = channel c.  The byte LUT mirrors the 8-byte
 // LUT entry for entry, so the entry address `e8` of a cell (lut32 + 8 * index) names its byte at lutb32 + index.
@@ -495,6 +504,32 @@ __device__ __forceinline__ void bulk_store(void* dst, uint32_t src, uint32_t byt
   asm volatile("cp.async.bulk.commit_group;" ::: "memory");
 }
 __device__ __forceinline__ void bulk_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+// The record tile's bulk copies between HBM (the ne records from e0 on) and shared memory (shared address s32), hinted
+// evict_last when the handle asks for it (KParams::l2_keep).  The address is spelled out in each branch on purpose:
+// computed once ahead of the branch, it changes the register allocation of every kernel instance.
+__device__ __forceinline__ void load_records(const KParams& p, int e0, uint32_t s32, uint32_t bytes, uint32_t mbar) {
+  if (p.l2_keep) bulk_load_hint(s32, p.recs + (size_t)e0 * p.d.hbm_rec_bytes, bytes, mbar, l2_policy_evict_last(p.l2_keep_frac));
+  else bulk_load(s32, p.recs + (size_t)e0 * p.d.hbm_rec_bytes, bytes, mbar);
+}
+// Write the tile's records back, shared -> HBM: the elected thread's bulk store, or without TMA 16-byte copies by the
+// tile's threads (first, step).  `wait`: the issuer waits for the store's shared-memory reads here; otherwise the
+// caller does before the shared memory is reused or the CTA exits.  `s` is the tile's first byte as it lies in HBM,
+// s32 its shared address.
+__device__ __forceinline__ void store_records(const KParams& p, int e0, int ne, const uint8_t* s, uint32_t s32,
+                                              uint32_t bytes, bool elected, bool wait, int first, int step) {
+  if (p.use_tma) {
+    if (elected) {
+      if (p.l2_keep) bulk_store_hint(p.recs + (size_t)e0 * p.d.hbm_rec_bytes, s32, bytes, l2_policy_evict_last(p.l2_keep_frac));
+      else bulk_store(p.recs + (size_t)e0 * p.d.hbm_rec_bytes, s32, bytes);
+      if (wait) bulk_store_wait_read();
+    }
+  } else {
+    uint4* dst = reinterpret_cast<uint4*>(p.recs + (size_t)e0 * p.d.hbm_rec_bytes);
+    const uint4* src = reinterpret_cast<const uint4*>(s);
+    const int n16 = ne * (p.d.hbm_rec_bytes >> 4);
+    for (int k = first; k < n16; k += step) dst[k] = src[k];
+  }
+}
 
 struct GroupOut {
   int fruit_taken;     // fruit draws owed by this lane's environment (same on all its lanes)
@@ -787,11 +822,16 @@ __device__ __forceinline__ void viewer_origin(const Dims& d, const uint8_t* base
   if (V > 0) { const int hr = hc / W; r0 = hr - V; c0 = hc - hr * W - V; }
 }
 
-// Valid window rows / columns of a viewer as bit masks (rows in bits 0..15, columns in 16..31).
+// Window rows / columns of a viewer that fall inside the grid, as bit masks: rows in bits 0..oh-1, columns from bit
+// `col_shift` on.
+__device__ __forceinline__ uint32_t window_valid(int oh, int ow, int H, int W, int r0, int c0, int col_shift) {
+  const int rlo = max(0, -r0), rhi = min(oh, H - r0), clo = max(0, -c0), chi = min(ow, W - c0);
+  return (((1u << rhi) - 1u) & ~((1u << rlo) - 1u)) | ((((1u << chi) - 1u) & ~((1u << clo) - 1u)) << col_shift);
+}
+// The same for the encode table's entries (rows in bits 0..15, columns in 16..31).
 __device__ __forceinline__ uint32_t window_mask(int V, int oh, int ow, int H, int W, int r0, int c0) {
   if (V <= 0) return 0u;
-  const int rlo = max(0, -r0), rhi = min(oh, H - r0), clo = max(0, -c0), chi = min(ow, W - c0);
-  return (((1u << rhi) - 1u) & ~((1u << rlo) - 1u)) | ((((1u << chi) - 1u) & ~((1u << clo) - 1u)) << 16);
+  return window_valid(oh, ow, H, W, r0, c0, 16);
 }
 
 // frame_stack 1: one warp encodes one viewer straight to global memory.  snake_env.py:474-519.
@@ -846,15 +886,8 @@ __device__ __forceinline__ void encode_viewer_fs1(const KParams& p, const SH& sh
       if (outv) {
         const uint2 qa0 = lds_v2(la0 + ka0 * 8u), qb0 = lds_v2(lb0 + kb0 * 8u);
         const uint2 qa1 = lds_v2(la1 + ka1 * 8u), qb1 = lds_v2(lb1 + kb1 * 8u);
-        uint8_t* dst0 = outv + (ptrdiff_t)ca0 * 8;
-        if (ca0 >= 0 && ca0 + 1 < ohw) st_cs_128(dst0, qa0, qb0);
-        else if (ca0 >= 0) st_cs_64(dst0, qa0);
-        else st_cs_64(dst0 + 8, qb0);
-        if (has1) {
-          uint8_t* dst1 = outv + (ptrdiff_t)ca1 * 8;
-          if (ca1 + 1 < ohw) st_cs_128(dst1, qa1, qb1);
-          else st_cs_64(dst1, qa1);
-        }
+        st_cs_unit(outv + (ptrdiff_t)ca0 * 8, ca0 >= 0, ca0 + 1 < ohw, qa0, qb0);
+        if (has1) st_cs_unit(outv + (ptrdiff_t)ca1 * 8, true, ca1 + 1 < ohw, qa1, qb1);
       }
       if (bitsv) {
         emit_bits(bitsv, ca0, ohw, lut32, lutb32, la0 + ka0 * 8u, lb0 + kb0 * 8u);
@@ -882,7 +915,7 @@ __device__ __forceinline__ void encode_viewer_fs1(const KParams& p, const SH& sh
         if ((unsigned)rr < (unsigned)H && (unsigned)cc < (unsigned)W) codeb = cell_code(d, grid[rr * W + cc]);
         qb = lut[codeb];
       }
-      if (outv) {
+      if (outv) {               // st_cs_unit, written out: through the helper this loop is scheduled differently
         uint8_t* dst = outv + (ptrdiff_t)ca * 8;
         if (va && vb) st_cs_128(dst, qa, qb);
         else if (va) st_cs_64(dst, qa);
@@ -905,21 +938,23 @@ __device__ __forceinline__ void encode_viewer_fs1(const KParams& p, const SH& sh
 // reads LUT entry 0 (all zero), the reference's zero padding (snake_env.py:506-515).
 struct CellWords { uint32_t w[2][4]; };     // [address parity of the viewer block][unit 0 cell a, b, unit 1 cell a, b]
 
+// Cell word of window cell c (inside the viewer block).
+template <class SH>
+__device__ __forceinline__ uint32_t cell_word(const SH& sh, int c, int B) {
+  const int ow = sh.ow(), ci = c / ow, cj = c - ci * ow;
+  return (1u << ci) | (1u << (sh.oh() + cj)) | ((uint32_t)(ci * sh.W() + cj) << B);
+}
+
 template <class SH>
 __device__ __forceinline__ CellWords make_cell_words(const SH& sh, int B) {
-  const int lane = (int)lane_id(), ohw = sh.ohw(), ow = sh.ow(), oh = sh.oh(), W = sh.W();
+  const int lane = (int)lane_id(), ohw = sh.ohw();
   CellWords cw;
 #pragma unroll
   for (int s = 0; s < 2; ++s)
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
       const int c = 2 * (lane + 32 * (k >> 1)) - s + (k & 1);
-      uint32_t w = 0x80000000u;
-      if (c >= 0 && c < ohw) {
-        const int ci = c / ow, cj = c - ci * ow;
-        w = (1u << ci) | (1u << (oh + cj)) | ((uint32_t)(ci * W + cj) << B);
-      }
-      cw.w[s][k] = w;
+      cw.w[s][k] = (c >= 0 && c < ohw) ? cell_word(sh, c, B) : 0x80000000u;
     }
   return cw;
 }
@@ -931,8 +966,7 @@ __device__ __forceinline__ uint32_t make_viewer_word(const KParams& p, const SH&
   const int W = sh.W(), oh = sh.oh(), ow = sh.ow(), B = sh.view_bits();
   int r0, c0;
   viewer_origin(d, base, sh.ns(), W, d.V, v, r0, c0);
-  const int rlo = max(0, -r0), rhi = min(oh, d.H - r0), clo = max(0, -c0), chi = min(ow, W - c0);
-  const uint32_t valid = (((1u << rhi) - 1u) & ~((1u << rlo) - 1u)) | ((((1u << chi) - 1u) & ~((1u << clo) - 1u)) << oh);
+  const uint32_t valid = window_valid(oh, ow, d.H, W, r0, c0, oh);
   return (~valid & ((1u << B) - 1u)) | ((uint32_t)(r0 * W + c0 + sh.view_bias()) << B);
 }
 
@@ -956,7 +990,7 @@ __device__ __forceinline__ bool pair_unit_used(const SH& sh, int k, int lane) {
 
 template <class SH>
 __device__ __forceinline__ CellWords make_pair_cell_words(const SH& sh) {
-  const int lane = (int)lane_id(), ohw = sh.ohw(), ow = sh.ow(), oh = sh.oh(), W = sh.W(), B = sh.view_bits();
+  const int lane = (int)lane_id(), ohw = sh.ohw(), B = sh.view_bits();
   CellWords cw;
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
@@ -966,12 +1000,7 @@ __device__ __forceinline__ CellWords make_pair_cell_words(const SH& sh) {
     for (int s = 0; s < 2; ++s) {
       int c = 2 * u + s;
       if (c >= ohw) c -= ohw;                                  // window cell inside its own viewer
-      uint32_t w = 0x80000000u;
-      if (used) {
-        const int ci = c / ow, cj = c - ci * ow;
-        w = (1u << ci) | (1u << (oh + cj)) | ((uint32_t)(ci * W + cj) << B);
-      }
-      cw.w[s][k] = w;
+      cw.w[s][k] = used ? cell_word(sh, c, B) : 0x80000000u;
     }
   }
   return cw;
@@ -1047,17 +1076,8 @@ __device__ __forceinline__ void encode_viewer_reg(const KParams& p, const SH& sh
   if (outv) {
     const uint2 q0 = lds_v2(lutv32 + k0 * 8u), q1 = lds_v2(lutv32 + k1 * 8u);
     const uint2 q2 = lds_v2(lutv32 + k2 * 8u), q3 = lds_v2(lutv32 + k3 * 8u);
-    if (lane < units) {
-      uint8_t* dst0 = outv + (ptrdiff_t)ca0 * 8;
-      if (ca0 >= 0 && ca0 + 1 < ohw) st_cs_128(dst0, q0, q1);
-      else if (ca0 >= 0) st_cs_64(dst0, q0);
-      else st_cs_64(dst0 + 8, q1);
-    }
-    if (lane + 32 < units) {
-      uint8_t* dst1 = outv + (ptrdiff_t)ca1 * 8;
-      if (ca1 + 1 < ohw) st_cs_128(dst1, q2, q3);
-      else st_cs_64(dst1, q2);
-    }
+    if (lane < units) st_cs_unit(outv + (ptrdiff_t)ca0 * 8, ca0 >= 0, ca0 + 1 < ohw, q0, q1);
+    if (lane + 32 < units) st_cs_unit(outv + (ptrdiff_t)ca1 * 8, true, ca1 + 1 < ohw, q2, q3);
   }
   if (bitsv) {
     emit_bits(bitsv, ca0, ohw, lut32, lutb32, lutv32 + k0 * 8u, lutv32 + k1 * 8u);
@@ -1110,17 +1130,8 @@ __device__ __forceinline__ void encode_viewer_pad(const KParams& p, const SH& sh
     const int ca0 = 2 * u0 - shift, ca1 = 2 * u1 - shift;
     if (outv) {
       const uint2 q0 = lds_v2(a0), q1 = lds_v2(a1), q2 = lds_v2(a2), q3 = lds_v2(a3);
-      if (u0 < units) {
-        uint8_t* dst0 = outv + (ptrdiff_t)ca0 * 8;
-        if (ca0 >= 0 && ca0 + 1 < ohw) st_cs_128(dst0, q0, q1);
-        else if (ca0 >= 0) st_cs_64(dst0, q0);
-        else st_cs_64(dst0 + 8, q1);
-      }
-      if (u1 < units) {
-        uint8_t* dst1 = outv + (ptrdiff_t)ca1 * 8;
-        if (ca1 + 1 < ohw) st_cs_128(dst1, q2, q3);
-        else st_cs_64(dst1, q2);
-      }
+      if (u0 < units) st_cs_unit(outv + (ptrdiff_t)ca0 * 8, ca0 >= 0, ca0 + 1 < ohw, q0, q1);
+      if (u1 < units) st_cs_unit(outv + (ptrdiff_t)ca1 * 8, true, ca1 + 1 < ohw, q2, q3);
     }
     if (bitsv) {
       emit_bits(bitsv, ca0, ohw, lut32, lutb32, a0, a1);
@@ -1149,21 +1160,25 @@ __device__ __forceinline__ void encode_viewer_direct(const SH& sh, uint32_t grid
     if (outv) {
       const uint2 q0 = lds_v2(lutv32 + k0 * 8u), q1 = lds_v2(lutv32 + k1 * 8u);
       const uint2 q2 = lds_v2(lutv32 + k2 * 8u), q3 = lds_v2(lutv32 + k3 * 8u);
-      uint8_t* dst0 = outv + (ptrdiff_t)ca0 * 8;
-      if (ca0 >= 0 && ca0 + 1 < ohw) st_cs_128(dst0, q0, q1);
-      else if (ca0 >= 0) st_cs_64(dst0, q0);
-      else st_cs_64(dst0 + 8, q1);
-      if (has1) {
-        uint8_t* dst1 = outv + (ptrdiff_t)ca1 * 8;
-        if (ca1 + 1 < ohw) st_cs_128(dst1, q2, q3);
-        else st_cs_64(dst1, q2);
-      }
+      st_cs_unit(outv + (ptrdiff_t)ca0 * 8, ca0 >= 0, ca0 + 1 < ohw, q0, q1);
+      if (has1) st_cs_unit(outv + (ptrdiff_t)ca1 * 8, true, ca1 + 1 < ohw, q2, q3);
     }
     if (bitsv) {
       emit_bits(bitsv, ca0, ohw, lut32, lutb32, lutv32 + k0 * 8u, lutv32 + k1 * 8u);
       if (has1) emit_bits(bitsv, ca1, ohw, lut32, lutb32, lutv32 + k2 * 8u, lutv32 + k3 * 8u);
     }
   }
+}
+
+// frame_stack 1, one viewer in the flavour kEnc (not the viewer pairs): grid `base` of the environment at shared address
+// grid32, its virtual record base vb, the viewer's packed word vw (ENC_REG).
+template <int kEnc, class SH>
+__device__ __forceinline__ void encode_viewer(const KParams& p, const SH& sh, const uint8_t* base, const uint8_t* vb,
+                                              uint32_t grid32, uint32_t vw, const CellWords& cw, int v, uint8_t* outv,
+                                              uint32_t lut32, uint8_t* bitsv, uint32_t lutb32) {
+  if (kEnc == ENC_REG) encode_viewer_reg(p, sh, grid32, vw, cw, v, outv, lut32, bitsv, lutb32);
+  else if (kEnc == ENC_DIRECT) encode_viewer_direct(sh, grid32, v, outv, lut32, (uint32_t)p.d.code_mask, bitsv, lutb32);
+  else encode_viewer_fs1(p, sh, base, vb, grid32, v, outv, lut32, bitsv, lutb32);
 }
 
 // frame_stack > 1: one warp encodes one environment.  Channel-bit bytes of all fs frames are staged in
@@ -1316,17 +1331,16 @@ __device__ __forceinline__ void encode_env_stacked(const KParams& p, const SH& s
 // bulk: compact records with H*W a multiple of 16 (off_c0 == H*W, so the tile's grids are ONE contiguous block, and
 // they carry no direction bits) and a 16-byte aligned output: one bulk copy by the tile's elected thread, after the
 // rule warp's fence.proxy.async; the issuer waits for its shared-memory reads before the CTA exits or the next step's
-// rules run.  Otherwise plain stores of cell codes (full records: stride rec_bytes, direction bits masked off).
-template <bool kCoop>
+// rules run.  Otherwise plain stores of cell codes by the tile's threads (first, step) (full records: stride rec_bytes,
+// direction bits masked off).
 __device__ __forceinline__ void store_grid_rows(const KParams& p, const TilePtr& tp, int e0, int ne, uint8_t* out,
-                                                bool bulk, bool elected) {
+                                                bool bulk, bool elected, int first, int step) {
   const Dims& d = p.d;
   uint8_t* const rows = out + (size_t)e0 * d.HW;
   if (bulk) {
     if (elected) bulk_store(rows, (uint32_t)__cvta_generic_to_shared(tp.g), (uint32_t)(ne * d.HW));
     return;
   }
-  const int first = kCoop ? (int)threadIdx.x : (int)lane_id(), step = kCoop ? (int)blockDim.x : 32;
   if (((d.HW | (int)reinterpret_cast<uintptr_t>(rows)) & 15) == 0) {
     const uint32_t cm4 = (uint32_t)d.code_mask * 0x01010101u;
     const int n16 = d.HW >> 4;
@@ -1419,6 +1433,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
   // ---- stage the tile's records: HBM -> shared.  One bulk asynchronous copy (TMA) issued by the tile's
   //      elected thread and awaited on an mbarrier, or 128-bit coalesced loads (p.use_tma == 0).
   const bool elected = kCoop ? tid == 0 : lane == 0;
+  const int first = kCoop ? tid : (int)lane, step = kCoop ? nt : 32;    // the tile's threads, for strided copies
   const uint32_t rec32 = (uint32_t)__cvta_generic_to_shared(s_c);
   const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(s_flag) + 32u;     // flags: 32 B, mbarrier: 8 B
   const uint32_t tile_load_bytes = (uint32_t)ne * (uint32_t)d.hbm_rec_bytes;
@@ -1432,8 +1447,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
       mbar_init(mbar, 1);
       if (ne > 0) {
         mbar_expect_tx(mbar, tile_load_bytes + grid_load_bytes + hist_load_bytes + (blob_by_tma ? (uint32_t)p.enc_copy_bytes : 0u));
-        if (p.l2_keep) bulk_load_hint(rec32, p.recs + (size_t)e0 * d.hbm_rec_bytes, tile_load_bytes, mbar, l2_policy_evict_last(p.l2_keep_frac));
-        else bulk_load(rec32, p.recs + (size_t)e0 * d.hbm_rec_bytes, tile_load_bytes, mbar);
+        load_records(p, e0, rec32, tile_load_bytes, mbar);
         if (!kPool && grid_load_bytes) bulk_load((uint32_t)__cvta_generic_to_shared(s_rec), p.base_grid, grid_load_bytes, mbar);
         if (hist_load_bytes) bulk_load((uint32_t)__cvta_generic_to_shared(s_hist), p.hist + (size_t)e0 * d.hist_env_bytes, hist_load_bytes, mbar);
         if (blob_by_tma) bulk_load((uint32_t)__cvta_generic_to_shared(s_lut), p.enc_blob, (uint32_t)p.enc_copy_bytes, mbar);
@@ -1445,7 +1459,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
       if (grid_load_bytes && (!kCoop || warp == 0)) {
         __syncwarp();
         if ((int)lane < ne) {
-          const uint32_t m = checked_map(p, p.cur_map[e0 + (int)lane]);
+          const uint32_t m = checked_map(p.cur_map[e0 + (int)lane], p.num_maps, p.err);
           bulk_load((uint32_t)__cvta_generic_to_shared(s_rec) + lane * (uint32_t)d.off_c0, p.pool + (size_t)m * d.off_c0,
                     (uint32_t)d.off_c0, mbar);
         }
@@ -1455,25 +1469,24 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
     const uint4* src = reinterpret_cast<const uint4*>(p.recs + (size_t)e0 * d.hbm_rec_bytes);
     uint4* dst = reinterpret_cast<uint4*>(s_c);
     const int n16 = ne * (d.hbm_rec_bytes >> 4);
-    if (kCoop) { for (int k = tid; k < n16; k += nt) dst[k] = __ldcs(src + k); }
-    else { for (int k = (int)lane; k < n16; k += 32) dst[k] = __ldcs(src + k); }
+    for (int k = first; k < n16; k += step) dst[k] = __ldcs(src + k);
     const uint4* gsrc = reinterpret_cast<const uint4*>(p.base_grid);
     uint4* gdst = reinterpret_cast<uint4*>(s_rec);
     const int g16 = (int)(grid_load_bytes >> 4);
     if constexpr (kPool) {       // unit k of the tile's grids is unit k % (off_c0 / 16) of environment k / (off_c0 / 16)'s map
       const int u16 = d.off_c0 >> 4;
-      for (int k = kCoop ? tid : (int)lane; k < g16; k += kCoop ? nt : 32) {
+      for (int k = first; k < g16; k += step) {
         const int q = k / u16;
-        const uint32_t m = checked_map(p, p.cur_map[e0 + q]);
+        const uint32_t m = checked_map(p.cur_map[e0 + q], p.num_maps, p.err);
         gdst[k] = __ldg(reinterpret_cast<const uint4*>(p.pool + (size_t)m * d.off_c0) + (k - q * u16));
       }
-    } else if (kCoop) { for (int k = tid; k < g16; k += nt) gdst[k] = __ldg(gsrc + k); }
-    else { for (int k = (int)lane; k < g16; k += 32) gdst[k] = __ldg(gsrc + k); }
+    } else {
+      for (int k = first; k < g16; k += step) gdst[k] = __ldg(gsrc + k);
+    }
     const uint4* hsrc = reinterpret_cast<const uint4*>(p.hist + (size_t)e0 * d.hist_env_bytes);
     uint4* hdst = reinterpret_cast<uint4*>(s_hist);
     const int h16 = (int)(hist_load_bytes >> 4);
-    if (kCoop) { for (int k = tid; k < h16; k += nt) hdst[k] = __ldcs(hsrc + k); }
-    else { for (int k = (int)lane; k < h16; k += 32) hdst[k] = __ldcs(hsrc + k); }
+    for (int k = first; k < h16; k += step) hdst[k] = __ldcs(hsrc + k);
   }
   // ---- encode tables: host-built blob, L2-resident, copied with 128-bit loads.  fs == 1: {cell code ->
   //      8 output bytes, window-cell table}; fs > 1: {cell code -> channel-bit byte, table}.
@@ -1558,26 +1571,13 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
   SNK_T(t_synced);
   if (ne == 0) return;
   if constexpr (kGrid) {
-    if (grid_t) store_grid_rows<kCoop>(p, tp, e0, ne, grid_t, grid_bulk, elected);
+    if (grid_t) store_grid_rows(p, tp, e0, ne, grid_t, grid_bulk, elected, first, step);
   }
 
   if (fs == 1) {
     // ---- write the records back: shared -> HBM (nothing below modifies them).  The bulk store runs
     //      asynchronously under the encode; its issuer waits for the shared-memory reads before exiting.
-    if (last) {
-      if (p.use_tma) {
-        if (elected) {
-          if (p.l2_keep) bulk_store_hint(p.recs + (size_t)e0 * d.hbm_rec_bytes, rec32, tile_load_bytes, l2_policy_evict_last(p.l2_keep_frac));
-          else bulk_store(p.recs + (size_t)e0 * d.hbm_rec_bytes, rec32, tile_load_bytes);
-        }
-      } else {
-        uint4* dst = reinterpret_cast<uint4*>(p.recs + (size_t)e0 * d.hbm_rec_bytes);
-        const uint4* src = reinterpret_cast<const uint4*>(s_c);
-        const int n16 = ne * (d.hbm_rec_bytes >> 4);
-        if (kCoop) { for (int k = tid; k < n16; k += nt) dst[k] = src[k]; }
-        else { for (int k = (int)lane; k < n16; k += 32) dst[k] = src[k]; }
-      }
-    }
+    if (last) store_records(p, e0, ne, s_c, rec32, tile_load_bytes, elected, false, first, step);
     // this step's observation block (every step of a multi-step launch, or only the last one)
     const bool render = want_obs && (last || (kMulti && p.obs_every_step));
     uint8_t* const obs_t = (p.obs && render) ? p.obs + ((kMulti && p.obs_every_step) ? (size_t)t * d.N * d.obs_env_bytes : 0) : nullptr;
@@ -1653,9 +1653,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
           const uint32_t grid32 = (uint32_t)__cvta_generic_to_shared(base);
           uint8_t* outv = obs_t ? obs_t + ((size_t)(e0 + q) * ns + v) * (size_t)ohw * 8 : nullptr;
           uint8_t* bitsv = bits_t ? bits_t + ((size_t)(e0 + q) * ns + v) * (size_t)ohw : nullptr;
-          if (kEnc == ENC_REG) encode_viewer_reg(p, sh, grid32, s_view[q * G + v], cw, v, outv, lut32, bitsv, lutb32);
-          else if (kEnc == ENC_DIRECT) encode_viewer_direct(sh, grid32, v, outv, lut32, (uint32_t)d.code_mask, bitsv, lutb32);
-          else encode_viewer_fs1(p, sh, base, tp.VB(q), grid32, v, outv, lut32, bitsv, lutb32);
+          encode_viewer<kEnc>(p, sh, base, tp.VB(q), grid32, s_view[q * G + v], cw, v, outv, lut32, bitsv, lutb32);
         }
       } else {
 #pragma unroll 1
@@ -1669,9 +1667,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
           for (int v = 0; v < ns; ++v) {
             uint8_t* outv = outq ? outq + (size_t)v * ohw * 8 : nullptr;
             uint8_t* bitsv = bitsq ? bitsq + (size_t)v * ohw : nullptr;
-            if (kEnc == ENC_REG) encode_viewer_reg(p, sh, grid32, s_view[q * G + v], cw, v, outv, lut32, bitsv, lutb32);
-            else if (kEnc == ENC_DIRECT) encode_viewer_direct(sh, grid32, v, outv, lut32, (uint32_t)d.code_mask, bitsv, lutb32);
-            else encode_viewer_fs1(p, sh, base, tp.VB(q), grid32, v, outv, lut32, bitsv, lutb32);
+            encode_viewer<kEnc>(p, sh, base, tp.VB(q), grid32, s_view[q * G + v], cw, v, outv, lut32, bitsv, lutb32);
           }
         }
       }
@@ -1715,19 +1711,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
   if (p.use_tma && (!kCoop || warp == 0)) fence_proxy_async();        // hpos updates -> async proxy
   if (kCoop) __syncthreads(); else __syncwarp();
   // ---- write the records back: shared -> HBM
-  if (p.use_tma) {
-    if (elected) {
-      if (p.l2_keep) bulk_store_hint(p.recs + (size_t)e0 * d.hbm_rec_bytes, rec32, tile_load_bytes, l2_policy_evict_last(p.l2_keep_frac));
-      else bulk_store(p.recs + (size_t)e0 * d.hbm_rec_bytes, rec32, tile_load_bytes);
-      bulk_store_wait_read();
-    }
-  } else {
-    uint4* dst = reinterpret_cast<uint4*>(p.recs + (size_t)e0 * d.hbm_rec_bytes);
-    const uint4* src = reinterpret_cast<const uint4*>(s_c);
-    const int n16 = ne * (d.hbm_rec_bytes >> 4);
-    if (kCoop) { for (int k = tid; k < n16; k += nt) dst[k] = src[k]; }
-    else { for (int k = (int)lane; k < n16; k += 32) dst[k] = src[k]; }
-  }
+  store_records(p, e0, ne, s_c, rec32, tile_load_bytes, elected, true, first, step);
 }
 
 // ---- state export / import (parity + checkpoint interface; thread per environment) ----------------
@@ -1737,8 +1721,7 @@ snk_tile_kernel(const __grid_constant__ KParams p) {
 __device__ __forceinline__ const uint8_t* env_walls(const Dims& d, const uint8_t* base_grid, const MapView& mv, int e,
                                                     uint32_t* err) {
   if (!mv.pool) return base_grid;
-  uint32_t m = mv.map_ids[e];
-  if (m >= (uint32_t)mv.num_maps) { atomicOr(err, ERR_MAP_RANGE); m = 0u; }
+  const uint32_t m = checked_map(mv.map_ids[e], mv.num_maps, err);
   if (mv.cur_out) mv.cur_out[e] = (uint8_t)m;
   return mv.pool + (size_t)m * d.off_c0;
 }
@@ -1912,27 +1895,24 @@ void encode_blob_fill(const Dims& d, uint8_t* out) {
   size_t off, lutb;
   encode_blob_bytes(d, &off, &lutb);
   uint8_t* wb = out + lutb;                                       // fs == 1: the byte LUT
+  auto put_fs1 = [&](int k, uint32_t bits) {                      // fs == 1 entry k: 8 output bytes and the bits byte
+    w[2 * k] = spread4(bits & 15u);
+    w[2 * k + 1] = spread4(bits >> 4);
+    wb[k] = (uint8_t)bits;
+  };
   if (encode_lut_dual(d)) {
     for (int own = 0; own < 2; ++own)
       for (int code = 0; code < LS; ++code) {
         // viewer = owner of the code for the as-own half, some other snake for the as-other half
         const uint32_t owner = (uint32_t)code / 10u;
-        const uint32_t bits = cell_bits((uint32_t)code, own ? owner : owner + 1u);
-        w[2 * (own * LS + code)] = spread4(bits & 15u);
-        w[2 * (own * LS + code) + 1] = spread4(bits >> 4);
-        wb[own * LS + code] = (uint8_t)bits;
+        put_fs1(own * LS + code, cell_bits((uint32_t)code, own ? owner : owner + 1u));
       }
   } else {
     for (int v = 0; v < d.ns; ++v)
       for (int code = 0; code < LS; ++code) {
         const uint32_t bits = cell_bits((uint32_t)code, (uint32_t)v);
-        if (d.fs == 1) {
-          w[2 * (v * LS + code)] = spread4(bits & 15u);
-          w[2 * (v * LS + code) + 1] = spread4(bits >> 4);
-          wb[v * LS + code] = (uint8_t)bits;
-        } else {
-          out[v * LS + code] = (uint8_t)bits;
-        }
+        if (d.fs == 1) put_fs1(v * LS + code, bits);
+        else out[v * LS + code] = (uint8_t)bits;
       }
   }
   if (!encode_uses_table(d)) return;
