@@ -60,8 +60,11 @@ enum {
                                     bodies (the resident record stores only those), or it holds more fruit cells than
                                     the record has slots (num_fruits + num_snakes, rounded up to 8); with a
                                     wall-map pool, in either record layout: its walls are not those of next_map */
-  SNK_DEV_MAP_RANGE = 128        /* wall-map pool: a map id (next_map, or cur_map rewritten by the caller) was not below
+  SNK_DEV_MAP_RANGE = 128,       /* wall-map pool: a map id (next_map, or cur_map rewritten by the caller) was not below
                                     the number of maps; map 0 was used instead                          */
+  SNK_DEV_SNAPSHOT = 256         /* snk_snapshot: an env id outside [0, N) (its slot matches no handle); snk_restore: a slot
+                                    index neither -1 nor below num_slots, or a slot of a handle whose digest differs --
+                                    that env was left unchanged and its observation not written          */
 };
 
 enum { SNK_RNG_PHILOX = 0, SNK_RNG_REPLAY = 1 };
@@ -285,6 +288,43 @@ int snk_set_state(snk_env* env, const snk_state_view* in, uint8_t* obs_dev, void
 size_t snk_checkpoint_bytes(const snk_env* env);
 int snk_checkpoint_save(snk_env* env, void* blob_host, size_t bytes);
 int snk_checkpoint_load(snk_env* env, const void* blob_host, size_t bytes);
+
+/* Per-env SNAPSHOT / RESTORE on the device, for search and lookahead (save a root, clone it into many envs, expand each
+ * with other actions, rewind), restarts from an archive of states, fair population evaluation and A/B checks.
+ *
+ * A slot is a small header (a 64-bit configuration digest and the env's cur_map), then the env's raw record as it lies in
+ * device memory, then its frame history (frame_stack > 1).  The digest covers what gives those bytes their meaning:
+ * height, width, num_snakes, vision_range, frame_stack, the record layout (compact / full, body directions in the grid
+ * byte or in a plane) and its sizes, the episode counters' width (16 bits unless max_episode_steps > 65535), the fruit
+ * slots, and the wall layout (the pool's digest with a wall-map pool, else the single layout's).  Slots restore into any
+ * handle with the same digest -- which may differ in num_envs, seed, env_id_offset, rewards and auto_reset -- and are
+ * refused (SNK_DEV_SNAPSHOT) by every other.
+ *
+ * Restore copies the record byte for byte, so the whole episode carries over: bodies, fruit slots, directions,
+ * alive_counter, episode_length, the per-snake episode statistics (the terminal info of a restored episode is the
+ * original's), the frame ring and its position, the Philox event counter and the replay cursor.  Draws stay keyed by the
+ * DESTINATION's global env id: a slot restored into the env it was taken from continues exactly as that env did after the
+ * snapshot; restored into another env it continues that env's own stream from the source's event count -- a different,
+ * deterministic future (a chance node).  In replay mode the cursor likewise indexes the destination's stream.  cur_map
+ * comes from the slot; next_map is left alone.  No step is executed: snk_stats (SNK_STAT_ENV_STEPS included) does not
+ * change.  Both calls only enqueue work on `stream` (stream rules as for the other device-pointer calls), never
+ * synchronise and allocate nothing, so they can be captured in a CUDA graph.  Either call before the handle's first
+ * reset returns SNK_E_STATE. */
+/* Bytes of one snapshot slot (a 16-byte multiple).  Depends on the configuration, not on num_envs; 0 for NULL. */
+size_t snk_snapshot_bytes(const snk_env* env);
+/* Slot i of snap_dev := the state of env env_ids_dev[i], for i < count (env_ids_dev NULL: envs 0..count-1).  snap_dev is
+ * count * snk_snapshot_bytes, 16-byte aligned (SNK_E_INVALID otherwise, and for count outside [1, N]).  Duplicated ids
+ * are fine.  An id outside [0, N) raises SNK_DEV_SNAPSHOT and writes a slot that no handle accepts. */
+int snk_snapshot(snk_env* env, const int32_t* env_ids_dev, int32_t count, void* snap_dev, void* stream);
+/* For every env e with src_dev[e] >= 0 (int32 [N]), env e := slot src_dev[e] of snap_dev (num_slots >= 1 slots, 16-byte
+ * aligned); src_dev[e] == -1 keeps env e.  Indexed by destination, so one slot may fan out to any number of envs.  Then
+ * writes the observation of the restored envs into obs_dev / bits_dev and their grid rows into grid_dev (the formats of
+ * snk_reset_grid; any of the three may be NULL, in any combination): the bytes the step that reached the restored state
+ * returned.  Rows of other envs keep their bytes; grid rows of other envs may be rewritten with their unchanged grid.  A
+ * slot index neither -1 nor below num_slots, or a slot whose digest differs, raises SNK_DEV_SNAPSHOT and leaves that env
+ * and its rows unchanged. */
+int snk_restore(snk_env* env, const int32_t* src_dev, int32_t num_slots, const void* snap_dev, uint8_t* obs_dev,
+                uint8_t* bits_dev, uint8_t* grid_dev, void* stream);
 
 /* Replay mode: per-env streams of recorded draw OUTPUTS in consumption order -- per reset the ns
  * accepted spawn-candidate indices (np.random.permutation, snake_env.py:581) then the fruit ranks

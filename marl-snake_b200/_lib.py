@@ -18,7 +18,9 @@ DEV_ERRORS = {1: 'action outside {0,1,2}', 2: 'replay stream exhausted',
               16: 'internal bounds check failed (debug build)',
               32: "a record tile's bulk copy timed out; the tile was skipped",
               64: 'set_state: grid is not walls + fruits + live snakes, or too many fruit cells',
-              128: 'a map id was not below the number of wall maps; map 0 was used'}
+              128: 'a map id was not below the number of wall maps; map 0 was used',
+              256: 'snapshot of an env id outside [0, N), or restore from a slot index out of range or a slot of '
+                   'another configuration; that env was left unchanged'}
 SNK_MAX_MAPS = 256
 STAT_NAMES = ('episodes', 'return_sum', 'episode_steps_sum', 'fruits_sum', 'kills_sum', 'deaths',
               'env_steps', 'reserved')
@@ -91,6 +93,10 @@ PROTOTYPES = {
     'snk_checkpoint_bytes': (C.c_size_t, [C.c_void_p]),
     'snk_checkpoint_save': (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
     'snk_checkpoint_load': (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
+    'snk_snapshot_bytes': (C.c_size_t, [C.c_void_p]),
+    'snk_snapshot': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    'snk_restore': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                              C.c_void_p]),
     'snk_set_replay': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     'snk_replay_cursors': (C.c_int, [C.c_void_p, C.c_void_p]),
     'snk_device_errors': (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32), C.c_int]),

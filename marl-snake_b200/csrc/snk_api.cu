@@ -83,6 +83,8 @@ struct snk_env {
   int many_tile_envs = 0, many_threads = 0;      // tile shape of multi-step launches (snk_step_many, cooperative tiles)
   size_t many_smem_bytes = 0;
   uint64_t pool_digest = 0;                      // layouts + spawn-table sizes: a checkpoint only loads into the same pool
+  uint64_t snap_digest = 0;                      // what gives a snapshot slot's bytes their meaning (snapshot_digest)
+  uint8_t* restore_mask = nullptr;               // [N] envs the last snk_restore restored: its encode's mask
   // ordering between the caller's streams (device-pointer calls) and own_stream (host-buffer calls)
   cudaStream_t last_user_stream = nullptr;
   bool user_work_pending = false;
@@ -142,6 +144,17 @@ static uint64_t fnv1a(uint64_t h, const void* data, size_t n) {
   return h;
 }
 
+// Snapshot slots (snk_snapshot) hold raw records: they restore only into handles whose records mean the same bytes --
+// shape, record layout, counter width, fruit slots and wall layout (pool digest or the single layout's).  Never 0.
+static uint64_t snapshot_digest(const Dims& d, uint64_t walls) {
+  struct { int32_t H, W, ns, V, fs, ohw_p, compact, dig, hbm_rec_bytes, hist_env_bytes, stat16, fcap; uint64_t walls; } k;
+  memset(&k, 0, sizeof k);
+  k.H = d.H; k.W = d.W; k.ns = d.ns; k.V = d.V; k.fs = d.fs; k.ohw_p = d.ohw_p; k.compact = d.compact; k.dig = d.dig;
+  k.hbm_rec_bytes = d.hbm_rec_bytes; k.hist_env_bytes = d.hist_env_bytes; k.stat16 = d.stat16; k.fcap = d.fcap; k.walls = walls;
+  const uint64_t h = fnv1a(0xCBF29CE484222325ull, &k, sizeof k);
+  return h ? h : 1;
+}
+
 static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_host, const uint8_t* map_ids_host, snk_env** out) {
   if (!c || !out) return fail(SNK_E_INVALID, "null argument");
   if (c->abi_version != SNK_ABI_VERSION) return fail(SNK_E_INVALID, "abi_version %d != %d", c->abi_version, SNK_ABI_VERSION);
@@ -195,6 +208,7 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
     }
   }
   const uint8_t* wm = walls_host ? walls.data() : nullptr;
+  uint64_t layout_digest = 0;                    // of the single wall layout (walled box or custom map), no pool
 
   // spawn table (host) -- core/grid_util.py:73-115.  A pool concatenates one table per map.
   std::vector<uint64_t> table;
@@ -361,6 +375,7 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
     const int copies = !d.compact ? 1 : h->kp.E > h->many_tile_envs ? h->kp.E : h->many_tile_envs;
     std::vector<uint8_t> tpl((size_t)copies * d.off_c0, 0);
     for (int i = 0; i < d.HW; ++i) tpl[i] = wm ? wm[i] : wall_or_empty(i, d.H, d.W);
+    layout_digest = fnv1a(0xCBF29CE484222325ull, tpl.data(), (size_t)d.HW);
     for (int k = 1; k < copies; ++k) memcpy(tpl.data() + (size_t)k * d.off_c0, tpl.data(), (size_t)d.off_c0);
     CUH(upload(h->kp.base_grid, tpl.data(), tpl.size()));
   }
@@ -386,8 +401,10 @@ static int create_impl(const snk_config* c, int num_maps, const uint8_t* walls_h
   CUH(launch_init_records(d, h->kp.recs, nullptr));
   CUH(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
   CUH(cudaEventCreateWithFlags(&h->user_ev, cudaEventDisableTiming));
+  CUH(cudaMalloc(&h->restore_mask, (size_t)d.N));     // last: every buffer before it lies where it did without it
   CUH(cudaDeviceSynchronize());
 #undef CUH
+  h->snap_digest = snapshot_digest(d, num_maps ? h->pool_digest : layout_digest);
   {
     // host entry points: ship channel bits and widen on the host once the observation block is large
     // enough for the PCIe link to matter (SNK_HOST_TRANSPORT = raw | packed overrides)
@@ -411,6 +428,7 @@ extern "C" int snk_destroy(snk_env* h) {
   cudaFree(h->h_actions); cudaFree(h->h_obs); cudaFree(h->h_rew); cudaFree(h->h_done);
   for (uint8_t* b : h->h_extra) cudaFree(b);
   cudaFree(h->small_dev);
+  cudaFree(h->restore_mask);
   if (h->small_host) cudaFreeHost(h->small_host);
   cudaFree(h->d_bits);
   if (h->p_bits) cudaFreeHost(h->p_bits);
@@ -1032,6 +1050,55 @@ extern "C" int snk_set_state(snk_env* h, const snk_state_view* in, uint8_t* obs_
   CU(launch_tile_kernel(p, h->threads, h->smem_bytes, (cudaStream_t)stream));
   note_user_stream(h, (cudaStream_t)stream);
   h->was_reset = true;
+  return SNK_OK;
+}
+
+// ---- per-env snapshot / restore on the device: slots of SnapHdr + raw record + frame history (snapshot_slot_bytes)
+extern "C" size_t snk_snapshot_bytes(const snk_env* h) { return h ? snapshot_slot_bytes(h->kp.d) : 0; }
+
+extern "C" int snk_snapshot(snk_env* h, const int32_t* env_ids_dev, int32_t count, void* snap_dev, void* stream) {
+  if (!h || !snap_dev) return fail(SNK_E_INVALID, "null argument");
+  if (!h->was_reset) return fail(SNK_E_STATE, "snapshot before reset");
+  if ((uintptr_t)snap_dev & 15) return fail(SNK_E_INVALID, "snap must be 16-byte aligned");
+  if (count < 1 || count > h->kp.d.N) return fail(SNK_E_INVALID, "count must be in 1..%d", h->kp.d.N);
+  ON_DEVICE(h);
+  const KParams& p = h->kp;
+  CU(launch_snapshot(p.d, p.recs, p.hist, p.cur_map, env_ids_dev, count, h->snap_digest, (uint8_t*)snap_dev, p.err,
+                     (cudaStream_t)stream));
+  note_user_stream(h, (cudaStream_t)stream);
+  return SNK_OK;
+}
+
+extern "C" int snk_restore(snk_env* h, const int32_t* src_dev, int32_t num_slots, const void* snap_dev, uint8_t* obs_dev,
+                           uint8_t* bits_dev, uint8_t* grid_dev, void* stream) {
+  if (!h || !src_dev || !snap_dev) return fail(SNK_E_INVALID, "null argument");
+  if (!h->was_reset) return fail(SNK_E_STATE, "restore before reset");
+  if ((uintptr_t)snap_dev & 15) return fail(SNK_E_INVALID, "snap must be 16-byte aligned");
+  if (num_slots < 1) return fail(SNK_E_INVALID, "num_slots must be >= 1");
+  ON_DEVICE(h);
+  const Dims& d = h->kp.d;
+  const bool out = obs_dev || bits_dev || grid_dev;
+  KParams p;                                     // the observation's launch: the encode of the restored envs only
+  if (out && d.fs == 1) {
+    const int rc = call_params(h, p, MODE_ENCODE, nullptr, obs_dev, bits_dev, grid_dev, nullptr, nullptr, nullptr);
+    if (rc) return rc;
+    p.mask = h->restore_mask;
+  } else if (obs_dev && ((uintptr_t)obs_dev & 7)) {
+    return fail(SNK_E_INVALID, "obs must be 8-byte aligned");
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  CU(launch_restore(d, h->kp.recs, h->kp.hist, h->kp.cur_map, src_dev, num_slots, (const uint8_t*)snap_dev, h->snap_digest,
+                    h->restore_mask, h->kp.err, s));
+  // frame_stack 1: MODE_ENCODE rebuilds each restored env's grid from its record (and cur_map) and encodes it; it skips
+  // the other envs and writes no record byte that differs.  frame_stack > 1: its F_INIT would refill the history, so
+  // the restored ring is widened as it stands.
+  if (out && d.fs == 1) CU(launch_tile_kernel(p, h->threads, h->smem_bytes, s));
+  if (out && d.fs > 1) {
+    const MapView mv = {h->kp.pool, h->kp.cur_map, nullptr, h->kp.num_maps};
+    CU(launch_emit_stacked(d, h->kp.recs, h->kp.hist, h->kp.base_grid, mv, h->restore_mask, obs_dev, bits_dev, grid_dev,
+                           h->kp.err, s));
+  }
+  note_user_stream(h, s);
   return SNK_OK;
 }
 

@@ -28,7 +28,9 @@ enum : uint32_t { ERR_BAD_ACTION = 1, ERR_REPLAY_UNDERRUN = 2, ERR_REPLAY_RANGE 
                   ERR_TMA_TIMEOUT = 32,    // a record tile's bulk copy did not land within two seconds; tile skipped
                   ERR_STATE = 64,          // compact records: set_state grid is not walls + fruits + live snakes, or more
                                            // fruit cells than the record has slots for
-                  ERR_MAP_RANGE = 128 };   // wall-map pool: a map id was not below the number of maps; map 0 was used
+                  ERR_MAP_RANGE = 128,     // wall-map pool: a map id was not below the number of maps; map 0 was used
+                  ERR_SNAPSHOT = 256 };    // snapshot of an env id outside [0, N), or restore from a slot index out of
+                                           // range or a slot of another configuration; that env was left unchanged
 enum : int { DRAW_STEP_FRUIT = 0, DRAW_SPAWN = 1, DRAW_RESET_FRUIT = 2 };
 enum : int { STAT_EPISODES = 0, STAT_RETURN, STAT_EP_STEPS, STAT_FRUITS, STAT_KILLS, STAT_DEATHS,
              STAT_ENV_STEPS, STAT_COUNT = 8 };

@@ -1865,6 +1865,128 @@ __global__ void snk_init_records_kernel(const Dims d, uint8_t* __restrict__ recs
     reinterpret_cast<uint4*>(recs)[i] = make_uint4(0, 0, 0, 0);
 }
 
+// ---- snapshot / restore: slots of SnapHdr + record + history, moved as 16-byte units, one per thread ----------------
+// Unit j of a slot: 0 the header, 1 .. ru the record, then the history.  I is the index type: 32-bit while every unit
+// index of the launch fits it (the division by the slot's unit count is the costly part of the address arithmetic).
+template <class I>
+__global__ void __launch_bounds__(256) snk_snapshot_kernel(const Dims d, const uint8_t* __restrict__ recs,
+                                                           const uint8_t* __restrict__ hist, const uint8_t* __restrict__ cur_map,
+                                                           const int32_t* __restrict__ ids, int count, uint64_t digest,
+                                                           uint8_t* __restrict__ snap, uint32_t* err) {
+  const I ru = (I)(d.hbm_rec_bytes >> 4), hu = (I)(d.hist_env_bytes >> 4), su = 1 + ru + hu;
+  const I n = (I)count * su;
+  const uint4* rec4 = reinterpret_cast<const uint4*>(recs);
+  const uint4* hist4 = reinterpret_cast<const uint4*>(hist);
+  uint4* out = reinterpret_cast<uint4*>(snap);
+  for (I k = (I)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (I)gridDim.x * blockDim.x) {
+    const I i = k / su, j = k - i * su;
+    const int e = ids ? __ldg(ids + i) : (int)i;
+    const bool ok = (unsigned)e < (unsigned)d.N;
+    uint4 v = make_uint4(0u, 0u, 0u, 0u);
+    if (j == 0) {
+      if (ok) { v.x = (uint32_t)digest; v.y = (uint32_t)(digest >> 32); v.z = cur_map ? cur_map[e] : 0u; }
+      else atomicOr(err, ERR_SNAPSHOT);                 // digest 0: the slot matches no handle
+    } else if (ok) {
+      v = j <= ru ? __ldg(rec4 + (I)e * ru + (j - 1)) : __ldg(hist4 + (I)e * hu + (j - 1 - ru));
+    }
+    __stcs(out + k, v);
+  }
+}
+
+// Indexed by destination: env e takes slot src[e] (-1 keeps it), so no two slots race for one env and one slot may
+// fan out to any number of envs.  mask[e] ends 1 where env e was restored, 0 otherwise.
+template <class I>
+__global__ void __launch_bounds__(256) snk_restore_kernel(const Dims d, uint8_t* __restrict__ recs, uint8_t* __restrict__ hist,
+                                                          uint8_t* __restrict__ cur_map, const int32_t* __restrict__ src,
+                                                          int num_slots, const uint8_t* __restrict__ snap, uint64_t digest,
+                                                          uint8_t* __restrict__ mask, uint32_t* err) {
+  const I ru = (I)(d.hbm_rec_bytes >> 4), hu = (I)(d.hist_env_bytes >> 4), su = 1 + ru + hu;
+  const I n = (I)d.N * su;
+  uint4* rec4 = reinterpret_cast<uint4*>(recs);
+  uint4* hist4 = reinterpret_cast<uint4*>(hist);
+  const uint4* in = reinterpret_cast<const uint4*>(snap);
+  for (I k = (I)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (I)gridDim.x * blockDim.x) {
+    const I e = k / su, j = k - e * su;
+    const int s = __ldg(src + e);
+    if (s == -1) {
+      if (j == 0) mask[e] = 0;
+      continue;
+    }
+    bool ok = s >= 0 && s < num_slots;
+    const uint4* slot = in + (I)(ok ? s : 0) * su;
+    uint4 h = make_uint4(0u, 0u, 0u, 0u);
+    if (ok) {
+      h = __ldg(slot);                                  // every unit's thread checks the header it shares (one line)
+      ok = h.x == (uint32_t)digest && h.y == (uint32_t)(digest >> 32);
+    }
+    if (!ok) {
+      if (j == 0) { mask[e] = 0; atomicOr(err, ERR_SNAPSHOT); }
+      continue;
+    }
+    if (j == 0) {
+      mask[e] = 1;
+      if (cur_map) cur_map[e] = (uint8_t)h.z;
+    } else if (j <= ru) {
+      rec4[e * ru + (j - 1)] = __ldg(slot + j);
+    } else {
+      hist4[e * hu + (j - 1 - ru)] = __ldg(slot + j);
+    }
+  }
+}
+
+// frame_stack > 1 after a restore: one warp per env with mask[e] != 0.  The observation is the env's history ring
+// widened in ring order (oldest frame at hpos, the newest -- the current frame -- last), i.e. the bytes the step that
+// wrote the newest frame returned; the tile kernel's encode cannot serve here, as its F_INIT refills every frame.  The
+// grid row is rebuilt as snk_get_state_kernel does (walls of cur_map, fruit slots, bodies from the tail).
+__global__ void __launch_bounds__(256) snk_emit_stacked_kernel(const Dims d, const uint8_t* __restrict__ recs,
+                                                               const uint8_t* __restrict__ hist,
+                                                               const uint8_t* __restrict__ base_grid, const MapView mv,
+                                                               const uint8_t* __restrict__ mask, uint8_t* __restrict__ obs,
+                                                               uint8_t* __restrict__ bits, uint8_t* __restrict__ grid,
+                                                               uint32_t* err) {
+  const int e = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5);
+  if (e >= d.N || !mask[e]) return;                     // the whole warp leaves together
+  const int lane = (int)lane_id();
+  uint8_t* hb = const_cast<uint8_t*>(recs) + (size_t)e * d.hbm_rec_bytes;
+  const Rec r = rec_view2(hb, hb + d.hbm_c0, d);
+  if (obs || bits) {
+    const int fs = d.fs, hpos = r.hdr->hpos, per_v = d.ohw * fs;
+    const uint8_t* he = hist + (size_t)e * d.hist_env_bytes;
+    uint8_t* be = bits ? bits + (size_t)e * d.stage_env_bytes : nullptr;
+    uint2* oe = obs ? reinterpret_cast<uint2*>(obs + (size_t)e * d.obs_env_bytes) : nullptr;
+    for (int u = lane; u < d.stage_env_bytes; u += 32) {        // u = (viewer, cell, frame), the staging order
+      const int v = u / per_v, rem = u - v * per_v, cell = rem / fs, f = rem - cell * fs;
+      int slot = hpos + f;
+      if (slot >= fs) slot -= fs;
+      const uint32_t b = he[(size_t)(v * fs + slot) * d.ohw_p + cell];
+      if (be) be[u] = (uint8_t)b;
+      if (oe) __stcs(oe + u, make_uint2(spread4(b & 15u), spread4(b >> 4)));
+    }
+  }
+  if (!grid) return;
+  uint8_t* out = grid + (size_t)e * d.HW;
+  if (!d.compact) {
+    for (int c = lane; c < d.HW; c += 32) out[c] = (uint8_t)cell_code(d, r.grid[c]);
+    return;
+  }
+  const uint8_t* walls = env_walls(d, base_grid, mv, e, err);
+  for (int c = lane; c < d.HW; c += 32) out[c] = walls[c];
+  __syncwarp();
+  for (int j = lane; j < d.fcap; j += 32)
+    if (r.fruit[j]) out[r.fruit[j] - 1] = (uint8_t)FRUIT;
+  __syncwarp();
+  if (lane < d.ns && r.alive[lane]) {
+    const int i = lane;
+    int c = r.tail[i];
+    uint8_t code = (uint8_t)(TAIL + 10 * i);
+    for (int guard = 0; guard < d.HW && c != r.head[i]; ++guard) {
+      out[c] = code; code = (uint8_t)(BODY + 10 * i);
+      c += dir_delta(dirp_get(r.dirp, c), d.W);
+    }
+    out[r.head[i]] = (uint8_t)(HEAD + 10 * i);
+  }
+}
+
 // ---- launch wrappers -----------------------------------------------------------------------------
 int tile_group(int ns) { return ns <= 1 ? 1 : ns <= 2 ? 2 : ns <= 4 ? 4 : ns <= 8 ? 8 : ns <= 16 ? 16 : 32; }
 
@@ -2080,6 +2202,35 @@ extern "C" int snk_prof_set_trace2(unsigned long long* dev_buf) {
 
 cudaError_t launch_init_records(const Dims& d, uint8_t* recs, cudaStream_t s) {
   snk_init_records_kernel<<<592, 256, 0, s>>>(d, recs);
+  return cudaGetLastError();
+}
+
+// One 16-byte unit per thread (a grid-stride loop only beyond 2^20 blocks), 32-bit unit indices where they fit.
+static bool units_fit_u32(size_t n) { return n + ((size_t)256 << 20) <= 0xffffffffull; }
+static int unit_blocks(size_t n) { const size_t b = (n + 255) / 256; return (int)(b < ((size_t)1 << 20) ? b : (size_t)1 << 20); }
+
+cudaError_t launch_snapshot(const Dims& d, const uint8_t* recs, const uint8_t* hist, const uint8_t* cur_map, const int32_t* ids,
+                            int count, uint64_t digest, uint8_t* snap, uint32_t* err, cudaStream_t s) {
+  const size_t n = (size_t)count * (snapshot_slot_bytes(d) / 16);
+  if (units_fit_u32(n) && units_fit_u32((size_t)d.N * (snapshot_slot_bytes(d) / 16)))
+    snk_snapshot_kernel<uint32_t><<<unit_blocks(n), 256, 0, s>>>(d, recs, hist, cur_map, ids, count, digest, snap, err);
+  else
+    snk_snapshot_kernel<uint64_t><<<unit_blocks(n), 256, 0, s>>>(d, recs, hist, cur_map, ids, count, digest, snap, err);
+  return cudaGetLastError();
+}
+cudaError_t launch_restore(const Dims& d, uint8_t* recs, uint8_t* hist, uint8_t* cur_map, const int32_t* src, int num_slots,
+                           const uint8_t* snap, uint64_t digest, uint8_t* mask, uint32_t* err, cudaStream_t s) {
+  const size_t n = (size_t)d.N * (snapshot_slot_bytes(d) / 16);
+  if (units_fit_u32(n) && units_fit_u32((size_t)num_slots * (snapshot_slot_bytes(d) / 16)))
+    snk_restore_kernel<uint32_t><<<unit_blocks(n), 256, 0, s>>>(d, recs, hist, cur_map, src, num_slots, snap, digest, mask, err);
+  else
+    snk_restore_kernel<uint64_t><<<unit_blocks(n), 256, 0, s>>>(d, recs, hist, cur_map, src, num_slots, snap, digest, mask, err);
+  return cudaGetLastError();
+}
+cudaError_t launch_emit_stacked(const Dims& d, const uint8_t* recs, const uint8_t* hist, const uint8_t* base_grid,
+                                const MapView& mv, const uint8_t* mask, uint8_t* obs, uint8_t* bits, uint8_t* grid,
+                                uint32_t* err, cudaStream_t s) {
+  snk_emit_stacked_kernel<<<(d.N + 7) / 8, 256, 0, s>>>(d, recs, hist, base_grid, mv, mask, obs, bits, grid, err);
   return cudaGetLastError();
 }
 

@@ -106,6 +106,23 @@ cudaError_t launch_get_state(const Dims& d, const uint8_t* recs, const uint8_t* 
 cudaError_t launch_set_state(const Dims& d, uint8_t* recs, const uint8_t* base_grid, const MapView& mv, uint32_t* err,
                              const StateView& sv, cudaStream_t s);
 cudaError_t launch_init_records(const Dims& d, uint8_t* recs, cudaStream_t s);
+
+// Snapshot slot (snk_snapshot / snk_restore): this header, the env's HBM record (hbm_rec_bytes), then its frame history
+// (hist_env_bytes, frame_stack > 1).  Every part is a multiple of 16 bytes.  digest 0 marks a slot that matches no handle.
+struct SnapHdr { uint64_t digest; uint8_t cur_map; uint8_t pad[7]; };
+static_assert(sizeof(SnapHdr) == 16, "a snapshot slot is moved in 16-byte units");
+inline size_t snapshot_slot_bytes(const Dims& d) { return sizeof(SnapHdr) + (size_t)d.hbm_rec_bytes + (size_t)d.hist_env_bytes; }
+// slot i := env ids[i] (ids null: env i), i < count.  cur_map null: a handle without a wall-map pool
+cudaError_t launch_snapshot(const Dims& d, const uint8_t* recs, const uint8_t* hist, const uint8_t* cur_map, const int32_t* ids,
+                            int count, uint64_t digest, uint8_t* snap, uint32_t* err, cudaStream_t s);
+// env e := slot src[e] where src[e] >= 0; mask[e] := 1 where it was restored, else 0
+cudaError_t launch_restore(const Dims& d, uint8_t* recs, uint8_t* hist, uint8_t* cur_map, const int32_t* src, int num_slots,
+                           const uint8_t* snap, uint64_t digest, uint8_t* mask, uint32_t* err, cudaStream_t s);
+// frame_stack > 1: observation (obs NHWC and / or channel bits) of every env with mask[e] != 0, widened from its history
+// ring as the step that wrote it returned it, and its grid row (grid null: none)
+cudaError_t launch_emit_stacked(const Dims& d, const uint8_t* recs, const uint8_t* hist, const uint8_t* base_grid,
+                                const MapView& mv, const uint8_t* mask, uint8_t* obs, uint8_t* bits, uint8_t* grid,
+                                uint32_t* err, cudaStream_t s);
 // obs: n_units * 8 bytes of 0/1 (16-byte aligned) -> bits: n_units bytes, bit c = byte c of the unit
 cudaError_t launch_pack_obs(const uint8_t* obs, uint8_t* bits, size_t n_units, cudaStream_t s);
 

@@ -425,6 +425,79 @@ class SnakeBatch:
         self._refresh_global_state()
         self._mutated('load_checkpoint')
 
+    # ---- per-env snapshot / restore on the device (snk_snapshot / snk_restore) --------------------------------------
+    @property
+    def snapshot_bytes(self):
+        """Bytes of one snapshot slot: a row of the tensors snapshot() returns and restore() takes."""
+        return int(lib.snk_snapshot_bytes(self._h))
+
+    def _ids(self, x, name):
+        if not isinstance(x, torch.Tensor) or x.device != self.device or x.dim() != 1 \
+                or x.dtype.is_floating_point or x.dtype.is_complex or x.dtype == torch.bool:
+            raise ValueError(f'{name} must be a 1-d integer CUDA tensor on the batch device')
+        return x.to(torch.int32).contiguous()
+
+    def _slots(self, x, name, rows=None):
+        if not isinstance(x, torch.Tensor) or x.dtype != torch.uint8 or x.device != self.device or x.dim() != 2 \
+                or not x.is_contiguous() or x.data_ptr() % 16 or x.shape[0] < 1 \
+                or x.shape[1] != self.snapshot_bytes or (rows is not None and x.shape[0] != rows):
+            want = f'[{rows if rows is not None else "K"}, {self.snapshot_bytes}]'
+            raise ValueError(f'{name} must be a contiguous, 16-byte aligned uint8 CUDA tensor of shape {want} '
+                             '(rows of snapshot_bytes)')
+        return x
+
+    def snapshot(self, env_ids=None, out=None):
+        """The exact state of envs env_ids (an integer CUDA tensor, duplicates allowed; None = all envs) as uint8 [K,
+        snapshot_bytes] on the device: record, frame history and wall map of each env, byte for byte.  `out` may be a
+        preallocated tensor of that shape.  Rows restore into this batch or any batch of the same configuration (see
+        restore); ids outside [0, N) raise a device error (raise_on_device_errors) and give rows nothing accepts."""
+        if env_ids is not None:
+            env_ids = self._ids(env_ids, 'env_ids')
+        K = self.num_envs if env_ids is None else env_ids.numel()
+        if not 1 <= K <= self.num_envs:
+            raise ValueError(f'snapshot takes 1..{self.num_envs} env ids, got {K}')
+        if out is None:
+            out = torch.empty((K, self.snapshot_bytes), dtype=torch.uint8, device=self.device)
+        self._slots(out, 'out', K)
+        check(lib.snk_snapshot(self._h, _ptr(env_ids), K, _ptr(out), self._stream()))
+        return out
+
+    def restore(self, snapshots, src=None, *, env_ids=None, slots=None, copy=False, bits=False):
+        """Put envs back into snapshotted states.  Either src (integer CUDA [N]: env e takes row src[e] of snapshots,
+        -1 keeps it) or env_ids (integer CUDA [K]) with slots (row of each, default 0..K-1; ids outside [0, N) are
+        skipped).  One row may go to any number of envs.  The restored episode continues exactly -- statistics,
+        frame stack, replay cursor and Philox event count included -- with draws keyed by the destination env's id, so
+        a row restored into another env continues that env's own stream (snk.h).  Writes the restored envs' rows of
+        the observation buffer (the channel-bit buffer with bits=True) and of global_state, and returns that buffer."""
+        snapshots = self._slots(snapshots, 'snapshots')
+        N = self.num_envs
+        if src is not None:
+            if env_ids is not None or slots is not None:
+                raise ValueError('give either src or env_ids (and slots), not both')
+            src = self._ids(src, 'src')
+            if src.numel() != N:
+                raise ValueError('src must have one entry per environment')
+        else:
+            if env_ids is None:
+                raise ValueError('restore needs src or env_ids')
+            env_ids = self._ids(env_ids, 'env_ids')
+            slots = torch.arange(env_ids.numel(), dtype=torch.int32, device=self.device) if slots is None \
+                else self._ids(slots, 'slots')
+            if slots.numel() != env_ids.numel():
+                raise ValueError('slots must have one entry per env id')
+            # built on the device without a synchronisation: ids outside [0, N) land in a spare last entry
+            ids = torch.where((env_ids >= 0) & (env_ids < N), env_ids, N).long()
+            src = torch.full((N + 1,), -1, dtype=torch.int32, device=self.device)
+            src.index_put_((ids,), slots)
+            src = src[:N]
+        with torch.cuda.device(self.device):
+            out = self._bits_buffer() if bits else self._obs
+            check(lib.snk_restore(self._h, _ptr(src), snapshots.shape[0], _ptr(snapshots), None if bits else _ptr(out),
+                                  _ptr(out) if bits else None, _ptr(self.global_state), self._stream()))
+        # as a masked reset: only the restored envs' observation rows are rewritten
+        self._mutated('restore(bits=True)' if bits else False)
+        return out.clone() if copy else out
+
     def set_replay(self, draws_per_env):
         """draws_per_env: sequence of N int arrays -- recorded draw outputs in consumption order."""
         assert len(draws_per_env) == self.num_envs
