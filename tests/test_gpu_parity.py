@@ -378,8 +378,28 @@ def test_gpu_alternative_code_paths(monkeypatch, knob, kw, N):
         k, v = kv.split('=')
         monkeypatch.setenv(k, v)
     ns = kw['num_snakes']
+    # the uncapped instance: a step into the batch's own (compressible) block runs the capped one, so step into a
+    # plain buffer, and check through the launch witness (in a fresh process, where the profiler records reliably)
+    # that the steps run the warp-private variant 3
+    bigreg = 'SNK_BIGREG_TILES' in knob
+    if bigreg:
+        from test_gpu_instances import witnessed_tiles
+        tiles = witnessed_tiles(f"""
+import json, numpy as np
+from gpu_backend import GpuBackend
+from test_gpu_instances import witness
+be = GpuBackend({N}, {kw!r}, rng_mode=0, auto_reset=1, seed=8, plain_obs=True)
+be.reset()
+rng = np.random.RandomState(4)
+tiles = []
+for t in range(2):
+    be.step(rng.randint(0, 3, size=({N}, {kw['num_snakes']})).astype(np.uint8), around=witness)
+    tiles.append(be.around_value.tiles)
+print(json.dumps(tiles))
+""")
+        assert len(tiles) == 2 and all(len(w) == 1 and w[0][5] == 0 and w[0][7] == 3 for w in tiles), tiles
     hs = HostSim(N, kw, rng_mode=0, auto_reset=1, seed=8)
-    be = GpuBackend(N, kw, rng_mode=0, auto_reset=1, seed=8)
+    be = GpuBackend(N, kw, rng_mode=0, auto_reset=1, seed=8, plain_obs=bigreg)
     assert np.array_equal(hs.reset(), be.reset())
     rng = np.random.RandomState(4)
     for t in range(60):
